@@ -3,6 +3,7 @@
 buffers through the C ABI), reference-on-the-same-GPU and CPU-baseline legs.  Prints ONE JSON line (rank 0).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--scaling weak|strong] [--graph]
+                    [--dump-outputs DIR]
     python bench.py --impl reference ...          (the reference's own CPU implementation, same metric/config)
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
@@ -38,6 +39,7 @@ WORKLOADS = {
     "sot512-logf-cut": (512, True, "logf"),          # configs[2]
 }
 L2_BYTES = 126e6
+DUMP_BYTES = 48 << 20  # both sampled gradients of --dump-outputs (+ 4 bytes of loss), within a 64 MB budget
 
 
 def parse():
@@ -60,7 +62,40 @@ def parse():
     ap.add_argument("--no-ref-cuda", action="store_true")
     ap.add_argument("--no-check", action="store_true", help="skip the rank-0 recomputation of the sharded value")
     ap.add_argument("--cpu-frames", type=int, default=4096, help="frames per call of the CPU reference")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (loss.npy, grad_x.npy, grad_y.npy, "
+                         "float32; rank 0's shard) to DIR, the gradients cut to a fixed sample of frames if larger "
+                         f"than {DUMP_BYTES >> 20} MiB: the inputs are seeded, so two builds can be compared file by file")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
+    return args
+
+
+def sample_frames(frames, bins):
+    """Frames whose gradients `--dump-outputs` writes: all of them when both gradients fit DUMP_BYTES, else a sorted
+    sample drawn from a fixed seed, so that the same arguments select the same frames in every run."""
+    keep = DUMP_BYTES // (2 * 4 * bins)
+    if frames <= keep:
+        return None
+    return torch.randperm(frames, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+
+
+def dump_outputs(out_dir, value, grad_x, grad_y):
+    """Writes the loss and the two gradients one step returned as float32 .npy files; returns what was written."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    frames, bins = grad_x.shape
+    idx = sample_frames(frames, bins)
+    if idx is not None:
+        idx = idx.to(grad_x.device)
+        grad_x, grad_y = grad_x[idx], grad_y[idx]
+    for name, t in (("loss", value.detach().reshape(1)), ("grad_x", grad_x), ("grad_y", grad_y)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    return {"dir": out_dir, "frames_written": frames if idx is None else int(idx.numel()), "frames": frames,
+            "sample": None if idx is None else "sorted randperm(frames), torch generator seed 0"}
 
 
 def peaks():
@@ -384,6 +419,12 @@ def main():
     sampler.end()
     torch.cuda.cudart().cudaProfilerStop()
     launches = _capi.launch_count() - launches0
+    last_set = (args.steps - 1) % n_sets
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # now, before the legs below reuse the leaves (the graph leg clears their gradients)
+        xg, yg = leaves[last_set]
+        dumped = dump_outputs(args.dump_outputs, value, xg.grad, yg.grad)
     host_issue = None if host_s[2] == 0 else {"forward_us": 1e6 * host_s[0] / host_s[2],
                                               "backward_us": 1e6 * host_s[1] / host_s[2],
                                               "note": "host time to ISSUE one step (no synchronisation)"}
@@ -399,7 +440,6 @@ def main():
     ms_step = ms_total.item() / args.steps
     frames_s = frames * world / (ms_step * 1e-3)
     value_last = float(value.item())
-    last_set = (args.steps - 1) % n_sets
     exchange = loss_fn.exchange
     collective = {"used": getattr(exchange, "collective_used", None) if world > 1 else "none (one rank)",
                   "requested": args.collective, "fallback_reason": getattr(exchange, "fallback_reason", None),
@@ -554,6 +594,8 @@ def main():
                 "collective_used": collective["used"], "value_check": value_check, "step_modes": other,
                 "host_issue": host_issue,
                 "loss": value_last, "backward_mode": loss_fn.backward_mode}
+        if dumped is not None:
+            line["dumped_outputs"] = dumped
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

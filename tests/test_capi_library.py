@@ -67,10 +67,13 @@ def test_sass_contains_tma_bulk_copies():
     """The hot kernels move rows with cp.async.bulk (SASS UBLKCP), not with per-thread loads."""
     import shutil
     import subprocess
+    from torch.utils.cpp_extension import CUDA_HOME
     from sot_b200 import _capi
-    if shutil.which("cuobjdump") is None:
+    # the CUDA toolkit's own copy when its bin/ is not on PATH
+    tool = shutil.which("cuobjdump") or os.path.join(CUDA_HOME or "", "bin", "cuobjdump")
+    if not os.path.isfile(tool):
         pytest.skip("cuobjdump not available")
-    sass = subprocess.run(["cuobjdump", "-sass", _capi.library_path()], capture_output=True, text=True).stdout
+    sass = subprocess.run([tool, "-sass", _capi.library_path()], capture_output=True, text=True).stdout
     assert "UBLKCP" in sass and "SYNCS" in sass
 
 

@@ -135,20 +135,8 @@ def _run_example(*extra):
 
 def test_training_step_example_reduces_the_loss():
     """examples/train_step.py (SURVEY section 8 row f2): the paper's loss mix inside a plain training loop."""
-    line = _run_example("--steps", "60", "--batch", "32", "--lr", "1e-3", "--model", "standin")
+    line = _run_example("--steps", "60", "--batch", "32", "--lr", "1e-3", "--model", "standin", "--loss-share")
     assert line["last_loss"] < line["first_loss"] and line["frames_per_s"] > 0
-
-
-def test_training_step_example_with_the_references_encoder_and_synth():
-    """The same step around the reference's own PESTO encoder (46 012 parameters) and DDSP oscillator bank, imported
-    unmodified from the staged copy baseline/_ref/ (git-ignored; made by `__graft_entry__.build()`)."""
-    import os
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    if not (os.path.isfile("/root/reference/encoder.py") or os.path.isfile(os.path.join(root, "baseline", "_ref", "encoder.py"))):
-        pytest.skip("the reference's files are not staged on this box")
-    line = _run_example("--steps", "40", "--batch", "64", "--model", "reference", "--loss-share")  # paper config: lr 1e-4
-    assert line["model"] == "reference" and line["trainable_parameters"] == 46012
-    assert line["last_loss"] == line["last_loss"] and line["last_loss"] < line["first_loss"]  # finite and going down
     assert 0.0 <= line["loss_share"]["share_of_step_in_the_two_losses"] <= 1.0
 
 

@@ -15,6 +15,7 @@ from . import build as _build
 
 SOT_SQUARE, SOT_CUT_SCALE, SOT_LIMIT, SOT_RAW_WEIGHTS, SOT_UNIFORM_GRID, SOT_COMPLEX_INPUT = 1, 2, 4, 8, 16, 32
 ABI_VERSION = 2
+MAX_COMPLEX_BINS = 4352  # longest SOT_COMPLEX_INPUT row (include/sot_b200.h: sot_max_bins); real rows take 2^24 - 1
 
 _c_float_p = ctypes.c_void_p  # device pointers travel as integers
 
@@ -429,6 +430,8 @@ def loss_grad_host(u, v, pos_u, pos_v, p, flags, upstream=None, want_loss=True, 
 
 
 def set_tuning(threads_per_frame: int = 0, bins_per_thread: int = 0, chains_per_thread: int = 0):
+    """Select a kernel configuration (benchmarks, tests); (0, 0, 0) restores the built-in choice and (-1, 0, 0)
+    routes every real-row loss / gradient request through the split-frame path of long rows."""
     _check(load().sot_set_tuning(threads_per_frame, bins_per_thread, chains_per_thread))
 
 

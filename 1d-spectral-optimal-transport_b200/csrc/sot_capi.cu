@@ -30,6 +30,9 @@ SOT_DECLARE_CONFIG(32, 33, 1064, 2)
 #endif
 
 namespace sot {
+// rows longer than shared memory holds (sot_long.cu)
+cudaError_t sot_launch_long(const LaunchRequest& r, cudaStream_t stream);
+
 // ------------------------------------------------------------------------------------------
 // grad rows scaled by a per-frame factor: out[r, :] = unit[r, :] * s[r]   (backward of the
 // "fused" mode, where the forward launch already produced d loss_r / d input)
@@ -143,6 +146,9 @@ thread_local char g_error[512] = "";
 std::atomic<long long> g_launches{0};
 std::atomic<int> g_tune_tpf{0}, g_tune_e{0}, g_tune_nch{0};
 std::atomic<bool> g_prefer_sub{true};   // sub-warp configurations by default (when the request allows)
+std::atomic<bool> g_force_long{false};  // sot_set_tuning(-1, 0, 0): every request the split-frame path serves takes it
+constexpr int kMaxRowBins = (1 << 24) - 1;  // longest row (split-frame path)
+constexpr int kMaxComplexBins = 4352;       // longest complex row: the two double-width landing rows fit shared memory
 
 int fail(int code, const char* fmt, ...) {
     va_list ap;
@@ -177,7 +183,8 @@ int validate(const sot_problem* p) {
     if (p == nullptr) return fail(SOT_EINVAL, "problem is NULL");
     if (p->n_frames < 0 || p->n_u < 1 || p->n_v < 1)
         return fail(SOT_EINVAL, "bad sizes: n_frames=%lld n_u=%d n_v=%d", (long long)p->n_frames, p->n_u, p->n_v);
-    if (p->n_u >= 65536 || p->n_v >= 65536) return fail(SOT_ETOOBIG, "rows longer than 65535 bins");
+    if (p->n_u > kMaxRowBins || p->n_v > kMaxRowBins)
+        return fail(SOT_ETOOBIG, "rows longer than %d bins", kMaxRowBins);
     if (p->n_frames > 0 && (p->u == nullptr || p->v == nullptr)) return fail(SOT_EINVAL, "u or v is NULL");
     if (p->pos_u == nullptr || p->pos_v == nullptr)
         return fail(SOT_EINVAL, "support positions are required (pos_u / pos_v is NULL)");
@@ -219,15 +226,37 @@ int launch(const sot_problem* p, sot::LaunchRequest& r, void* stream) {
     const bool sub_ok = r.mode == sot::MODE_SPECTRA && r.out != sot::OUT_PLAN &&
                         !(p->flags & (SOT_RAW_WEIGHTS | SOT_COMPLEX_INPUT)) && r.args.coranks_in == nullptr &&
                         r.args.coranks_out == nullptr;
-    const Config* c = pick_config(p->n_u, p->n_v, sub_ok);
-    if (c == nullptr)
-        return fail(SOT_ETOOBIG, "rows of %d / %d bins exceed the largest kernel configuration (%d bins)", p->n_u,
-                    p->n_v, sot_max_bins(1, 1));
+    // the split-frame path (global-memory scratch): real rows, loss and gradients
+    const bool long_ok = r.mode == sot::MODE_SPECTRA && r.out != sot::OUT_PLAN && !(p->flags & SOT_COMPLEX_INPUT);
+    const Config* c = (long_ok && g_force_long.load()) ? nullptr : pick_config(p->n_u, p->n_v, sub_ok);
     // complex input keeps two double-width landing rows on top of the real rows: up to 10 rows of 4*rs bytes (+ pad, head)
-    if ((p->flags & SOT_COMPLEX_INPUT) && 41 * c->rs + 8192 > 227 * 1024)
+    if ((p->flags & SOT_COMPLEX_INPUT) && (c == nullptr || 41 * c->rs + 8192 > 227 * 1024))
         return fail(SOT_ETOOBIG, "complex rows of %d / %d bins do not fit in shared memory (limit %d bins)", p->n_u,
-                    p->n_v, 4352);
-    cudaError_t e = c->fn(r, static_cast<cudaStream_t>(stream));
+                    p->n_v, kMaxComplexBins);
+    if (c == nullptr && !long_ok)
+        return fail(SOT_ETOOBIG, "rows of %d / %d bins exceed the largest kernel configuration of this entry point "
+                    "(%d bins: quantile taps and the CDF harness run in shared memory)", p->n_u, p->n_v,
+                    kConfigs[kNumConfigs - 1].max_bins());
+    if (c == nullptr) {
+        // Rows longer than shared memory holds run on the split-frame path, which re-reads its rows and positions from
+        // global memory: it takes them only where the runtime confirms the device can reach them (a host buffer handed
+        // to a device entry point, or no usable device, is refused here rather than faulting in the kernel).
+        const void* rows_and_positions[] = {p->u, p->v, p->pos_u, p->pos_v};
+        for (const void* q : rows_and_positions) {
+            cudaPointerAttributes attr;
+            const cudaError_t pe = cudaPointerGetAttributes(&attr, q);
+            if (pe != cudaSuccess || attr.devicePointer == nullptr) {
+                if (pe != cudaSuccess) cudaGetLastError();  // (not sticky: leave no error behind for the caller)
+                return fail(SOT_ETOOBIG,
+                            "rows of %d / %d bins exceed shared memory (%d bins) and the split-frame path needs rows "
+                            "and positions in device-accessible memory (%s)",
+                            p->n_u, p->n_v, kConfigs[kNumConfigs - 1].max_bins(),
+                            pe != cudaSuccess ? cudaGetErrorString(pe) : "a pointer the device cannot reach");
+            }
+        }
+    }
+    cudaError_t e = c != nullptr ? c->fn(r, static_cast<cudaStream_t>(stream))
+                                 : sot::sot_launch_long(r, static_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) return cuda_fail(e, "sot_frames_kernel launch");
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return SOT_OK;
@@ -249,6 +278,11 @@ int sot_set_tuning(int32_t tpf, int32_t e, int32_t chains) {
         g_tune_tpf = 0;
         g_tune_e = 0;
         g_tune_nch = 0;
+        g_force_long = false;
+        return SOT_OK;
+    }
+    if (tpf == -1 && e == 0 && chains == 0) {
+        g_force_long = true;
         return SOT_OK;
     }
     for (int i = 0; i < kNumConfigs; ++i)
@@ -262,12 +296,7 @@ int sot_set_tuning(int32_t tpf, int32_t e, int32_t chains) {
                 e, chains);
 }
 
-int sot_max_bins(int32_t /*with_grad*/, int32_t /*shared_positions*/) {
-    int best = 0;
-    for (int i = 0; i < kNumConfigs; ++i)
-        if (kConfigs[i].max_bins() > best) best = kConfigs[i].max_bins();
-    return best;
-}
+int sot_max_bins(int32_t /*with_grad*/, int32_t /*shared_positions*/) { return kMaxRowBins; }
 
 int sot_forward_device(const sot_problem* prob, float* loss, void* stream) {
     if (int rc = validate(prob)) return rc;
@@ -293,6 +322,7 @@ int sot_forward_backward_device(const sot_problem* prob, const float* upstream, 
 // configurations with the same threads x chains cut the merged grid identically, so co-ranks saved by one are valid
 // for the other -- the count is the whole compatibility condition.
 int sot_coranks_per_frame(int32_t n_u, int32_t n_v) {
+    if (g_force_long.load()) return 0;  // (the split-frame path keeps no co-ranks)
     const Config* c = pick_config(n_u, n_v);
     return c == nullptr ? 0 : c->tpf * c->nch;
 }
@@ -586,7 +616,9 @@ int sot_loss_grad_host(const sot_problem* hp, const float* upstream, float* loss
     // Zero-copy (SOT_HOST_ZEROCOPY=1; shared supports; every buffer pinned and mapped): ONE launch over the whole batch
     // whose bulk loads and stores go over PCIe themselves -- no staging buffers, no fill and drain of a copy pipeline.
     // Anything else (pageable memory, per-frame supports) takes the chunked pipeline below.
-    if (const char* zc = getenv("SOT_HOST_ZEROCOPY"); zc != nullptr && zc[0] == '1' && su && sv) {
+    // (rows longer than shared memory holds: the split-frame path re-reads its rows, so they are staged on the device)
+    if (const char* zc = getenv("SOT_HOST_ZEROCOPY");
+        zc != nullptr && zc[0] == '1' && su && sv && !g_force_long.load() && pick_config(n, m) != nullptr) {
         const float* du = mapped_device_pointer(hp->u);
         const float* dv = mapped_device_pointer(hp->v);
         const float* dup = mapped_device_pointer(upstream);

@@ -208,6 +208,9 @@ def _prepare(x, y, x_pos, y_pos, p, square, cut_scale, limit, require_sort, raw_
     u, v = _rows(x, "x"), _rows(y, "y")
     if u.is_complex() != v.is_complex():  # one side already a magnitude: take |.| of the other in torch
         u, v = (u.abs() if u.is_complex() else u), (v.abs() if v.is_complex() else v)
+    if u.is_complex() and max(u.shape[1], v.shape[1]) > _capi.MAX_COMPLEX_BINS:
+        # complex rows too long for the fused |z| prologue (shared memory): |z| in torch, the real path takes any length
+        u, v = u.abs(), v.abs()
     if u.is_complex() and raw_weights:
         raise TypeError("sot_b200: `wasserstein_1d` weights must be real")
     if u.shape[0] != v.shape[0]:

@@ -49,7 +49,7 @@ extern "C" {
 /* error codes */
 #define SOT_OK 0
 #define SOT_EINVAL (-1)   /* bad pointer / size / flag combination        */
-#define SOT_ETOOBIG (-2)  /* row does not fit the largest kernel config   */
+#define SOT_ETOOBIG (-2)  /* row longer than the entry point accepts       */
 #define SOT_EDOMAIN (-3)  /* p < 1 (reference: AssertionError, losses.py:271) */
 
 /* One batch of frames.  Mirrors the arguments of `wasserstein_1d` (losses.py:223-232) plus the
@@ -182,7 +182,12 @@ int sot_host_release(int32_t device);
 /* ---- housekeeping ---------------------------------------------------------------------------- */
 int sot_abi_version(void);
 const char* sot_last_error(void);
-/* Largest row length (max(n_u, n_v)) the kernels accept for the given outputs. */
+/* Largest row length (max(n_u, n_v)) the loss / gradient entry points accept: 2^24 - 1.  Real rows longer than one
+ * CTA's shared memory holds (more than 8448 bins) run on the split-frame path (global-memory scratch, allocated
+ * stream-ordered on the call's stream: no host synchronisation, capturable in a CUDA graph), which needs u, v and the
+ * positions in memory the device can reach (else SOT_ETOOBIG); co-ranks are not kept for them (sot_coranks_per_frame
+ * returns 0).  Shared memory bounds the rest: sot_quantiles_device and the CDF
+ * harness take up to 8448 bins, SOT_COMPLEX_INPUT rows up to 4352; longer rows there return SOT_ETOOBIG. */
 int sot_max_bins(int32_t with_grad, int32_t shared_positions);
 /* ---- Multi-scale spectral loss term (row f3; losses.py:365-425 `MSSLoss`, :7-36 `mean_difference`,
  * utils.py:145-151 `safe_log`) for ONE fft size, straight from the two complex64 spectrograms zt (target) and zv
@@ -227,7 +232,8 @@ int sot_p2p_wait_mean_device(float* mean_out, double expected_count, int32_t* st
 
 /* Tuning override for benchmarking: threads per frame (32/64/128/256), bins per thread (odd) and
  * merge chains per thread (1/2, 0 = any); 0, 0, 0 restores the built-in choice.  Returns SOT_EINVAL
- * if that combination is not compiled in. */
+ * if that combination is not compiled in.  -1, 0, 0 routes every real-row loss / gradient request through the
+ * split-frame path, whatever the row length (tests and benchmarks compare it with the shared-memory kernels). */
 int sot_set_tuning(int32_t threads_per_frame, int32_t bins_per_thread, int32_t chains_per_thread);
 /* Number of kernel launches issued by this library in the calling process so far. */
 int64_t sot_launch_count(void);

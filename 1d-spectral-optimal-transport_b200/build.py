@@ -28,19 +28,8 @@ def _nvcc() -> str:
     return exe
 
 
-# configurations that only `sot_set_tuning` could ever reach: compiled with SOT_BUILD_TUNING=1
-TUNING_ONLY = ("sot_cfg_32_9_296_2", "sot_cfg_64_17_1096_2", "sot_cfg_32_33_1064_2")
-
-
-def _tuning() -> bool:
-    return os.environ.get("SOT_BUILD_TUNING", "0") not in ("", "0")
-
-
 def _sources():
-    srcs = sorted(glob.glob(os.path.join(CSRC, "*.cu")))
-    if not _tuning():
-        srcs = [s for s in srcs if os.path.basename(s)[:-3] not in TUNING_ONLY]
-    return srcs
+    return sorted(glob.glob(os.path.join(CSRC, "*.cu")))
 
 
 def _deps():
@@ -57,7 +46,7 @@ def is_stale() -> bool:
 
 def _compile(src: str) -> str:
     obj = os.path.join(OBJ_DIR, os.path.basename(src)[:-3] + ".o")
-    cmd = [_nvcc(), *NVCC_FLAGS, *(["-DSOT_TUNING_CONFIGS"] if _tuning() else []), "-c", src, "-o", obj]
+    cmd = [_nvcc(), *NVCC_FLAGS, "-c", src, "-o", obj]
     res = subprocess.run(cmd, capture_output=True, text=True)
     with open(obj[:-2] + ".ptxas.log", "w") as f:
         f.write(res.stdout + res.stderr)

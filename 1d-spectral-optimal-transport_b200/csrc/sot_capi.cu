@@ -10,28 +10,18 @@
 #include <mutex>
 
 #include "../../include/sot_b200.h"
+#include "sot_internal.cuh"
 #include "sot_launch.cuh"
 
-// Production configurations (one per row-length class).  The alternatives that were only ever reachable through
-// `sot_set_tuning` are compiled in with -DSOT_TUNING_CONFIGS (`SOT_BUILD_TUNING=1 python -m sot_b200.build`).
-SOT_DECLARE_SUBWARP_CONFIG(16, 17, 280, 1)
-SOT_DECLARE_CONFIG(32, 9, 296, 1)
-SOT_DECLARE_CONFIG(64, 9, 584, 2)
-SOT_DECLARE_CONFIG(32, 33, 1064, 1)
-SOT_DECLARE_CONFIG(64, 17, 1096, 1)
-SOT_DECLARE_CONFIG(128, 9, 1160, 1)
-SOT_DECLARE_CONFIG(128, 17, 2184, 2)
-SOT_DECLARE_CONFIG(256, 17, 4360, 2)
-SOT_DECLARE_CONFIG(256, 33, 8456, 1)
-#ifdef SOT_TUNING_CONFIGS
-SOT_DECLARE_CONFIG(32, 9, 296, 2)
-SOT_DECLARE_CONFIG(64, 17, 1096, 2)
-SOT_DECLARE_CONFIG(32, 33, 1064, 2)
-#endif
+// the launcher of every configuration of sot_configs.cuh, defined in its own csrc/sot_cfg_*.cu
+#define SOT_CONFIG(TPF, E, RS, NCH, FPW) \
+    cudaError_t sot_launch_##TPF##_##E##_##RS##_##NCH(const sot::LaunchRequest& r, cudaStream_t stream);
+#include "sot_configs.cuh"
+#undef SOT_CONFIG
+
+using sot::fail;
 
 namespace sot {
-// rows longer than shared memory holds (sot_long.cu)
-cudaError_t sot_launch_long(const LaunchRequest& r, cudaStream_t stream);
 
 // ------------------------------------------------------------------------------------------
 // grad rows scaled by a per-frame factor: out[r, :] = unit[r, :] * s[r]   (backward of the
@@ -120,62 +110,34 @@ struct Config {
     bool sub;  // sub-warp frames (several frames per warp): real spectra -> loss / gradients only
     int max_bins() const { return tpf * e < rs - 7 ? tpf * e : rs - 7; }
 };
-// Ordered by preference for a given row length: the first entry that holds the row is used
-// (choices from measurements on B200, profiles/).  Shared memory per CTA = (4 or 6) * 4 * rs bytes.
+// in order of preference, see sot_configs.cuh
 const Config kConfigs[] = {
-    {16, 17, 280, 1, sot_launch_sub_16_17_280_1, true},  // <= 272 bins (n_fft 512: 257): two frames per warp
-    {32, 9, 296, 1, sot_launch_32_9_296_1},      // <= 288 bins   (one warp per frame: plans, CDF harness, raw, complex)
-    {64, 9, 584, 2, sot_launch_64_9_584_2},      // <= 576 bins   (n_fft 1024: 513)
-    {32, 33, 1064, 1, sot_launch_32_33_1064_1},  // <= 1056 bins  (n_fft 2048: 1025): ONE WARP per frame, 33 bins per thread --
-                                                 // no CTA barriers, half the per-frame fixed cost; since the gradient stage
-                                                 // rebuilds its suffix sums (162 registers, no spills) 14 % faster than 64 x 17
-    {64, 17, 1096, 1, sot_launch_64_17_1096_1},  // <= 1088 bins  (two warps per frame: the round-1 / early round-2 choice)
-#ifdef SOT_TUNING_CONFIGS
-    {32, 9, 296, 2, sot_launch_32_9_296_2},      // two-chain variant: measured slower
-    {64, 17, 1096, 2, sot_launch_64_17_1096_2},  // alternatives for 1025 bins (profiles/r01j_tuning_experiments.txt)
-    {32, 33, 1064, 2, sot_launch_32_33_1064_2},  // two merge chains per thread: 165 vs 182 M frames/s
-#endif
-    {128, 9, 1160, 1, sot_launch_128_9_1160_1},    // <= 1152 bins
-    {128, 17, 2184, 2, sot_launch_128_17_2184_2},  // <= 2176 bins  (n_fft 4096: 2049)
-    {256, 17, 4360, 2, sot_launch_256_17_4360_2},  // <= 4352 bins  (n_fft 8192: 4097)
-    {256, 33, 8456, 1, sot_launch_256_33_8456_1},  // <= 8448 bins  (n_fft 16384: 8193)
+#define SOT_CONFIG(TPF, E, RS, NCH, FPW) {TPF, E, RS, NCH, sot_launch_##TPF##_##E##_##RS##_##NCH, FPW > 1},
+#include "sot_configs.cuh"
+#undef SOT_CONFIG
 };
 constexpr int kNumConfigs = sizeof(kConfigs) / sizeof(kConfigs[0]);
 
 thread_local char g_error[512] = "";
 std::atomic<long long> g_launches{0};
-std::atomic<int> g_tune_tpf{0}, g_tune_e{0}, g_tune_nch{0};
-std::atomic<bool> g_prefer_sub{true};   // sub-warp configurations by default (when the request allows)
-std::atomic<bool> g_force_long{false};  // sot_set_tuning(-1, 0, 0): every request the split-frame path serves takes it
+// sot_set_tuning: the built-in choice, every request the split-frame path serves on that path, or an index of kConfigs
+constexpr int kTuneAuto = -1, kTuneLong = -2;
+std::atomic<int> g_tuning{kTuneAuto};
 constexpr int kMaxRowBins = (1 << 24) - 1;  // longest row (split-frame path)
 constexpr int kMaxComplexBins = 4352;       // longest complex row: the two double-width landing rows fit shared memory
 
-int fail(int code, const char* fmt, ...) {
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_error, sizeof(g_error), fmt, ap);
-    va_end(ap);
-    return code;
-}
 int cuda_fail(cudaError_t e, const char* what) {
     snprintf(g_error, sizeof(g_error), "%s: %s", what, cudaGetErrorString(e));
     return static_cast<int>(e);
 }
 
-// `sub_ok`: the request is one the sub-warp configurations serve (see Config::sub)
-const Config* pick_config(int n, int m, bool sub_ok = false) {
+// `tuning`: a value of g_tuning.  `sub_ok`: the request is one the sub-warp configurations serve (see Config::sub).
+const Config* pick_config(int tuning, int n, int m, bool sub_ok = false) {
     const int need = n > m ? n : m;
-    const int tt = g_tune_tpf.load(), te = g_tune_e.load();
-    if (tt != 0) {
-        for (int i = 0; i < kNumConfigs; ++i) {
-            const Config& c = kConfigs[i];
-            if (c.tpf == tt && c.e == te && (g_tune_nch.load() == 0 || c.nch == g_tune_nch.load()) &&
-                c.max_bins() >= need && (!c.sub || sub_ok))
-                return &c;
-        }
-    }
-    for (int i = 0; i < kNumConfigs; ++i)
-        if (kConfigs[i].max_bins() >= need && (!kConfigs[i].sub || (sub_ok && g_prefer_sub.load()))) return &kConfigs[i];
+    if (tuning >= 0 && kConfigs[tuning].max_bins() >= need && (!kConfigs[tuning].sub || sub_ok))
+        return &kConfigs[tuning];
+    for (const Config& c : kConfigs)
+        if (c.max_bins() >= need && (!c.sub || sub_ok)) return &c;
     return nullptr;
 }
 
@@ -228,7 +190,8 @@ int launch(const sot_problem* p, sot::LaunchRequest& r, void* stream) {
                         r.args.coranks_out == nullptr;
     // the split-frame path (global-memory scratch): real rows, loss and gradients
     const bool long_ok = r.mode == sot::MODE_SPECTRA && r.out != sot::OUT_PLAN && !(p->flags & SOT_COMPLEX_INPUT);
-    const Config* c = (long_ok && g_force_long.load()) ? nullptr : pick_config(p->n_u, p->n_v, sub_ok);
+    const int tuning = g_tuning.load();
+    const Config* c = (long_ok && tuning == kTuneLong) ? nullptr : pick_config(tuning, p->n_u, p->n_v, sub_ok);
     // complex input keeps two double-width landing rows on top of the real rows: up to 10 rows of 4*rs bytes (+ pad, head)
     if ((p->flags & SOT_COMPLEX_INPUT) && (c == nullptr || 41 * c->rs + 8192 > 227 * 1024))
         return fail(SOT_ETOOBIG, "complex rows of %d / %d bins do not fit in shared memory (limit %d bins)", p->n_u,
@@ -255,41 +218,48 @@ int launch(const sot_problem* p, sot::LaunchRequest& r, void* stream) {
             }
         }
     }
-    cudaError_t e = c != nullptr ? c->fn(r, static_cast<cudaStream_t>(stream))
-                                 : sot::sot_launch_long(r, static_cast<cudaStream_t>(stream));
-    if (e != cudaSuccess) return cuda_fail(e, "sot_frames_kernel launch");
+    if (c != nullptr) return sot::launched(c->fn(r, static_cast<cudaStream_t>(stream)), "sot_frame_kernel");
+    return sot::launched(sot::sot_launch_long(r, static_cast<cudaStream_t>(stream)), "sot_long_kernel");
+}
+
+}  // namespace
+
+namespace sot {
+
+int fail(int code, const char* fmt, ...) {
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(g_error, sizeof(g_error), fmt, ap);
+    va_end(ap);
+    return code;
+}
+
+int launched(cudaError_t e, const char* kernel) {
+    if (e != cudaSuccess) return fail(static_cast<int>(e), "%s launch: %s", kernel, cudaGetErrorString(e));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return SOT_OK;
 }
 
-}  // namespace
+}  // namespace sot
 
 extern "C" {
 
 int sot_abi_version(void) { return SOT_B200_ABI_VERSION; }
 const char* sot_last_error(void) { return g_error; }
 int64_t sot_launch_count(void) { return g_launches.load(); }
-// shared with sot_mss.cu (not part of the public header)
-int sot_mss_launch_count_add(void) { return static_cast<int>(g_launches.fetch_add(1, std::memory_order_relaxed)); }
-int sot_mss_fail(int code, const char* msg) { return code < 0 ? fail(code, "%s", msg) : (snprintf(g_error, sizeof(g_error), "%s", msg), code); }
 
 int sot_set_tuning(int32_t tpf, int32_t e, int32_t chains) {
     if (tpf == 0 && e == 0) {
-        g_tune_tpf = 0;
-        g_tune_e = 0;
-        g_tune_nch = 0;
-        g_force_long = false;
+        g_tuning = kTuneAuto;
         return SOT_OK;
     }
     if (tpf == -1 && e == 0 && chains == 0) {
-        g_force_long = true;
+        g_tuning = kTuneLong;
         return SOT_OK;
     }
     for (int i = 0; i < kNumConfigs; ++i)
         if (kConfigs[i].tpf == tpf && kConfigs[i].e == e && (chains == 0 || kConfigs[i].nch == chains)) {
-            g_tune_tpf = tpf;
-            g_tune_e = e;
-            g_tune_nch = chains;
+            g_tuning = i;
             return SOT_OK;
         }
     return fail(SOT_EINVAL, "no kernel configuration with %d threads per frame, %d bins per thread, %d chain(s)", tpf,
@@ -322,8 +292,9 @@ int sot_forward_backward_device(const sot_problem* prob, const float* upstream, 
 // configurations with the same threads x chains cut the merged grid identically, so co-ranks saved by one are valid
 // for the other -- the count is the whole compatibility condition.
 int sot_coranks_per_frame(int32_t n_u, int32_t n_v) {
-    if (g_force_long.load()) return 0;  // (the split-frame path keeps no co-ranks)
-    const Config* c = pick_config(n_u, n_v);
+    const int tuning = g_tuning.load();
+    if (tuning == kTuneLong) return 0;  // (the split-frame path keeps no co-ranks)
+    const Config* c = pick_config(tuning, n_u, n_v);
     return c == nullptr ? 0 : c->tpf * c->nch;
 }
 
@@ -334,9 +305,9 @@ int sot_forward_sum_device(const sot_problem* prob, float* loss, double* loss_su
     r.args.loss = loss;
     r.args.loss_sum = loss_sum;
     if (coranks_out != nullptr) {
-        if (coranks_per_frame != sot_coranks_per_frame(prob->n_u, prob->n_v))
-            return fail(SOT_EINVAL, "coranks_per_frame = %d, this configuration needs %d", coranks_per_frame,
-                        sot_coranks_per_frame(prob->n_u, prob->n_v));
+        const int need = sot_coranks_per_frame(prob->n_u, prob->n_v);
+        if (coranks_per_frame != need)
+            return fail(SOT_EINVAL, "coranks_per_frame = %d, this configuration needs %d", coranks_per_frame, need);
         r.args.coranks_out = coranks_out;
     }
     return launch(prob, r, stream);
@@ -367,10 +338,7 @@ int sot_scale_rows_device(const float* unit, const float* scale, float* out, int
     if (blocks > 148LL * 8) blocks = 148LL * 8;
     sot::sot_scale_rows_kernel<<<static_cast<unsigned>(blocks), 256, 0, static_cast<cudaStream_t>(stream)>>>(
         unit, scale, out, rows, width);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "sot_scale_rows_kernel launch");
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return SOT_OK;
+    return sot::launched(cudaGetLastError(), "sot_scale_rows_kernel");
 }
 
 int sot_scale_inplace_device(float* rows_a, int64_t count_a, float* rows_b, int64_t count_b, const float* scale,
@@ -385,10 +353,7 @@ int sot_scale_inplace_device(float* rows_a, int64_t count_a, float* rows_b, int6
     if (blocks > 148LL * 8) blocks = 148LL * 8;
     sot::sot_scale_inplace_kernel<<<static_cast<unsigned>(blocks), 256, 0, static_cast<cudaStream_t>(stream)>>>(
         rows_a, rows_a != nullptr ? count_a : 0, rows_b, rows_b != nullptr ? count_b : 0, scale);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "sot_scale_inplace_kernel launch");
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return SOT_OK;
+    return sot::launched(cudaGetLastError(), "sot_scale_inplace_kernel");
 }
 
 int sot_mean_step_device(const sot_problem* prob, const sot_mean_plan* plan, float* loss, float* grad_u, float* grad_v,
@@ -433,10 +398,7 @@ int sot_quantile_lookup_device(const float* qs, const float* cws, const float* x
     if (blocks > 148LL * 16) blocks = 148LL * 16;
     sot::sot_quantile_lookup_kernel<<<static_cast<unsigned>(blocks), 256, 0, static_cast<cudaStream_t>(stream)>>>(
         qs, cws, xs, out, rows, n_levels, n_bins);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "sot_quantile_lookup_kernel launch");
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return SOT_OK;
+    return sot::launched(cudaGetLastError(), "sot_quantile_lookup_kernel");
 }
 
 int sot_quantiles_device(const sot_problem* prob, float* uq, float* vq, float* qs, float* cu, float* cv, int32_t* iu,
@@ -617,8 +579,9 @@ int sot_loss_grad_host(const sot_problem* hp, const float* upstream, float* loss
     // whose bulk loads and stores go over PCIe themselves -- no staging buffers, no fill and drain of a copy pipeline.
     // Anything else (pageable memory, per-frame supports) takes the chunked pipeline below.
     // (rows longer than shared memory holds: the split-frame path re-reads its rows, so they are staged on the device)
+    const int tuning = g_tuning.load();
     if (const char* zc = getenv("SOT_HOST_ZEROCOPY");
-        zc != nullptr && zc[0] == '1' && su && sv && !g_force_long.load() && pick_config(n, m) != nullptr) {
+        zc != nullptr && zc[0] == '1' && su && sv && tuning != kTuneLong && pick_config(tuning, n, m) != nullptr) {
         const float* du = mapped_device_pointer(hp->u);
         const float* dv = mapped_device_pointer(hp->v);
         const float* dup = mapped_device_pointer(upstream);

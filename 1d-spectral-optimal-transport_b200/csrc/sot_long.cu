@@ -20,8 +20,6 @@
 // Every reduction runs in a fixed order: two runs give the same bits.
 #include <cuda_runtime.h>
 
-#include <atomic>
-
 #include "sot_launch.cuh"
 
 namespace sot {
@@ -390,25 +388,14 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
 template <bool GRAD, bool RAW>
 cudaError_t launch_kind(const FrameArgs& a, cudaStream_t stream) {
     auto kernel = sot_long_kernel<GRAD, RAW>;
-    constexpr int kMaxDev = 64;  // resident CTAs of the chip, per device (see launch_one)
-    static std::atomic<int> resident_of_dev[kMaxDev];
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
+    static ResidentCache resident;
+    int resident_grid = 0;
+    cudaError_t e = resident_ctas(resident, kernel, TPB, 0, [] { return cudaSuccess; }, resident_grid);
     if (e != cudaSuccess) return e;
-    int resident = (dev >= 0 && dev < kMaxDev) ? resident_of_dev[dev].load(std::memory_order_acquire) : 0;
-    if (resident == 0) {
-        int per_sm = 0, sms = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, TPB, 0);
-        if (e != cudaSuccess) return e;
-        e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (e != cudaSuccess) return e;
-        resident = (per_sm < 1 ? 1 : per_sm) * sms;
-        if (dev >= 0 && dev < kMaxDev) resident_of_dev[dev].store(resident, std::memory_order_release);
-    }
     const long long slot_bytes = 4LL * slot_floats(a.n, a.m, GRAD);
     long long grid = kScratchBytes / slot_bytes;
     if (grid < 1) grid = 1;
-    if (grid > resident) grid = resident;
+    if (grid > resident_grid) grid = resident_grid;
     if (grid > a.n_frames) grid = a.n_frames;
     // stream-ordered scratch: no host synchronisation, several streams may run the path at once, and a CUDA graph
     // that captures the launch captures the allocation with it

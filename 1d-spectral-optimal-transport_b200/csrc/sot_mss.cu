@@ -11,6 +11,7 @@
 #include <cstdint>
 
 #include "../../include/sot_b200.h"
+#include "sot_internal.cuh"
 
 namespace sot {
 
@@ -139,40 +140,31 @@ int mss_grid(long long count) {
 
 extern "C" {
 
-int sot_mss_launch_count_add(void);  // (sot_capi.cu) counts the launch for sot_launch_count()
-int sot_mss_fail(int code, const char* msg);
-
 int sot_mss_forward_device(const float* zt, const float* zv, int64_t count, float mag_weight, float logmag_weight,
                            int32_t loss_type, float post_scale, double* sum_out, void* stream) {
     if (count < 0 || (count > 0 && (zt == nullptr || zv == nullptr)) || sum_out == nullptr)
-        return sot_mss_fail(SOT_EINVAL, "sot_mss_forward_device: NULL pointer or negative count");
+        return sot::fail(SOT_EINVAL, "sot_mss_forward_device: NULL pointer or negative count");
     if (loss_type != SOT_MSS_L1 && loss_type != SOT_MSS_L2)
-        return sot_mss_fail(SOT_EINVAL, "Loss type must be \"L1\" or \"L2\"");
+        return sot::fail(SOT_EINVAL, "Loss type must be \"L1\" or \"L2\"");
     if (count == 0) return SOT_OK;
     sot::MssArgs a{zt, zv, count, mag_weight, logmag_weight, loss_type == SOT_MSS_L2, post_scale, sum_out, nullptr,
                    nullptr, nullptr};
     sot::sot_mss_kernel<false><<<sot::mss_grid(count), 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return sot_mss_fail(static_cast<int>(e), cudaGetErrorString(e));
-    sot_mss_launch_count_add();
-    return SOT_OK;
+    return sot::launched(cudaGetLastError(), "sot_mss_kernel");
 }
 
 int sot_mss_backward_device(const float* zt, const float* zv, int64_t count, float mag_weight, float logmag_weight,
                             int32_t loss_type, float post_scale, const float* scale, float* grad_zt, float* grad_zv,
                             void* stream) {
     if (count < 0 || (count > 0 && (zt == nullptr || zv == nullptr)))
-        return sot_mss_fail(SOT_EINVAL, "sot_mss_backward_device: NULL pointer or negative count");
+        return sot::fail(SOT_EINVAL, "sot_mss_backward_device: NULL pointer or negative count");
     if (loss_type != SOT_MSS_L1 && loss_type != SOT_MSS_L2)
-        return sot_mss_fail(SOT_EINVAL, "Loss type must be \"L1\" or \"L2\"");
+        return sot::fail(SOT_EINVAL, "Loss type must be \"L1\" or \"L2\"");
     if (count == 0 || (grad_zt == nullptr && grad_zv == nullptr)) return SOT_OK;
     sot::MssArgs a{zt, zv, count, mag_weight, logmag_weight, loss_type == SOT_MSS_L2, post_scale, nullptr, scale,
                    grad_zt, grad_zv};
     sot::sot_mss_kernel<true><<<sot::mss_grid(count), 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return sot_mss_fail(static_cast<int>(e), cudaGetErrorString(e));
-    sot_mss_launch_count_add();
-    return SOT_OK;
+    return sot::launched(cudaGetLastError(), "sot_mss_kernel");
 }
 
 }  // extern "C"

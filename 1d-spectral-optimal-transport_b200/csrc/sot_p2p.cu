@@ -20,6 +20,7 @@
 #include <cstdlib>
 
 #include "../../include/sot_b200.h"
+#include "sot_internal.cuh"
 
 namespace sot {
 
@@ -125,9 +126,6 @@ __global__ void __launch_bounds__(32) sot_p2p_allreduce_kernel(const P2PArgs a) 
 
 extern "C" {
 
-int sot_mss_launch_count_add(void);
-int sot_mss_fail(int code, const char* msg);
-
 int sot_p2p_mailbox_doubles(int32_t world) { return world * sot::kP2PPhases * sot::kP2PSlot; }
 
 static int p2p_launch(sot::P2PArgs& a, void* const* mailboxes, int32_t world, int32_t rank, uint64_t seq, void* stream);
@@ -135,7 +133,7 @@ static int p2p_launch(sot::P2PArgs& a, void* const* mailboxes, int32_t world, in
 int sot_p2p_global_mean_device(const double* local_sum, double local_count, float* mean_out, float* inv_count_out,
                                void* const* mailboxes, int32_t world, int32_t rank, uint64_t seq, void* stream) {
     if (local_sum == nullptr || mean_out == nullptr || inv_count_out == nullptr || mailboxes == nullptr)
-        return sot_mss_fail(SOT_EINVAL, "sot_p2p_global_mean_device: NULL pointer");
+        return sot::fail(SOT_EINVAL, "sot_p2p_global_mean_device: NULL pointer");
     sot::P2PArgs a{};
     a.in = local_sum;
     a.local_count = local_count;
@@ -150,7 +148,7 @@ int sot_p2p_wait_mean_device(float* mean_out, double expected_count, int32_t* st
                              int32_t world, int32_t rank, uint64_t seq, uint64_t* seq_device, uint32_t timeout_ms,
                              void* stream) {
     if (mean_out == nullptr || mailboxes == nullptr)
-        return sot_mss_fail(SOT_EINVAL, "sot_p2p_wait_mean_device: NULL pointer");
+        return sot::fail(SOT_EINVAL, "sot_p2p_wait_mean_device: NULL pointer");
     sot::P2PArgs a{};
     a.mean_out = mean_out;
     a.count = 2;
@@ -166,9 +164,9 @@ int sot_p2p_wait_mean_device(float* mean_out, double expected_count, int32_t* st
 int sot_p2p_allreduce_device(const double* in, double* out, int32_t count, void* const* mailboxes, int32_t world,
                              int32_t rank, uint64_t seq, void* stream) {
     if (in == nullptr || out == nullptr || mailboxes == nullptr)
-        return sot_mss_fail(SOT_EINVAL, "sot_p2p_allreduce_device: NULL pointer");
+        return sot::fail(SOT_EINVAL, "sot_p2p_allreduce_device: NULL pointer");
     if (count < 1 || count > sot::kP2PMaxVals)
-        return sot_mss_fail(SOT_EINVAL, "sot_p2p_allreduce_device: bad count");
+        return sot::fail(SOT_EINVAL, "sot_p2p_allreduce_device: bad count");
     sot::P2PArgs a{};
     a.in = in;
     a.out = out;
@@ -181,9 +179,9 @@ static int p2p_launch(sot::P2PArgs& a, void* const* mailboxes, int32_t world, in
     const int32_t count = a.count;
     if (count < 1 || count > sot::kP2PMaxVals || world < 1 || world > sot::kP2PMaxWorld || rank < 0 || rank >= world ||
         seq == 0)
-        return sot_mss_fail(SOT_EINVAL, "sot_p2p_allreduce_device: bad count / world / rank / seq");
+        return sot::fail(SOT_EINVAL, "sot_p2p_allreduce_device: bad count / world / rank / seq");
     for (int r = 0; r < world; ++r) {
-        if (mailboxes[r] == nullptr) return sot_mss_fail(SOT_EINVAL, "sot_p2p_allreduce_device: NULL mailbox");
+        if (mailboxes[r] == nullptr) return sot::fail(SOT_EINVAL, "sot_p2p_allreduce_device: NULL mailbox");
         a.mailbox[r] = static_cast<double*>(mailboxes[r]);
     }
     a.world = world;
@@ -198,10 +196,7 @@ static int p2p_launch(sot::P2PArgs& a, void* const* mailboxes, int32_t world, in
         a.timeout_ns = 1000000ULL * ms;
     }
     sot::sot_p2p_allreduce_kernel<<<1, 32, 0, static_cast<cudaStream_t>(stream)>>>(a);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return sot_mss_fail(static_cast<int>(e), cudaGetErrorString(e));
-    sot_mss_launch_count_add();
-    return SOT_OK;
+    return sot::launched(cudaGetLastError(), "sot_p2p_allreduce_kernel");
 }
 
 }  // extern "C"

@@ -232,7 +232,7 @@ int sot_p2p_wait_mean_device(float* mean_out, double expected_count, int32_t* st
 
 /* Tuning override for benchmarking: threads per frame (32/64/128/256), bins per thread (odd) and
  * merge chains per thread (1/2, 0 = any); 0, 0, 0 restores the built-in choice.  Returns SOT_EINVAL
- * if that combination is not compiled in.  -1, 0, 0 routes every real-row loss / gradient request through the
+ * if no kernel configuration has that combination.  -1, 0, 0 routes every real-row loss / gradient request through the
  * split-frame path, whatever the row length (tests and benchmarks compare it with the shared-memory kernels). */
 int sot_set_tuning(int32_t threads_per_frame, int32_t bins_per_thread, int32_t chains_per_thread);
 /* Number of kernel launches issued by this library in the calling process so far. */

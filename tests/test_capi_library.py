@@ -63,8 +63,7 @@ def test_argument_validation_happens_before_any_launch():
     assert _capi.launch_count() == before
 
 
-def test_sass_contains_tma_bulk_copies():
-    """The hot kernels move rows with cp.async.bulk (SASS UBLKCP), not with per-thread loads."""
+def _cuobjdump(option):
     import shutil
     import subprocess
     from torch.utils.cpp_extension import CUDA_HOME
@@ -73,8 +72,29 @@ def test_sass_contains_tma_bulk_copies():
     tool = shutil.which("cuobjdump") or os.path.join(CUDA_HOME or "", "bin", "cuobjdump")
     if not os.path.isfile(tool):
         pytest.skip("cuobjdump not available")
-    sass = subprocess.run([tool, "-sass", _capi.library_path()], capture_output=True, text=True).stdout
+    return subprocess.run([tool, option, _capi.library_path()], capture_output=True, text=True).stdout
+
+
+def test_sass_contains_tma_bulk_copies():
+    """The hot kernels move rows with cp.async.bulk (SASS UBLKCP), not with per-thread loads."""
+    sass = _cuobjdump("-sass")
     assert "UBLKCP" in sass and "SYNCS" in sass
+
+
+def test_library_has_every_kernel_of_each_configuration_and_no_other():
+    """sot_frame_kernel instantiations per (threads per frame, bins per thread, row floats, chains, frames per CTA):
+    27 for a full configuration (10 real-spectra, 8 complex-input, 4 CDF-input, 3 raw-weight and 2 plan kernels),
+    10 for the sub-warp one (real spectra, loss and gradients)."""
+    names = re.findall(r"Function (_ZN3sot16sot_frame_kernelI\S+):", _cuobjdump("-res-usage"))
+    counts = {}
+    for name in names:
+        args = tuple(int(a) for a in re.findall(r"L[ib](\d+)E", name))
+        assert len(args) == 10, name
+        key = args[:4] + args[9:]
+        counts[key] = counts.get(key, 0) + 1
+    full = [(32, 9, 296, 1), (64, 9, 584, 2), (32, 33, 1064, 1), (64, 17, 1096, 1), (128, 9, 1160, 1),
+            (128, 17, 2184, 2), (256, 17, 4360, 2), (256, 33, 8456, 1)]
+    assert counts == {**{c + (1,): 27 for c in full}, (16, 17, 280, 1, 2): 10}
 
 
 def _build_c_demo(tmp_path):

@@ -14,7 +14,7 @@ import torch
 from . import build as _build
 
 SOT_SQUARE, SOT_CUT_SCALE, SOT_LIMIT, SOT_RAW_WEIGHTS, SOT_UNIFORM_GRID, SOT_COMPLEX_INPUT = 1, 2, 4, 8, 16, 32
-ABI_VERSION = 2
+ABI_VERSION = 3
 MAX_COMPLEX_BINS = 4352  # longest SOT_COMPLEX_INPUT row (include/sot_b200.h: sot_max_bins); real rows take 2^24 - 1
 
 _c_float_p = ctypes.c_void_p  # device pointers travel as integers
@@ -61,9 +61,6 @@ _V = ctypes.c_void_p
 SIGNATURES = {
     "sot_forward_device": (ctypes.c_int, [_P, _V, _V]),
     "sot_forward_backward_device": (ctypes.c_int, [_P, _V, _V, _V, _V, _V]),
-    "sot_forward_sum_device": (ctypes.c_int, [_P, _V, _V, _V, ctypes.c_int32, _V]),
-    "sot_forward_backward_scaled_device": (ctypes.c_int, [_P, _V, _V, _V, ctypes.c_int32, _V, _V, _V, _V]),
-    "sot_coranks_per_frame": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32]),
     "sot_scale_rows_device": (ctypes.c_int, [_V, _V, _V, ctypes.c_int64, ctypes.c_int32, _V]),
     "sot_mean_step_device": (ctypes.c_int, [_P, ctypes.POINTER(SotMeanPlan), _V, _V, _V, _V]),
     "sot_scale_inplace_device": (ctypes.c_int, [_V, ctypes.c_int64, _V, ctypes.c_int64, _V, _V]),
@@ -228,41 +225,6 @@ def forward_backward(u, v, pos_u, pos_v, p, flags, upstream=None, want_loss=True
         _check(lib.sot_forward_backward_device(ctypes.byref(prob), _ptr(upstream), _ptr(loss), _ptr(gu), _ptr(gv),
                                                _stream(u.device)))
     return loss, gu, gv
-
-
-def forward_sum(u, v, pos_u, pos_v, p, flags, want_rows=False, save_coranks=False):
-    """Sum over frames of the per-frame loss as a (1,) float64 device tensor, the rows if asked, and
-    (if asked) the merge-path co-ranks for the backward launch, an (N, chunks) int16 tensor."""
-    lib = load()
-    prob = make_problem(u, v, pos_u, pos_v, p, flags)
-    total = torch.zeros(1, dtype=torch.float64, device=u.device)
-    rows = torch.empty(u.shape[0], dtype=torch.float32, device=u.device) if want_rows else None
-    per_frame = lib.sot_coranks_per_frame(u.shape[1], v.shape[1]) if save_coranks else 0
-    coranks = torch.empty(u.shape[0], per_frame, dtype=torch.int16, device=u.device) if per_frame > 0 else None
-    with torch.cuda.device(u.device):
-        _check(lib.sot_forward_sum_device(ctypes.byref(prob), _ptr(rows), _ptr(total), _ptr(coranks), per_frame,
-                                          _stream(u.device)))
-    return total, rows, coranks
-
-
-def forward_backward_scaled(u, v, pos_u, pos_v, p, flags, scale, coranks=None, want_gu=True, want_gv=True):
-    """Gradients of scale * sum_n loss_n; `scale` is a (1,) float32 DEVICE tensor (no host sync);
-    `coranks` = what `forward_sum(..., save_coranks=True)` returned for the same inputs."""
-    lib = load()
-    prob = make_problem(u, v, pos_u, pos_v, p, flags)
-    _dev_tensor(scale, "scale")
-    if scale.numel() != 1:
-        raise ValueError("sot_b200: the upstream scale must hold one element")
-    if coranks is not None and (coranks.dtype != torch.int16 or not coranks.is_contiguous()
-                                or coranks.shape[0] != u.shape[0] or coranks.device != u.device):
-        raise ValueError("sot_b200: coranks must be the contiguous (N, chunks) int16 tensor of the forward launch")
-    gu = torch.empty_like(u) if want_gu else None
-    gv = torch.empty_like(v) if want_gv else None
-    with torch.cuda.device(u.device):
-        _check(lib.sot_forward_backward_scaled_device(ctypes.byref(prob), None, _ptr(scale), _ptr(coranks),
-                                                      0 if coranks is None else coranks.shape[1], None, _ptr(gu),
-                                                      _ptr(gv), _stream(u.device)))
-    return gu, gv
 
 
 _workspaces: dict = {}  # (device index, stream handle) -> 2 zeroed doubles the mean-step kernel keeps zero

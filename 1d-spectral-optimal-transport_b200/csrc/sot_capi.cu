@@ -132,7 +132,7 @@ int cuda_fail(cudaError_t e, const char* what) {
 }
 
 // `tuning`: a value of g_tuning.  `sub_ok`: the request is one the sub-warp configurations serve (see Config::sub).
-const Config* pick_config(int tuning, int n, int m, bool sub_ok = false) {
+const Config* pick_config(int tuning, int n, int m, bool sub_ok) {
     const int need = n > m ? n : m;
     if (tuning >= 0 && kConfigs[tuning].max_bins() >= need && (!kConfigs[tuning].sub || sub_ok))
         return &kConfigs[tuning];
@@ -186,8 +186,7 @@ int launch(const sot_problem* p, sot::LaunchRequest& r, void* stream) {
         return fail(SOT_EINVAL, "SOT_RAW_WEIGHTS rows are real weights, not complex spectra");
     if (p->n_frames == 0) return SOT_OK;
     const bool sub_ok = r.mode == sot::MODE_SPECTRA && r.out != sot::OUT_PLAN &&
-                        !(p->flags & (SOT_RAW_WEIGHTS | SOT_COMPLEX_INPUT)) && r.args.coranks_in == nullptr &&
-                        r.args.coranks_out == nullptr;
+                        !(p->flags & (SOT_RAW_WEIGHTS | SOT_COMPLEX_INPUT));
     // the split-frame path (global-memory scratch): real rows, loss and gradients
     const bool long_ok = r.mode == sot::MODE_SPECTRA && r.out != sot::OUT_PLAN && !(p->flags & SOT_COMPLEX_INPUT);
     const int tuning = g_tuning.load();
@@ -284,48 +283,6 @@ int sot_forward_backward_device(const sot_problem* prob, const float* upstream, 
     r.args.loss = loss;
     r.args.grad_u = grad_u;
     r.args.grad_v = grad_v;
-    return launch(prob, r, stream);
-}
-
-// One co-rank per merge chunk.  The chunk boundaries depend on the row lengths and on the NUMBER of chunks only
-// (L = ceil((n_u + n_v) / chunks) | 1, chunk c starts at merged slot c * L), not on how many bins a thread holds: two
-// configurations with the same threads x chains cut the merged grid identically, so co-ranks saved by one are valid
-// for the other -- the count is the whole compatibility condition.
-int sot_coranks_per_frame(int32_t n_u, int32_t n_v) {
-    const int tuning = g_tuning.load();
-    if (tuning == kTuneLong) return 0;  // (the split-frame path keeps no co-ranks)
-    const Config* c = pick_config(tuning, n_u, n_v);
-    return c == nullptr ? 0 : c->tpf * c->nch;
-}
-
-int sot_forward_sum_device(const sot_problem* prob, float* loss, double* loss_sum, uint16_t* coranks_out,
-                           int32_t coranks_per_frame, void* stream) {
-    if (int rc = validate(prob)) return rc;
-    sot::LaunchRequest r{base_args(prob), sot::OUT_LOSS, sot::MODE_SPECTRA};
-    r.args.loss = loss;
-    r.args.loss_sum = loss_sum;
-    if (coranks_out != nullptr) {
-        const int need = sot_coranks_per_frame(prob->n_u, prob->n_v);
-        if (coranks_per_frame != need)
-            return fail(SOT_EINVAL, "coranks_per_frame = %d, this configuration needs %d", coranks_per_frame, need);
-        r.args.coranks_out = coranks_out;
-    }
-    return launch(prob, r, stream);
-}
-
-int sot_forward_backward_scaled_device(const sot_problem* prob, const float* upstream, const float* upstream_scale,
-                                       const uint16_t* coranks_in, int32_t coranks_per_frame, float* loss,
-                                       float* grad_u, float* grad_v, void* stream) {
-    if (int rc = validate(prob)) return rc;
-    sot::LaunchRequest r{base_args(prob), sot::OUT_GRAD, sot::MODE_SPECTRA};
-    r.args.upstream = upstream;
-    r.args.upstream_scale = upstream_scale;
-    r.args.loss = loss;
-    r.args.grad_u = grad_u;
-    r.args.grad_v = grad_v;
-    // co-ranks saved by a launch of another configuration are useless: search again instead
-    if (coranks_in != nullptr && coranks_per_frame == sot_coranks_per_frame(prob->n_u, prob->n_v))
-        r.args.coranks_in = coranks_in;
     return launch(prob, r, stream);
 }
 
@@ -496,20 +453,6 @@ cudaError_t sync_positions(float** dev, size_t* cap, float** shadow, size_t* len
     return cudaMemcpyAsync(*dev, copy, 4 * n, cudaMemcpyHostToDevice, stream);
 }
 
-// Device address of a host buffer the GPU can reach directly (pinned by cudaHostAlloc / cudaHostRegister under unified
-// addressing), or nullptr: pageable memory, or a pointer the runtime does not know.
-template <typename T>
-T* mapped_device_pointer(T* host) {
-    if (host == nullptr) return nullptr;
-    cudaPointerAttributes attr;
-    if (cudaPointerGetAttributes(&attr, host) != cudaSuccess) {
-        cudaGetLastError();  // (older runtimes report unknown pointers as an error: clear it)
-        return nullptr;
-    }
-    if (attr.type != cudaMemoryTypeHost || attr.devicePointer == nullptr) return nullptr;
-    return static_cast<T*>(const_cast<void*>(static_cast<const void*>(attr.devicePointer)));
-}
-
 void release(HostWorkspace& w) {
     for (int k = 0; k < kSlots; ++k) {
         HostSlot& s = w.slot[k];
@@ -562,12 +505,7 @@ int sot_loss_grad_host(const sot_problem* hp, const float* upstream, float* loss
     if (N == 0) return SOT_OK;
     const int n = hp->n_u, m = hp->n_v;
     const bool want_grad = grad_u != nullptr || grad_v != nullptr;
-    long long chunk_bytes = 32LL << 20;  // ~32 MiB of input per chunk; SOT_HOST_CHUNK_MIB overrides (tuning)
-    if (const char* env = getenv("SOT_HOST_CHUNK_MIB")) {
-        const long long mib = atoll(env);
-        if (mib >= 1 && mib <= 4096) chunk_bytes = mib << 20;
-    }
-    long long chunk = chunk_bytes / (4LL * (n + m));
+    long long chunk = (32LL << 20) / (4LL * (n + m));  // ~32 MiB of input per chunk (4 to 64 MiB measured, DESIGN §5.3)
     chunk = (chunk / 4) * 4;
     if (chunk < 4) chunk = 4;
     if (chunk > N) chunk = ((N + 3) / 4) * 4;
@@ -575,47 +513,6 @@ int sot_loss_grad_host(const sot_problem* hp, const float* upstream, float* loss
 
     HostWorkspace& w = g_ws[device];
     int rc = SOT_OK;
-    // Zero-copy (SOT_HOST_ZEROCOPY=1; shared supports; every buffer pinned and mapped): ONE launch over the whole batch
-    // whose bulk loads and stores go over PCIe themselves -- no staging buffers, no fill and drain of a copy pipeline.
-    // Anything else (pageable memory, per-frame supports) takes the chunked pipeline below.
-    // (rows longer than shared memory holds: the split-frame path re-reads its rows, so they are staged on the device)
-    const int tuning = g_tuning.load();
-    if (const char* zc = getenv("SOT_HOST_ZEROCOPY");
-        zc != nullptr && zc[0] == '1' && su && sv && tuning != kTuneLong && pick_config(tuning, n, m) != nullptr) {
-        const float* du = mapped_device_pointer(hp->u);
-        const float* dv = mapped_device_pointer(hp->v);
-        const float* dup = mapped_device_pointer(upstream);
-        float* dl = mapped_device_pointer(loss);
-        float* dgu = mapped_device_pointer(grad_u);
-        float* dgv = mapped_device_pointer(grad_v);
-        const bool all_mapped = du != nullptr && dv != nullptr && (upstream == nullptr || dup != nullptr) &&
-                                (loss != nullptr && dl != nullptr) && (grad_u == nullptr || dgu != nullptr) &&
-                                (grad_v == nullptr || dgv != nullptr);
-        if (all_mapped) {
-            if (w.s_k == nullptr) {
-                e = cudaStreamCreateWithFlags(&w.s_k, cudaStreamNonBlocking);
-                if (e != cudaSuccess) return cuda_fail(e, "cudaStreamCreateWithFlags");
-            }
-            e = sync_positions(&w.d_pu, &w.cap_dpu, &w.h_pu, &w.len_pu, hp->pos_u, n, w.s_k);
-            if (e == cudaSuccess) e = sync_positions(&w.d_pv, &w.cap_dpv, &w.h_pv, &w.len_pv, hp->pos_v, m, w.s_k);
-            if (e != cudaSuccess) return cuda_fail(e, "sync_positions");
-            sot_problem dp = *hp;
-            dp.u = du;
-            dp.v = dv;
-            dp.pos_u = w.d_pu;
-            dp.pos_v = w.d_pv;
-            rc = want_grad ? sot_forward_backward_device(&dp, dup, dl, dgu, dgv, w.s_k) : sot_forward_device(&dp, dl, w.s_k);
-            e = cudaStreamSynchronize(w.s_k);
-            if (rc == SOT_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaStreamSynchronize");
-            return rc;
-        }
-    }
-    constexpr int kTraceChunks = 64;
-    const bool trace = getenv("SOT_HOST_TRACE") != nullptr;
-    cudaEvent_t tev[4 * kTraceChunks] = {};
-    long long n_traced = 0;
-    if (trace)
-        for (int k = 0; k < 4 * kTraceChunks; ++k) cudaEventCreate(&tev[k]);
 #define SOT_CK(call)                             \
     do {                                         \
         cudaError_t _e = (call);                 \
@@ -627,7 +524,7 @@ int sot_loss_grad_host(const sot_problem* hp, const float* upstream, float* loss
     {
         if (!w.ready) {
             if (w.s_in == nullptr) SOT_CK(cudaStreamCreateWithFlags(&w.s_in, cudaStreamNonBlocking));
-            if (w.s_k == nullptr) SOT_CK(cudaStreamCreateWithFlags(&w.s_k, cudaStreamNonBlocking));  // (zero-copy calls make it too)
+            if (w.s_k == nullptr) SOT_CK(cudaStreamCreateWithFlags(&w.s_k, cudaStreamNonBlocking));
             if (w.s_out == nullptr) SOT_CK(cudaStreamCreateWithFlags(&w.s_out, cudaStreamNonBlocking));
             for (int k = 0; k < kSlots; ++k) {
                 SOT_CK(cudaEventCreateWithFlags(&w.slot[k].in_done, cudaEventDisableTiming));
@@ -654,7 +551,6 @@ int sot_loss_grad_host(const sot_problem* hp, const float* upstream, float* loss
             HostSlot& s = w.slot[c % kSlots];
             const long long nf = (N - f0 < chunk) ? (N - f0) : chunk;
             if (c >= kSlots) SOT_CK(cudaStreamWaitEvent(w.s_in, s.out_done, 0));  // slot drained
-            if (trace && c < kTraceChunks) SOT_CK(cudaEventRecord(tev[4 * c + 0], w.s_in));
             SOT_CK(cudaMemcpyAsync(s.u, hp->u + f0 * n, 4ULL * nf * n, cudaMemcpyHostToDevice, w.s_in));
             SOT_CK(cudaMemcpyAsync(s.v, hp->v + f0 * m, 4ULL * nf * m, cudaMemcpyHostToDevice, w.s_in));
             if (upstream != nullptr)
@@ -666,7 +562,6 @@ int sot_loss_grad_host(const sot_problem* hp, const float* upstream, float* loss
                 SOT_CK(cudaMemcpy2DAsync(s.pv, 4ULL * m, hp->pos_v + f0 * hp->pos_v_stride, 4ULL * hp->pos_v_stride,
                                          4ULL * m, nf, cudaMemcpyHostToDevice, w.s_in));
             SOT_CK(cudaEventRecord(s.in_done, w.s_in));
-            if (trace && c < kTraceChunks) SOT_CK(cudaEventRecord(tev[4 * c + 1], w.s_in));
             SOT_CK(cudaStreamWaitEvent(w.s_k, s.in_done, 0));
             sot_problem dp = *hp;
             dp.n_frames = nf;
@@ -686,31 +581,19 @@ int sot_loss_grad_host(const sot_problem* hp, const float* upstream, float* loss
             }
             SOT_CK(cudaEventRecord(s.k_done, w.s_k));
             SOT_CK(cudaStreamWaitEvent(w.s_out, s.k_done, 0));
-            if (trace && c < kTraceChunks) SOT_CK(cudaEventRecord(tev[4 * c + 2], w.s_out));
             if (loss != nullptr) SOT_CK(cudaMemcpyAsync(loss + f0, s.loss, 4ULL * nf, cudaMemcpyDeviceToHost, w.s_out));
             if (grad_u != nullptr)
                 SOT_CK(cudaMemcpyAsync(grad_u + f0 * n, s.gu, 4ULL * nf * n, cudaMemcpyDeviceToHost, w.s_out));
             if (grad_v != nullptr)
                 SOT_CK(cudaMemcpyAsync(grad_v + f0 * m, s.gv, 4ULL * nf * m, cudaMemcpyDeviceToHost, w.s_out));
             SOT_CK(cudaEventRecord(s.out_done, w.s_out));
-            if (trace && c < kTraceChunks) SOT_CK(cudaEventRecord(tev[4 * c + 3], w.s_out));
         }
-        n_traced = c < kTraceChunks ? c : kTraceChunks;
     }
 done:
     // drain everything that was queued (also on the error path) before the host buffers are reused
     if (w.s_out) cudaStreamSynchronize(w.s_out);
     if (w.s_k) cudaStreamSynchronize(w.s_k);
     if (w.s_in) cudaStreamSynchronize(w.s_in);
-    if (trace) {  // SOT_HOST_TRACE=1: when each chunk's H2D / D2H copies started and ended (ms since the first copy)
-        for (long long k = 0; k < n_traced && rc == SOT_OK; ++k) {
-            float t[4] = {0, 0, 0, 0};
-            for (int j = 0; j < 4; ++j) cudaEventElapsedTime(&t[j], tev[0], tev[4 * k + j]);
-            fprintf(stderr, "sot_loss_grad_host chunk %lld: h2d %.3f..%.3f  d2h %.3f..%.3f ms\n", k, t[0], t[1], t[2], t[3]);
-        }
-        for (int k = 0; k < 4 * kTraceChunks; ++k)
-            if (tev[k]) cudaEventDestroy(tev[k]);
-    }
 #undef SOT_CK
     return rc;
 }

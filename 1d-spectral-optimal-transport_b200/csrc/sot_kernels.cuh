@@ -102,11 +102,6 @@ struct FrameArgs {
     unsigned long long post_seq;
     unsigned long long* post_seq_dev;  // nullable: the sequence number lives on the device (*post_seq_dev + 1, stored
                                        // back), so that a CUDA graph holding this launch can be replayed
-    // "saved merge indices": the merge-path co-rank (number of u entries before the chunk) of every
-    // chunk of every frame, [n_frames, NCH * TPF] uint16.  The forward launch can save them, the backward
-    // launch of the same configuration can reuse them instead of searching again (both nullable).
-    unsigned short* coranks_out;
-    const unsigned short* coranks_in;
     float* grad_u;          // [n_frames, n] or nullptr
     float* grad_v;          // [n_frames, m] or nullptr
     // OUT_PLAN outputs, each nullable: [n_frames, n+m] merged grid, un-clamped lower-bound indices
@@ -734,10 +729,6 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
         double base_mass_u = 0.0, base_mass_v = 0.0;  // sum of the (unnormalised) weights of the threads before me
         bool u_live = false, v_live = false;  // mass above the safe_divide floor -> carries gradient
         f32x2 x2[E];  // my (u, v) bin pairs (the gradient kernel needs them again at the end)
-        int saved_corank[NCH];                // (loaded early: the global-memory latency hides behind stage 2)
-#pragma unroll
-        for (int ch = 0; ch < NCH; ++ch)
-            saved_corank[ch] = args.coranks_in != nullptr ? min(static_cast<int>(args.coranks_in[frame * NCHUNK + NCH * tid + ch]), n) : 0;
         (void)inv_v;
         (void)base_mass_u;
         (void)base_mass_v;
@@ -939,11 +930,7 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
             a[ch] = pa[ch] = b[ch] = pb[ch] = qprev[ch] = 0.0f;
             i0[ch] = 0;
         }
-        if (finite && args.coranks_in != nullptr) {
-            // ---- stage 3a': the forward launch already found the co-ranks (same CDFs, bit for bit) ------
-#pragma unroll
-            for (int ch = 0; ch < NCH; ++ch) i0[ch] = saved_corank[ch];
-        } else if (finite) {
+        if (finite) {
             // ---- stage 3a: merge-path partition (fixed-trip, branch-free bit descent) ---------------
             // i0 = number of u entries among the first k0 merged slots (u first on equal values):
             // the largest i in [lo, hi] with A[i-1] <= B[k0-i].  The NCH searches are interleaved.
@@ -957,13 +944,6 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
             search_descent<SEARCH_TOP, NCH>(cur, hiA, sumAB);
 #pragma unroll
             for (int ch = 0; ch < NCH; ++ch) i0[ch] = static_cast<int>((cur[ch] - A0) >> 2);
-        }
-        if (finite) {
-            if (args.coranks_out != nullptr) {
-#pragma unroll
-                for (int ch = 0; ch < NCH; ++ch)
-                    args.coranks_out[frame * NCHUNK + NCH * tid + ch] = static_cast<unsigned short>(i0[ch]);
-            }
 #pragma unroll
             for (int ch = 0; ch < NCH; ++ch) {
                 adrA[ch] = A0 + 4u * i0[ch];

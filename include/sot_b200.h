@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define SOT_B200_ABI_VERSION 2
+#define SOT_B200_ABI_VERSION 3
 
 /* flags (bit-or) */
 #define SOT_SQUARE 1    /* square_dist=True: weights = magnitude^2        losses.py:172-174 */
@@ -80,23 +80,6 @@ int sot_forward_device(const sot_problem* prob, float* loss, void* stream);
  * losses.py:172-313 (SURVEY.md section 3.3); tie attribution = stable sort order. */
 int sot_forward_backward_device(const sot_problem* prob, const float* upstream, float* loss,
                                 float* grad_u, float* grad_v, void* stream);
-
-/* The reference ends with `torch.mean` over all frames (losses.py:211).  These two fold that mean
- * into the launches: the forward also accumulates *loss_sum += sum_n loss[n] (fp64, one atomic per
- * CTA; the caller zeroes it; `loss` may be NULL), and the backward takes the upstream gradient as
- * upstream[n] * (*upstream_scale) with both factors optional -- for a mean, upstream = NULL and
- * *upstream_scale = dL/dmean / N, a DEVICE scalar, so no host synchronisation is needed. */
-int sot_forward_sum_device(const sot_problem* prob, float* loss, double* loss_sum, uint16_t* coranks_out,
-                           int32_t coranks_per_frame, void* stream);
-int sot_forward_backward_scaled_device(const sot_problem* prob, const float* upstream,
-                                       const float* upstream_scale, const uint16_t* coranks_in,
-                                       int32_t coranks_per_frame, float* loss, float* grad_u, float* grad_v,
-                                       void* stream);
-/* "Saved merge indices": the forward launch can write the merge-path co-rank of every chunk of every
- * frame into coranks_out[n_frames, sot_coranks_per_frame(n_u, n_v)] (nullable) and the backward launch
- * reuse them (coranks_in, nullable) instead of repeating the search -- the CDFs of the two launches are
- * bit-identical.  Co-ranks from another kernel configuration (other count) are ignored. */
-int sot_coranks_per_frame(int32_t n_u, int32_t n_v);
 
 /* ---- the training step in ONE launch ---------------------------------------------------------------
  * What `loss = Wasserstein1D(...)(x, y, x_pos, y_pos); loss.backward()` needs (trainer.py:209-221, 233-238) is the
@@ -168,11 +151,7 @@ int sot_loss_from_cdf_device(const sot_problem* prob, float* loss, float* g_cu, 
  * streams, runs the fused kernel, copies loss and gradients back.  Blocking.  `upstream` and
  * each output are nullable host pointers.  Pinned host memory is used as-is; pageable memory
  * works but is slower.  `device` = CUDA ordinal.  Device staging buffers are cached per device
- * (see sot_host_release); concurrent calls are serialised.
- * SOT_HOST_ZEROCOPY=1 in the environment: when every buffer is pinned and mapped (cudaHostAlloc /
- * cudaHostRegister) and the supports are shared rows, ONE launch reads the spectra from and writes loss and
- * gradients to host memory itself -- no staging buffers on the device; measured at the same PCIe-bound rate
- * as the copy pipeline (4.54 vs 4.64 M frames/s), hence opt-in.  Anything else falls back to the pipeline. */
+ * (see sot_host_release); concurrent calls are serialised. */
 int sot_loss_grad_host(const sot_problem* host_prob, const float* upstream, float* loss, float* grad_u,
                        float* grad_v, int32_t device);
 
@@ -185,9 +164,8 @@ const char* sot_last_error(void);
 /* Largest row length (max(n_u, n_v)) the loss / gradient entry points accept: 2^24 - 1.  Real rows longer than one
  * CTA's shared memory holds (more than 8448 bins) run on the split-frame path (global-memory scratch, allocated
  * stream-ordered on the call's stream: no host synchronisation, capturable in a CUDA graph), which needs u, v and the
- * positions in memory the device can reach (else SOT_ETOOBIG); co-ranks are not kept for them (sot_coranks_per_frame
- * returns 0).  Shared memory bounds the rest: sot_quantiles_device and the CDF
- * harness take up to 8448 bins, SOT_COMPLEX_INPUT rows up to 4352; longer rows there return SOT_ETOOBIG. */
+ * positions in memory the device can reach (else SOT_ETOOBIG).  Shared memory bounds the rest: sot_quantiles_device
+ * and the CDF harness take up to 8448 bins, SOT_COMPLEX_INPUT rows up to 4352; longer rows there return SOT_ETOOBIG. */
 int sot_max_bins(int32_t with_grad, int32_t shared_positions);
 /* ---- Multi-scale spectral loss term (row f3; losses.py:365-425 `MSSLoss`, :7-36 `mean_difference`,
  * utils.py:145-151 `safe_log`) for ONE fft size, straight from the two complex64 spectrograms zt (target) and zv

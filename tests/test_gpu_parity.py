@@ -388,29 +388,18 @@ def test_fused_mean_path_matches_the_per_frame_path(capi, L):
     assert capi.launch_count() - before == 1 and abs(v3.item() - v2.item()) <= 1e-6 * abs(v2.item())
 
 
-def test_saved_merge_indices_give_bit_identical_gradients(capi):
+def test_launch_total_is_the_fp64_sum_of_the_rows(capi):
+    """The fp64 total of a mean-step launch, loss-only or with gradients, is the fp64 sum of its per-frame losses."""
     g = G.load("sot2048_cut")
     F = 1025
     x, y = g["x"].reshape(-1, F).to(DEV), g["y"].reshape(-1, F).to(DEV)
     pos = g["pos_x"].to(DEV)
-    scale = torch.full((1,), 0.125, device=DEV)
     for flags in (capi.SOT_SQUARE, capi.SOT_SQUARE | capi.SOT_CUT_SCALE | capi.SOT_LIMIT | capi.SOT_UNIFORM_GRID):
-        total, rows, coranks = capi.forward_sum(x, y, pos, pos, 2.0, flags, want_rows=True, save_coranks=True)
-        assert coranks.shape == (x.shape[0], capi.load().sot_coranks_per_frame(F, F)) and coranks.dtype == torch.int16
-        assert (coranks >= 0).all() and (coranks <= F).all() and (coranks[:, 0] == 0).all()
-        assert (coranks[:, 1:] >= coranks[:, :-1]).all(), "co-ranks are non-decreasing along the merge path"
-        assert total.item() == pytest.approx(rows.double().sum().item(), rel=1e-12)
-        a = capi.forward_backward_scaled(x, y, pos, pos, 2.0, flags, scale, coranks=coranks)
-        b = capi.forward_backward_scaled(x, y, pos, pos, 2.0, flags, scale, coranks=None)
-        assert torch.equal(a[0], b[0]) and torch.equal(a[1], b[1])
-        # co-ranks of another configuration are ignored, not misused
-        capi.set_tuning(128, 9, 1)
-        try:
-            c = capi.forward_backward_scaled(x, y, pos, pos, 2.0, flags, scale, coranks=coranks)
-        finally:
-            capi.set_tuning(0, 0, 0)
-        # (another configuration sums other groups of bins: CDFs a few ulp apart, see the conditioning note)
-        assert (c[0] - b[0]).norm() <= 1e-3 * b[0].norm()
+        for grads in (False, True):
+            t = torch.zeros(2, dtype=torch.float64, device=DEV)
+            _, rows, _, _ = capi.mean_step(x, y, pos, pos, 2.0, flags, 1.0, 1.0, want_gu=grads, want_gv=grads,
+                                           want_rows=True, total_out=t)
+            assert t[0].item() == pytest.approx(rows.double().sum().item(), rel=1e-12), (flags, grads)
 
 
 def test_fused_and_recompute_modes_agree_bitwise(L):
@@ -864,39 +853,34 @@ def test_gradients_wrt_support_positions_match_reference_autograd(L, case):
 
 
 def test_host_buffer_entry_point_matches_device_path(capi):
-    g = G.load("sot2048_cut")
-    F = 1025
-    x = g["x"].reshape(-1, F).repeat(5, 1)[:37].contiguous().pin_memory()
-    y = g["y"].reshape(-1, F).repeat(5, 1)[:37].contiguous().pin_memory()
-    pos = g["pos_x"].contiguous()
-    flags = capi.SOT_SQUARE | capi.SOT_CUT_SCALE | capi.SOT_LIMIT
-    up = torch.rand(37)
-    loss, gu, gv = capi.loss_grad_host(x, y, pos, pos, 2.0, flags, upstream=up)
-    d = capi.forward_backward(x.to(DEV), y.to(DEV), pos.to(DEV), pos.to(DEV), 2.0, flags, upstream=up.to(DEV))
-    torch.cuda.synchronize()
-    assert torch.equal(loss, d[0].cpu()) and torch.equal(gu, d[1].cpu()) and torch.equal(gv, d[2].cpu())
+    """The copy pipeline of the host-buffer entry point gives the numbers of the device path, bit for bit, into
+    pinned and into pageable outputs.  The random shapes run on the 32x33, sub-warp 16x17 and 64x9 configurations."""
+    def inputs(case):
+        if case == "sot2048_cut":
+            g = G.load("sot2048_cut")
+            F = 1025
+            x = g["x"].reshape(-1, F).repeat(5, 1)[:37].contiguous().pin_memory()
+            y = g["y"].reshape(-1, F).repeat(5, 1)[:37].contiguous().pin_memory()
+            return x, y, g["pos_x"].contiguous(), torch.rand(37)
+        n_frames, n_bins = case
+        gen = torch.Generator().manual_seed(n_frames)
+        x = torch.rand(n_frames, n_bins, generator=gen).pin_memory()
+        y = torch.rand(n_frames, n_bins, generator=gen).pin_memory()
+        return x, y, torch.linspace(0, 1, n_bins), torch.rand(n_frames, generator=gen).pin_memory()
 
-
-@pytest.mark.parametrize("n_frames,n_bins", [(37, 1025), (300, 257), (5, 513)])
-def test_host_buffer_entry_point_zero_copy_matches_device_path(capi, monkeypatch, n_frames, n_bins):
-    """SOT_HOST_ZEROCOPY=1 with every buffer pinned: the kernels read the spectra from and write loss and gradients to
-    host memory themselves (one launch, no staging copies).  Same numbers as the device path, bit for bit; with a
-    pageable buffer among them the call falls back to the copy pipeline (same numbers again)."""
-    gen = torch.Generator().manual_seed(n_frames)
-    x = torch.rand(n_frames, n_bins, generator=gen).pin_memory()
-    y = torch.rand(n_frames, n_bins, generator=gen).pin_memory()
-    pos = torch.linspace(0, 1, n_bins)
     flags = capi.SOT_SQUARE | capi.SOT_CUT_SCALE | capi.SOT_LIMIT
-    up = torch.rand(n_frames, generator=gen).pin_memory()
-    d = capi.forward_backward(x.to(DEV), y.to(DEV), pos.to(DEV), pos.to(DEV), 2.0, flags, upstream=up.to(DEV))
-    torch.cuda.synchronize()
-    monkeypatch.setenv("SOT_HOST_ZEROCOPY", "1")
-    for pinned_out in (True, False):
-        out = {"loss": torch.full((n_frames,), -1.0), "grad_u": torch.full_like(x, -1.0), "grad_v": torch.full_like(y, -1.0)}
-        if pinned_out:
-            out = {k: v.pin_memory() for k, v in out.items()}
-        loss, gu, gv = capi.loss_grad_host(x, y, pos, pos, 2.0, flags, upstream=up, out=out)
-        assert torch.equal(loss, d[0].cpu()) and torch.equal(gu, d[1].cpu()) and torch.equal(gv, d[2].cpu()), pinned_out
+    for case in ("sot2048_cut", (37, 1025), (300, 257), (5, 513)):
+        x, y, pos, up = inputs(case)
+        d = capi.forward_backward(x.to(DEV), y.to(DEV), pos.to(DEV), pos.to(DEV), 2.0, flags, upstream=up.to(DEV))
+        torch.cuda.synchronize()
+        for pinned_out in (True, False):
+            out = {"loss": torch.full((x.shape[0],), -1.0), "grad_u": torch.full_like(x, -1.0),
+                   "grad_v": torch.full_like(y, -1.0)}
+            if pinned_out:
+                out = {k: v.pin_memory() for k, v in out.items()}
+            loss, gu, gv = capi.loss_grad_host(x, y, pos, pos, 2.0, flags, upstream=up, out=out)
+            assert torch.equal(loss, d[0].cpu()) and torch.equal(gu, d[1].cpu()) and torch.equal(gv, d[2].cpu()), \
+                (case, pinned_out)
 
 
 @pytest.mark.parametrize("n_bins", [257, 1025, 2049])

@@ -50,15 +50,6 @@
 namespace sot {
 
 enum : int {
-    FLAG_SQUARE = 1,     // square_dist          losses.py:172-174
-    FLAG_CUT_SCALE = 2,  // dont_normalize       losses.py:180-182
-    FLAG_LIMIT = 4,      // limit_quantile_range losses.py:306-307
-    FLAG_RAW = 8,        // rows are weights used as given (module-level wasserstein_1d, :223-313)
-    FLAG_UNIFORM = 16,   // caller asserts: shared supports with pos[i] = pos[0] + i*h EXACTLY in fp32
-    FLAG_COMPLEX = 32,   // u, v (and the gradients) are interleaved complex64 STFT rows: |z| is fused in
-};
-
-enum : int {
     MODE_SPECTRA = 0,  // inputs are magnitudes: full prologue
     MODE_RAW = 2,      // inputs are weights used as given (FLAG_RAW): no normalisation, CDF = cumsum with fp64
                        // accumulation exactly like the reference's (see stage 2)
@@ -72,59 +63,6 @@ enum : int {
     OUT_PLAN = 2,  // loss + the transport plan: qs, searchsorted indices, quantiles, CDFs
                    // (`return_quantiles=True`, losses.py:198-201, 299-300; also the parity harness)
 };
-
-struct FrameArgs {
-    const float* u;  // [n_frames, n]  target spectra (or CDF rows)
-    const float* v;  // [n_frames, m]  prediction spectra (or CDF rows)
-    const float* pos_u;
-    const float* pos_v;
-    long long pos_u_stride;  // 0: one shared support row; else elements between per-frame rows
-    long long pos_v_stride;
-    const float* upstream;        // [n_frames] dL_total/dloss_n, or nullptr (= 1)
-    const float* upstream_scale;  // device scalar multiplying every upstream value, or nullptr (= 1)
-    float upstream_value;         // host constant multiplying every upstream value (1 when unused)
-    float* loss;                  // [n_frames] or nullptr
-    double* loss_sum;             // device scalar: += sum of the per-frame losses of this launch, or nullptr
-    // Mean of the launch finished by its LAST CTA (the reference's closing `torch.mean`, losses.py:211, without
-    // a memset, a division or a cast kernel around the launch).  `ticket` (nullable; zero before the launch)
-    // counts the CTAs that have added their part to *loss_sum; the last one reads the total, writes
-    //   *mean_out = (float)(total * mean_scale)          (nullable)
-    //   total_out[0] = total, total_out[1] = post_count  (nullable; what an NCCL all-reduce of the shards sums)
-    //   (total, post_count, post_seq) into the mailbox of every peer (post_world > 0; layout of sot_p2p.cu)
-    // and leaves *loss_sum = 0, *ticket = 0 for the next launch on the same workspace.
-    unsigned int* ticket;
-    float* mean_out;
-    double mean_scale;
-    double* total_out;
-    double post_count;
-    double* post_mailbox[16];
-    int post_world, post_rank;
-    unsigned long long post_seq;
-    unsigned long long* post_seq_dev;  // nullable: the sequence number lives on the device (*post_seq_dev + 1, stored
-                                       // back), so that a CUDA graph holding this launch can be replayed
-    float* grad_u;          // [n_frames, n] or nullptr
-    float* grad_v;          // [n_frames, m] or nullptr
-    // OUT_PLAN outputs, each nullable: [n_frames, n+m] merged grid, un-clamped lower-bound indices
-    // and the quantile positions; [n_frames, n] / [n_frames, m] CDF rows
-    float* plan_qs;
-    int* plan_iu;
-    int* plan_iv;
-    float* plan_uq;
-    float* plan_vq;
-    float* plan_cu;
-    float* plan_cv;
-    long long n_frames;
-    int n, m;
-    float p;
-    int flags;
-    // 1.0f and -0.0f as RUN-TIME values (set by the launcher): x * one + neg_zero == x exactly, and because
-    // ptxas cannot fold it, a predicated FFMA (fma pipe, two warp-instructions per clock pair) can stand in
-    // for an FSEL (alu pipe, half that rate) in the merge walk, which is bound by the alu pipe
-    float one, neg_zero, one_b, neg_zero_b;  // (two copies: identical expressions would be merged and re-selected)
-};
-
-SOT_DEVINL float f_inf() { return __int_as_float(0x7f800000); }
-SOT_DEVINL float f_nan() { return __int_as_float(0x7fc00000); }
 
 // ---- compile-time shared-memory layout ---------------------------------------------------------
 template <int TPF, int RS, int OUT, int NCH, bool UNI, bool CPLX>
@@ -181,16 +119,6 @@ SOT_DEVINL void lds64(uint32_t a, float& x, float& y) {
 SOT_DEVINL void sts64(uint32_t a, float x, float y) {
     asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(a), "f"(x), "f"(y) : "memory");
 }
-// ---- packed fp32x2 arithmetic (sm_100: FADD2 / FMUL2 / FFMA2, two lanes per issued instruction).
-// The kernel is bound by instruction issue, so everything that is elementwise on (u, v) bin pairs
-// -- squares, local prefix sums, CDF scaling, the gradient chain rule -- runs on pairs.
-using f32x2 = unsigned long long;
-SOT_DEVINL f32x2 pack2(float lo, float hi) {
-    f32x2 r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-    return r;
-}
-SOT_DEVINL void unpack2(f32x2 v, float& lo, float& hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v)); }
 // (lo, hi) = (shared[a], shared[b]): the loads define the two halves of the pair directly
 SOT_DEVINL f32x2 lds32x2(uint32_t a, uint32_t b) {
     f32x2 r;
@@ -208,22 +136,6 @@ SOT_DEVINL f32x2 mask2(f32x2 v, bool keep_lo, bool keep_hi) {
         : "l"(v), "r"(static_cast<int>(keep_lo)), "r"(static_cast<int>(keep_hi)));
     return r;
 }
-SOT_DEVINL f32x2 add2(f32x2 a, f32x2 b) {
-    f32x2 r;
-    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-SOT_DEVINL f32x2 mul2(f32x2 a, f32x2 b) {
-    f32x2 r;
-    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-SOT_DEVINL f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) {
-    f32x2 r;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-    return r;
-}
-
 // One merge step's advance: the consumed side (v if b < a, else u: u first on equal values, the
 // stable order of `cat(cu, cv)`) gets its next CDF entry and that entry's position.  ONE load per
 // array from the SELECTED address: a pair of predicated loads (one per side, half the lanes each)
@@ -300,158 +212,12 @@ SOT_DEVINL void search_descent(uint32_t (&cur)[NCH], const uint32_t (&hi)[NCH], 
     if constexpr (STEP > 1) search_descent<STEP / 2, NCH>(cur, hi, sum);
 }
 
-// fp64 reciprocal of a positive float >= 1e-7: hardware approximation + two Newton steps
-SOT_DEVINL double recip_f64(float x) {
-    const double xd = static_cast<double>(x);
-    double r = static_cast<double>(__fdividef(1.0f, x));
-    r = fma(r, fma(-xd, r, 1.0), r);
-    r = fma(r, fma(-xd, r, 1.0), r);
-    return r;
-}
-
 template <int TPF>
 SOT_DEVINL void cta_sync() {
     if constexpr (TPF <= 32) {  // one warp per CTA (TPF < 32: sub-warp frames, several frames in the warp)
         __syncwarp();
     } else {
         __syncthreads();
-    }
-}
-
-// One Hillis-Steele step of a warp scan of an fp64 value that is carried as an EXCLUSIVE scan: the lane at the
-// edge (lane 0; lane 31 when REVERSE) holds 0.0 from start to end, so a lane whose partner would lie outside the
-// warp reads that lane instead (`src` = clamped partner lane) and adds 0.0 -- an unconditional add.  (A predicated
-// fp64 add costs DADD + 2 FSEL + moves after ptxas; `__shfl_up_sync(double)` three times as much.)
-SOT_DEVINL void scan_step(double& v, int src) {
-    asm volatile(
-        "{\n .reg .b32 lo, hi, ylo, yhi;\n .reg .f64 y;\n"
-        " mov.b64 {lo, hi}, %0;\n"
-        " shfl.sync.idx.b32 ylo, lo, %1, 0x1f, 0xffffffff;\n"
-        " shfl.sync.idx.b32 yhi, hi, %1, 0x1f, 0xffffffff;\n"
-        " mov.b64 y, {ylo, yhi};\n"
-        " add.f64 %0, %0, y;\n}"
-        : "+d"(v)
-        : "r"(src));
-}
-// Exclusive scans (prefix; suffix when REVERSE) over the TPF threads of the CTA of two fp32 values, carried
-// in fp64.  ta, tb: my values; returns my exclusive offsets and the CTA totals.  One CTA barrier when the
-// CTA has more than one warp; `slot` holds 2 * NW doubles.
-// nxt_a / nxt_b = the exclusive offset of the NEXT thread (the CTA total for the last one), bitwise: the
-// CDF stage caps my entries with it.
-template <int TPF, bool REVERSE, bool WANT_NEXT>
-SOT_DEVINL void cta_scan2(float ta, float tb, double& off_a, double& off_b, double& nxt_a, double& nxt_b,
-                          double& total_a, double& total_b, double* slot, int tid) {
-    // TPF < 32 (sub-warp frames: several frames share a warp, each in its own group of TPF lanes): the scan runs
-    // inside the group -- `lane` is the position in the group, `base` the warp lane the group starts at.
-    constexpr int W = TPF < 32 ? TPF : 32;
-    constexpr int NW = (TPF + 31) / 32;
-    const int lane = tid & (W - 1), w = tid >> 5;
-    const int base = static_cast<int>(threadIdx.x & 31u) - lane;
-    const int edge = REVERSE ? W - 1 : 0;  // the lane with nothing before it
-    // shift by one lane first: the inclusive scan of the shifted values is the exclusive scan
-    float sa = REVERSE ? __shfl_down_sync(FULL_MASK, ta, 1) : __shfl_up_sync(FULL_MASK, ta, 1);
-    float sb = REVERSE ? __shfl_down_sync(FULL_MASK, tb, 1) : __shfl_up_sync(FULL_MASK, tb, 1);
-    double ea = lane == edge ? 0.0 : static_cast<double>(sa);
-    double eb = lane == edge ? 0.0 : static_cast<double>(sb);
-#pragma unroll
-    for (int off = 1; off < W; off <<= 1) {
-        const int src = base + (REVERSE ? min(lane + off, W - 1) : max(lane - off, 0));
-        scan_step(ea, src);
-        scan_step(eb, src);
-    }
-    // warp totals, formed on the last lane of the scan direction
-    const double wa_mine = ea + static_cast<double>(ta), wb_mine = eb + static_cast<double>(tb);
-    if constexpr (NW == 1) {
-        off_a = ea;
-        off_b = eb;
-        total_a = __shfl_sync(FULL_MASK, wa_mine, base + W - 1 - edge);
-        total_b = __shfl_sync(FULL_MASK, wb_mine, base + W - 1 - edge);
-        if constexpr (WANT_NEXT) {
-            const double na = REVERSE ? __shfl_up_sync(FULL_MASK, ea, 1) : __shfl_down_sync(FULL_MASK, ea, 1);
-            const double nb = REVERSE ? __shfl_up_sync(FULL_MASK, eb, 1) : __shfl_down_sync(FULL_MASK, eb, 1);
-            nxt_a = lane == W - 1 - edge ? total_a : na;
-            nxt_b = lane == W - 1 - edge ? total_b : nb;
-        }
-    } else {
-        if (lane == 31 - edge) {
-            slot[w] = wa_mine;
-            slot[NW + w] = wb_mine;
-        }
-        __syncthreads();
-        double pa = 0.0, pb = 0.0, qa = 0.0, qb = 0.0, xa = 0.0, xb = 0.0;  // prefix before my warp, through my warp, total
-#pragma unroll
-        for (int k = 0; k < NW; ++k) {
-            const int kk = REVERSE ? (NW - 1 - k) : k;
-            const double va = slot[kk], vb = slot[NW + kk];
-            if (REVERSE ? (kk > w) : (kk < w)) {
-                pa = xa + va;
-                pb = xb + vb;
-            }
-            xa += va;
-            xb += vb;
-            if (kk == w) {
-                qa = xa;
-                qb = xb;
-            }
-        }
-        off_a = pa + ea;
-        off_b = pb + eb;
-        total_a = xa;
-        total_b = xb;
-        if constexpr (WANT_NEXT) {
-            // next thread in my warp: its offset is pa + (its ea), the same addition it performs itself; across
-            // the warp boundary: the next warp's pa is exactly qa (same sequence of additions), plus its ea = 0
-            const double na = REVERSE ? __shfl_up_sync(FULL_MASK, off_a, 1) : __shfl_down_sync(FULL_MASK, off_a, 1);
-            const double nb = REVERSE ? __shfl_up_sync(FULL_MASK, off_b, 1) : __shfl_down_sync(FULL_MASK, off_b, 1);
-            nxt_a = lane == 31 - edge ? qa : na;
-            nxt_b = lane == 31 - edge ? qb : nb;
-        }
-    }
-}
-
-// The same for two fp64 values (raw-weights mode, not a hot path): a, b in = my value, out = exclusive offset.
-template <int TPF>
-SOT_DEVINL void cta_scan2d(double& a, double& b, double& total_a, double& total_b, double* slot, int tid) {
-    constexpr int NW = TPF / 32;
-    const int lane = tid & 31, w = tid >> 5;
-    double ia = a, ib = b;
-#pragma unroll
-    for (int off = 1; off < 32; off <<= 1) {
-        const double ya = __shfl_up_sync(FULL_MASK, ia, off), yb = __shfl_up_sync(FULL_MASK, ib, off);
-        if (lane >= off) {
-            ia += ya;
-            ib += yb;
-        }
-    }
-    double ea = __shfl_up_sync(FULL_MASK, ia, 1), eb = __shfl_up_sync(FULL_MASK, ib, 1);
-    if (lane == 0) ea = eb = 0.0;
-    const double wa = __shfl_sync(FULL_MASK, ia, 31), wb = __shfl_sync(FULL_MASK, ib, 31);
-    if constexpr (NW == 1) {
-        a = ea;
-        b = eb;
-        total_a = wa;
-        total_b = wb;
-    } else {
-        if (lane == 0) {
-            slot[w] = wa;
-            slot[NW + w] = wb;
-        }
-        __syncthreads();
-        double pa = 0.0, xa = 0.0, pb = 0.0, xb = 0.0;
-#pragma unroll
-        for (int k = 0; k < NW; ++k) {
-            const double va = slot[k], vb = slot[NW + k];
-            if (k < w) {
-                pa = xa + va;
-                pb = xb + vb;
-            }
-            xa += va;
-            xb += vb;
-        }
-        a = pa + ea;
-        b = pb + eb;
-        total_a = xa;
-        total_b = xb;
     }
 }
 
@@ -504,44 +270,6 @@ SOT_DEVINL bool row_is_bulk(const float* base, long long f, int width, long long
 
 template <int N>
 using IC = std::integral_constant<int, N>;
-
-// Called by one thread per CTA after its atomicAdd into *loss_sum: the CTA that draws the last ticket owns the
-// total (every other CTA's add is ordered before its ticket by the fence) and finishes the mean -- see FrameArgs.
-// Mailbox layout = sot_p2p.cu: slot [rank][phase = seq & 7] of kP2PSlot = 9 doubles, entry [8] = sequence number.
-SOT_DEVINL void finish_mean(const FrameArgs& args) {
-    __threadfence();
-    if (atomicAdd(args.ticket, 1u) != gridDim.x - 1) return;
-    __threadfence();
-    const double total = __longlong_as_double(static_cast<long long>(
-        atomicExch(reinterpret_cast<unsigned long long*>(args.loss_sum), 0ULL)));
-    *args.ticket = 0;
-    if (args.mean_out != nullptr) *args.mean_out = static_cast<float>(total * args.mean_scale);
-    if (args.total_out != nullptr) {
-        args.total_out[0] = total;
-        args.total_out[1] = args.post_count;
-    }
-    if (args.post_world > 0) {
-        unsigned long long seq = args.post_seq;
-        if (args.post_seq_dev != nullptr) {
-            seq = *args.post_seq_dev + 1ULL;
-            *args.post_seq_dev = seq;
-        }
-        const int phase = static_cast<int>(seq & 7ULL);
-        for (int r = 0; r < args.post_world; ++r) {
-            double* dst = args.post_mailbox[r] + (static_cast<long long>(args.post_rank) * 8 + phase) * 9;
-            asm volatile("st.relaxed.sys.global.f64 [%0], %1;" ::"l"(dst), "d"(total) : "memory");
-            asm volatile("st.relaxed.sys.global.f64 [%0], %1;" ::"l"(dst + 1), "d"(args.post_count) : "memory");
-        }
-        // ONE system-scope fence between the values and the sequence numbers of all peers (a release store per peer
-        // is a fence per peer: measured 21 us per step at 8 GPUs against 10 us at 2), then plain stores
-        __threadfence_system();
-        const double seq_val = static_cast<double>(seq);
-        for (int r = 0; r < args.post_world; ++r) {
-            double* dst = args.post_mailbox[r] + (static_cast<long long>(args.post_rank) * 8 + phase) * 9;
-            asm volatile("st.relaxed.sys.global.f64 [%0], %1;" ::"l"(dst + 8), "d"(seq_val) : "memory");
-        }
-    }
-}
 
 // FPW > 1 ("sub-warp frames", short rows): TPF < 32 threads per frame and FPW = 32 / TPF frames per CTA, each frame in
 // its own group of TPF lanes of the one warp with its own block of shared memory, mbarrier and bulk copies.  Every
@@ -725,15 +453,11 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
 
         float acc[NCH] = {};  // my part of the frame's loss
         bool finite = true;  // masses (and the scaled totals) are finite numbers
-        double inv_u = 1.0, inv_v = 1.0;
+        Norm nm{1.0, 1.0, false, false};
         double base_mass_u = 0.0, base_mass_v = 0.0;  // sum of the (unnormalised) weights of the threads before me
-        bool u_live = false, v_live = false;  // mass above the safe_divide floor -> carries gradient
         f32x2 x2[E];  // my (u, v) bin pairs (the gradient kernel needs them again at the end)
-        (void)inv_v;
         (void)base_mass_u;
         (void)base_mass_v;
-        (void)u_live;
-        (void)v_live;
 
         // ---- stages 1 + 2: blocked read of my E bins (conflict free: E is odd), masses and CDFs
         //      (fp64 accumulation, one rounding to fp32 per entry) ---------------------------------------
@@ -772,40 +496,27 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
             }
             (void)inside;
             const bool sq = square && !CPLX;
-            // Weights used as given (module-level `wasserstein_1d`, kernel mode MODE_RAW): the CDF is a plain
-            // cumsum, which the reference accumulates in fp64 -- reproduced exactly, because with a handful of
-            // atoms the strict `qs > 1` mask decides over a whole atom on the last ulp of the CDF.  Normalised
-            // spectra (every `Wasserstein1D` call) take the packed fp32 route: a few ulp, at a third of the
-            // instructions.
+            // Normalised spectra (every `Wasserstein1D` call) take the packed fp32 route: a few ulp, at a third of the
+            // instructions of the fp64 cumsum of raw weights (module-level `wasserstein_1d`, kernel mode MODE_RAW).
             constexpr bool exact = (MODE == MODE_RAW);
-            constexpr int NSEG = E >= 25 ? 4 : 1;  // segments of a thread's local prefix sums (see pass 1)
-            auto seg_begin = [](int s) constexpr { return (E * s) / NSEG; };
-            double off_u, off_v, nxt_u = 0.0, nxt_v = 0.0, tot_u, tot_v;
+            double off_u = 0.0, off_v = 0.0, nxt_u = 0.0, nxt_v = 0.0, tot_u, tot_v;
             if constexpr (exact) {
-                off_u = off_v = 0.0;
-#pragma unroll
-                for (int c = 0; c < E; ++c) {
-                    float a_, b_;
-                    unpack2(x2[c], a_, b_);
-                    off_u += static_cast<double>(sq ? a_ * a_ : a_);
-                    off_v += static_cast<double>(sq ? b_ * b_ : b_);
-                }
+                raw_cumsum(x2, sq, off_u, off_v, [](int, float) {}, [](int, float) {});
                 cta_scan2d<TPF>(off_u, off_v, tot_u, tot_v, scratch, tid);
             } else {
-                // Long local runs (33 bins per thread) are summed in NSEG independent segments: the fp32 rounding
-                // error of a local prefix grows with the number of adds behind it (33 sequential adds: up to 5 ulp
-                // of the fp64 CDF on the paper's spectra, four runs of 8 or 9: <= 3), and four short dependency
-                // chains issue faster than one long one.
+                // the adds of cdf_entries (a segment's sum is its last prefix), written out like the local sums of
+                // sot_long.cu: as a call, ptxas allocates the 32 x 33 complex gradient kernel differently
+                constexpr int NSEG = cdf_segments(E);
                 f32x2 t2 = 0;
 #pragma unroll
                 for (int s = 0; s < NSEG; ++s) {
                     f32x2 acc2 = 0;
-                    if (sq) {  // (uniform branch: a per-element select costs three extra instructions)
+                    if (sq) {
 #pragma unroll
-                        for (int c = seg_begin(s); c < seg_begin(s + 1); ++c) acc2 = fma2(x2[c], x2[c], acc2);
-                    } else {   // (the same instructions as in pass 2: a segment's sum is its last prefix)
+                        for (int c = seg_begin<E>(s); c < seg_begin<E>(s + 1); ++c) acc2 = fma2(x2[c], x2[c], acc2);
+                    } else {
 #pragma unroll
-                        for (int c = seg_begin(s); c < seg_begin(s + 1); ++c) acc2 = add2(acc2, x2[c]);
+                        for (int c = seg_begin<E>(s); c < seg_begin<E>(s + 1); ++c) acc2 = add2(acc2, x2[c]);
                     }
                     t2 = NSEG == 1 ? acc2 : add2(t2, acc2);
                 }
@@ -816,73 +527,25 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
             }
             base_mass_u = off_u;
             base_mass_v = off_v;
-            const float mass_u = static_cast<float>(tot_u), mass_v = static_cast<float>(tot_v);
-            u_live = mass_u > SAFE_EPS;  // utils.py:137: den <= eps -> eps
-            v_live = mass_v > SAFE_EPS;
-            inv_u = recip_f64(u_live ? mass_u : SAFE_EPS);
-            inv_v = cut_scale ? inv_u : recip_f64(v_live ? mass_v : SAFE_EPS);
-            if constexpr (exact) {  // no normalisation, hence no mass term in the gradient
-                inv_u = inv_v = 1.0;
-                u_live = v_live = false;
-            }
+            nm = normalise<exact>(tot_u, tot_v, cut_scale);
             if constexpr (NW == 1) __syncwarp();
             if constexpr (exact) {
                 double tu = off_u, tv = off_v;
-#pragma unroll
-                for (int c = 0; c < E; ++c) {
-                    float a_, b_;
-                    unpack2(x2[c], a_, b_);
-                    tu += static_cast<double>(sq ? a_ * a_ : a_);
-                    tv += static_cast<double>(sq ? b_ * b_ : b_);
-                    if (in_u || e0 + c < n) sts32(A0 + 4 * (e0 + c), static_cast<float>(tu));
-                    if (in_v || e0 + c < m) sts32(B0 + 4 * (e0 + c), static_cast<float>(tv));
-                }
+                raw_cumsum(
+                    x2, sq, tu, tv, [&](int c, float x) { if (in_u || e0 + c < n) sts32(A0 + 4 * (e0 + c), x); },
+                    [&](int c, float x) { if (in_v || e0 + c < m) sts32(B0 + 4 * (e0 + c), x); });
             } else {
-                // Pass 2: CDF entry = base + (local prefix) * 1/mass with base = (sum of the threads before
-                // me) * 1/mass from the fp64 scan, split into an fp32 head and tail so that the one rounding
-                // that matters is the final add.  The local prefix is the SAME fp32 sequence as in pass 1, so
-                // the entry after my last bin is the next thread's base; each entry is capped by that value
-                // (bitwise the next thread's head), which keeps the row non-decreasing across thread
-                // boundaries whatever the roundings of the scaling do.
-                const double base_u = off_u * inv_u, base_v = off_v * inv_v;
-                const float bh_u = static_cast<float>(base_u), bh_v = static_cast<float>(base_v);
-                const float bl_u = static_cast<float>(base_u - static_cast<double>(bh_u));
-                const float bl_v = static_cast<float>(base_v - static_cast<double>(bh_v));
-                const float cap_u = static_cast<float>(nxt_u * inv_u), cap_v = static_cast<float>(nxt_v * inv_v);
-                const f32x2 bh2 = pack2(bh_u, bh_v), bl2 = pack2(bl_u, bl_v);
-                const f32x2 inv2 = pack2(static_cast<float>(inv_u), static_cast<float>(inv_v));
                 // Every thread stores all E entries (rows hold TPF * E floats and more): no per-element guards, one
                 // code path -- the few threads whose bins straddle or lie past the end of a row used to drag
                 // their whole warp through a second, guarded copy of this loop.  What they wrote past the row is
                 // overwritten below (sentinels).
-                // Segments (NSEG > 1): a segment's prefixes restart from 0 and ride on `sbl2` = the pre-head value of
-                // the previous segment's LAST entry (tail + everything before the segment, already scaled), so an
-                // entry still costs one FFMA2 + one FADD2, nothing is carried from pass 1, and -- fma and add being
-                // monotone in the prefix -- a segment's entries start from the last entry of the one before: the
-                // row is non-decreasing across segment boundaries by construction.
-                auto emit = [&](auto SQ) {
-                    f32x2 sbl2 = bl2;
-#pragma unroll
-                    for (int s = 0; s < NSEG; ++s) {
-                        f32x2 p2 = 0, in2 = sbl2;
-#pragma unroll
-                        for (int c = seg_begin(s); c < seg_begin(s + 1); ++c) {
-                            p2 = decltype(SQ)::value ? fma2(x2[c], x2[c], p2) : add2(p2, x2[c]);
-                            in2 = fma2(p2, inv2, sbl2);
-                            float ca, cb;
-                            unpack2(add2(in2, bh2), ca, cb);
-                            sts32(A0 + 4 * (e0 + c), fminf(ca, cap_u));
-                            sts32(B0 + 4 * (e0 + c), fminf(cb, cap_v));
-                        }
-                        sbl2 = in2;
-                    }
-                };
-                if (sq) emit(std::true_type{}); else emit(std::false_type{});  // (uniform branch)
+                const CdfScale k = cdf_scale(off_u, off_v, nxt_u, nxt_v, nm);
+                const auto store_u = [&](int c, float x) { sts32(A0 + 4 * (e0 + c), x); };
+                const auto store_v = [&](int c, float x) { sts32(B0 + 4 * (e0 + c), x); };
+                if (sq) cdf_entries<true>(x2, k, store_u, store_v); else cdf_entries<false>(x2, k, store_u, store_v);
             }
-            // NaN / inf anywhere (or an overflowing cut-mode scale) poisons the frame: the walk is skipped
-            // (its +inf sentinels must stay unique) and NaN is written instead
-            finite = (fabs(tot_u * inv_u) <= static_cast<double>(FLT_BIG)) &&
-                     (fabs(tot_v * inv_v) <= static_cast<double>(FLT_BIG));
+            // a poisoned frame skips the walk (its +inf sentinels must stay unique) and NaN is written instead
+            finite = finite_frame(tot_u, tot_v, nm);
         } else {
             float xu[E], xv[E];
 #pragma unroll
@@ -1052,6 +715,7 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
                         fmd = __fmul_rn(D, keep);
                     }
                     acc[ch] = fmaf(q - qprev[ch], fmd, acc[ch]);
+                    // tie_step(), written out here and below: as a call, ptxas allocates the gradient kernels differently
                     const bool same = (q == qprev[ch]);
                     const float md = same ? md_prev[ch] : fmd;
                     sts32o<LY::G_OFF>(consumed[ch], md_prev[ch] - md);  // dL/dCDF of the previous slot (0 inside a group)
@@ -1085,6 +749,8 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
                         const float qn = fminf(a[ch], b[ch]);
                         const float Dn = UNI ? cost_of_gap<PMODE>(pa[ch], args.p) : transport_cost<PMODE>(pa[ch], pb[ch], args.p);
                         const float mdn = (qn > thr) ? 0.0f : Dn;
+                        // tie_step() written out (see gstep), without the update of md_prev: the carry is the m*d of
+                        // my last group
                         const bool same = (qn == qprev[ch]);
                         const float md = same ? md_prev[ch] : mdn;
                         sts32o<LY::G_OFF>(consumed[ch], md_prev[ch] - md);
@@ -1099,12 +765,7 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
 #pragma unroll
                 for (int ch = 0; ch < NCH; ++ch) {
                     if (fix[ch] != NO_FIX) {
-                        uint32_t sa = carry + 4u * (NCH * tid + ch - 1);
-                        float c = lds32(sa);
-                        while (c < 0.0f) {  // chunk 0 never carries the marker
-                            sa -= 4;
-                            c = lds32(sa);
-                        }
+                        const float c = look_back(carry + 4u * (NCH * tid + ch - 1), 4u, lds32);
                         sts32o<LY::G_OFF>(fix[ch], lds32o<LY::G_OFF>(fix[ch]) + c);
                     }
                 }
@@ -1152,12 +813,8 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
 #pragma unroll
                 for (int ch = 0; ch < NCH; ++ch) {
                     if (n_inherited[ch] > 0) {
-                        uint32_t sa = carry + 4u * (NCH * tid + ch - 1);
-                        int c = __float_as_int(lds32(sa));
-                        while (c < 0) {
-                            sa -= 4;
-                            c = __float_as_int(lds32(sa));
-                        }
+                        const int c = look_back(carry + 4u * (NCH * tid + ch - 1), 4u,
+                                                [](uint32_t a) { return __float_as_int(lds32(a)); });
                         const int is2 = c >> 16, js2 = c & 0xffff;
                         for (int t = 0; t < n_inherited[ch]; ++t) {
                             const long long o = frame * K + k0[ch] + t;
@@ -1290,22 +947,19 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
                     __syncwarp();
                 }
                 write_loss();
-                dot_u *= inv_u;
-                dot_v *= inv_v;
+                dot_u *= nm.inv_u;
+                dot_v *= nm.inv_v;
                 // every thread has read its dL/dCDF entries and is done with the CDF rows (barrier above): the CDF
                 // rows can take the next frame, the dL/dCDF rows the finished gradients
                 if constexpr (!CPLX) {  // (complex: the landing rows are the output staging, see below)
                     if (elected && has_next && bulk_in) issue_load(fbase + fstride);
                 }
-                // a clamped mass has no derivative (torch.where picks the constant branch)
-                const double corr_u = u_live ? (cut_scale ? dot_u + dot_v : dot_u) : 0.0;
-                const double corr_v = (!cut_scale && v_live) ? dot_v : 0.0;
+                double corr_u, corr_v;
+                mass_terms(nm, cut_scale, dot_u, dot_v, corr_u, corr_v);
                 // gw = offset + local suffix; (offset - corr) is formed in fp64 before rounding
                 const float bu = static_cast<float>(off_u - corr_u), bv = static_cast<float>(off_v - corr_v);
-                const float up = (args.upstream != nullptr ? args.upstream[frame] : 1.0f) *
-                                 (args.upstream_scale != nullptr ? *args.upstream_scale : 1.0f) * args.upstream_value;
-                const float ku = finite ? static_cast<float>(inv_u) * up * (square ? 2.0f : 1.0f) : f_nan();
-                const float kv = finite ? static_cast<float>(inv_v) * up * (square ? 2.0f : 1.0f) : f_nan();
+                float ku, kv;
+                grad_scale(nm, upstream_of(args, frame), square, finite, ku, kv);
                 if constexpr (!CPLX) {
                     const f32x2 b2 = pack2(bu, bv), k2 = pack2(ku, kv);
                     const uint32_t out_u = GA0 + lead_u + 4 * e0, out_v = GB0 + lead_v + 4 * e0;
@@ -1411,10 +1065,7 @@ __global__ void __launch_bounds__(TPF * FPW, min_ctas(TPF * FPW, E, FPW * Layout
             if (threadIdx.x == 0) cta_loss += other;
         }
     }
-    if (threadIdx.x == 0 && args.loss_sum != nullptr) {
-        atomicAdd(args.loss_sum, cta_loss);  // one atomic per CTA
-        if (args.ticket != nullptr) finish_mean(args);
-    }
+    if (threadIdx.x == 0 && args.loss_sum != nullptr) add_cta_loss(args, cta_loss);  // one atomic per CTA
     if constexpr (WITH_GRAD) {
         if (tid == 0) bulk_wait_read_all();  // shared memory must outlive the last bulk store
     }

@@ -4,17 +4,13 @@
 //
 // One CTA per frame, persistent grid.  The CDFs and dL/dCDF live in library-owned global scratch, one slot per CTA
 // (allocated stream-ordered per launch, at most kScratchBytes unless a single frame needs more): a resident slice
-// of frames keeps its re-reads in L2.  Per frame:
+// of frames keeps its re-reads in L2.  The arithmetic is the frame kernel's: the helpers of sot_device.cuh.  Per frame:
 //   pass 0  masses: the fp64 carry of the per-tile sums of the CDF stage below (bitwise the same additions)
-//   pass 1  CDFs, tile by tile (TPB threads x E bins): the entry arithmetic of stage 2 of sot_kernels.cuh -- packed
-//           fp32 local prefixes, fp64 offsets (scan within the tile + carry across tiles), fp32 head / tail split of
-//           offset * 1/mass, every entry capped by the next thread's head.  A tile's last thread is capped by the
-//           next tile's first head (the same fp64 value), so the row is non-decreasing across tile borders, and the
-//           row end is set to fl32(mass * 1/mass).  Raw weights: fp64 per entry, like the reference's CPU cumsum.
+//   pass 1  CDFs, tile by tile (TPB threads x E bins, one segment), offsets = in-tile scan + carry of the tiles before.
+//           A tile's last thread is capped by the next tile's first head (the same fp64 value): the row is
+//           non-decreasing across tile borders.  The row end is set to fl32(mass * 1/mass).
 //   walk    merge-path co-rank search on the scratch CDFs, then each thread walks one chunk of the n + m merged
-//           slots: sum dq * |dx|^p (searchsorted-left, clamp to the last bin, strict `qs > 1` mask).  Gradient
-//           mode stores dL/dCDF at the last slot of each tie group (stable order, u before v) and patches groups
-//           opened by an earlier chunk with a look-back over per-chunk carries (stage 3 of sot_kernels.cuh).
+//           slots: sum dq * |dx|^p (searchsorted-left, clamp to the last bin, strict `qs > 1` mask), and dL/dCDF.
 //   grad    mass term sum_i gw_i w_i (per thread S_t * P_t + sum_i ls_i w_i, over all tiles), then the tiles in
 //           reverse: suffix sums of dL/dCDF (fp32 local, fp64 across threads and tiles), chain rule, x 2x, x upstream.
 // Every reduction runs in a fixed order: two runs give the same bits.
@@ -69,6 +65,8 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
             for (int c = 0; c < E; ++c)
                 x2[c] = pack2(e0 + c < n ? __ldg(xu + e0 + c) : 0.0f, e0 + c < m ? __ldg(xv + e0 + c) : 0.0f);
         };
+        // my local sums: pass 1 of the frame kernel with one segment, written out like there (as a shared helper, ptxas
+        // allocates this kernel and the frame kernel differently)
         auto local_sum = [&](const f32x2 (&x2)[E]) {
             f32x2 t2 = 0;
             if (square) {
@@ -80,21 +78,12 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
             }
             return t2;
         };
-        auto raw_sums = [&](const f32x2 (&x2)[E], double& a, double& b) {
-            a = b = 0.0;
-#pragma unroll
-            for (int c = 0; c < E; ++c) {
-                float a_, b_;
-                unpack2(x2[c], a_, b_);
-                a += static_cast<double>(square ? a_ * a_ : a_);
-                b += static_cast<double>(square ? b_ * b_ : b_);
-            }
-        };
         // exclusive fp64 offsets of my local sums within the tile, the next thread's, and the tile totals
         auto tile_scan = [&](const f32x2 (&x2)[E], double& ou, double& ov, double& nu, double& nv, double& tu,
                              double& tv) {
             if constexpr (RAW) {
-                raw_sums(x2, ou, ov);
+                ou = ov = 0.0;
+                raw_cumsum(x2, square, ou, ov, [](int, float) {}, [](int, float) {});
                 cta_scan2d<TPB>(ou, ov, tu, tv, red, tid);
             } else {
                 float Tu, Tv;
@@ -114,17 +103,8 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
             mass_u += tu;
             mass_v += tv;
         }
-        const float mu32 = static_cast<float>(mass_u), mv32 = static_cast<float>(mass_v);
-        bool u_live = mu32 > SAFE_EPS, v_live = mv32 > SAFE_EPS;  // utils.py:137
-        double inv_u = recip_f64(u_live ? mu32 : SAFE_EPS);
-        double inv_v = cut_scale ? inv_u : recip_f64(v_live ? mv32 : SAFE_EPS);
-        if constexpr (RAW) {  // weights used as given: no normalisation, no mass term
-            inv_u = inv_v = 1.0;
-            u_live = v_live = false;
-        }
-        // NaN / inf anywhere (or an overflowing cut-mode scale) poisons the frame (CTA uniform)
-        const bool finite = (fabs(mass_u * inv_u) <= static_cast<double>(FLT_BIG)) &&
-                            (fabs(mass_v * inv_v) <= static_cast<double>(FLT_BIG));
+        const Norm nm = normalise<RAW>(mass_u, mass_v, cut_scale);
+        const bool finite = finite_frame(mass_u, mass_v, nm);  // (CTA uniform)
 
         // ---- pass 1: CDFs ------------------------------------------------------------------------------------
         float acc = 0.0f;
@@ -136,37 +116,16 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
                 double ou, ov, nu = 0.0, nv = 0.0, tu, tv;
                 tile_scan(x2, ou, ov, nu, nv, tu, tv);
                 const int e0 = t0 + tid * E;
+                const auto store_u = [&](int c, float x) { if (e0 + c < n) cu[e0 + c] = x; };
+                const auto store_v = [&](int c, float x) { if (e0 + c < m) cv[e0 + c] = x; };
                 if constexpr (RAW) {
                     double ru = car_u + ou, rv = car_v + ov;
-#pragma unroll
-                    for (int c = 0; c < E; ++c) {
-                        float a_, b_;
-                        unpack2(x2[c], a_, b_);
-                        ru += static_cast<double>(square ? a_ * a_ : a_);
-                        rv += static_cast<double>(square ? b_ * b_ : b_);
-                        if (e0 + c < n) cu[e0 + c] = static_cast<float>(ru);
-                        if (e0 + c < m) cv[e0 + c] = static_cast<float>(rv);
-                    }
+                    raw_cumsum(x2, square, ru, rv, store_u, store_v);
                 } else {
                     // offsets across tiles: carry + in-tile offset; the last thread's `next` is carry + tile total =
                     // the next tile's carry, i.e. bitwise the head the next tile's first thread starts from
-                    const double base_u = (car_u + ou) * inv_u, base_v = (car_v + ov) * inv_v;
-                    const float bh_u = static_cast<float>(base_u), bh_v = static_cast<float>(base_v);
-                    const float bl_u = static_cast<float>(base_u - static_cast<double>(bh_u));
-                    const float bl_v = static_cast<float>(base_v - static_cast<double>(bh_v));
-                    const float cap_u = static_cast<float>((car_u + nu) * inv_u);
-                    const float cap_v = static_cast<float>((car_v + nv) * inv_v);
-                    const f32x2 bh2 = pack2(bh_u, bh_v), bl2 = pack2(bl_u, bl_v);
-                    const f32x2 inv2 = pack2(static_cast<float>(inv_u), static_cast<float>(inv_v));
-                    f32x2 p2 = 0;
-#pragma unroll
-                    for (int c = 0; c < E; ++c) {
-                        p2 = square ? fma2(x2[c], x2[c], p2) : add2(p2, x2[c]);
-                        float ca, cb;
-                        unpack2(add2(fma2(p2, inv2, bl2), bh2), ca, cb);
-                        if (e0 + c < n) cu[e0 + c] = fminf(ca, cap_u);
-                        if (e0 + c < m) cv[e0 + c] = fminf(cb, cap_v);
-                    }
+                    const CdfScale k = cdf_scale(car_u + ou, car_v + ov, car_u + nu, car_v + nv, nm);
+                    if (square) cdf_entries<true>(x2, k, store_u, store_v); else cdf_entries<false>(x2, k, store_u, store_v);
                 }
                 car_u += tu;
                 car_v += tv;
@@ -177,8 +136,8 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
             }
             __syncthreads();
             if constexpr (!RAW) {  // the row end is exact: fl32(mass * 1/mass) (never below the entry before it)
-                if (tid == 0) cu[n - 1] = fmaxf(static_cast<float>(mass_u * inv_u), n > 1 ? cu[n - 2] : 0.0f);
-                if (tid == 1) cv[m - 1] = fmaxf(static_cast<float>(mass_v * inv_v), m > 1 ? cv[m - 2] : 0.0f);
+                if (tid == 0) cu[n - 1] = fmaxf(static_cast<float>(mass_u * nm.inv_u), n > 1 ? cu[n - 2] : 0.0f);
+                if (tid == 1) cv[m - 1] = fmaxf(static_cast<float>(mass_v * nm.inv_v), m > 1 ? cv[m - 2] : 0.0f);
                 __syncthreads();
             }
 
@@ -226,8 +185,6 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
                     advance();
                 }
             } else {
-                // dL/dCDF = (m*d)_group - (m*d)_next group at a group's LAST slot, stored one step late (when the
-                // next slot is known); a group that started before my chunk has unknown m*d: it is patched below
                 constexpr int NO_FIX = -1;
                 int fix = NO_FIX;
                 float md_prev = 0.0f, carry_out = -1.0f;
@@ -245,12 +202,7 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
                     for (int s = 1; s <= cnt; ++s) {
                         const float q2 = fminf(a, b);
                         const float D2 = cost_of_gap<0>(pa - pb, p);
-                        const bool same = (q2 == qprev);
-                        const float md = same ? md_prev : (q2 > thr ? 0.0f : D2);
-                        g[consumed] = md_prev - md;
-                        fix = (inherited && !same) ? consumed : fix;
-                        inherited = inherited && same;
-                        md_prev = md;
+                        g[consumed] = tie_step(q2, qprev, q2 > thr ? 0.0f : D2, consumed, md_prev, inherited, fix);
                         if (s == cnt) break;
                         accumulate(q2, D2);
                         qprev = q2;
@@ -260,12 +212,7 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
                 }
                 carry[tid] = carry_out;
                 __syncthreads();
-                if (fix != NO_FIX) {  // look-back: chunk 0 never carries the marker
-                    int t = tid - 1;
-                    float c = carry[t];
-                    while (c < 0.0f) c = carry[--t];
-                    g[fix] += c;
-                }
+                if (fix != NO_FIX) g[fix] += look_back(tid - 1, 1, [&](int t) { return carry[t]; });
                 __syncthreads();
             }
         }
@@ -289,8 +236,7 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
         if constexpr (GRAD) {
             float* const ou = args.grad_u != nullptr ? args.grad_u + frame * n : nullptr;
             float* const ov = args.grad_v != nullptr ? args.grad_v + frame * m : nullptr;
-            const float up = (args.upstream != nullptr ? args.upstream[frame] : 1.0f) *
-                             (args.upstream_scale != nullptr ? *args.upstream_scale : 1.0f) * args.upstream_value;
+            const float up = upstream_of(args, frame);
             if (!finite) {
                 for (int k = tid; k < n && ou != nullptr; k += TPB) ou[k] = f_nan();
                 for (int k = tid; k < m && ov != nullptr; k += TPB) ov[k] = f_nan();
@@ -299,7 +245,7 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
             auto gpair = [&](int e) { return pack2(e < n ? g[e] : 0.0f, e < m ? g[n + e] : 0.0f); };
             // ---- mass term: sum_i gw_i w_i = sum_t (S_t P_t + sum_i ls_i w_i), P_t = the CDF stage's prefix ----
             double dot_u = 0.0, dot_v = 0.0;
-            if (u_live || v_live) {
+            if (nm.u_live || nm.v_live) {
                 double car_u = 0.0, car_v = 0.0;
                 for (int t0 = 0; t0 < rows; t0 += TILE) {
                     f32x2 x2[E];
@@ -338,14 +284,13 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
                     dot_v += red[3 * NW + k];
                 }
                 __syncthreads();
-                dot_u *= inv_u;
-                dot_v *= inv_v;
+                dot_u *= nm.inv_u;
+                dot_v *= nm.inv_v;
             }
-            // a clamped mass has no derivative (torch.where picks the constant branch)
-            const double corr_u = u_live ? (cut_scale ? dot_u + dot_v : dot_u) : 0.0;
-            const double corr_v = (!cut_scale && v_live) ? dot_v : 0.0;
-            const float ku = static_cast<float>(inv_u) * up * (square ? 2.0f : 1.0f);
-            const float kv = static_cast<float>(inv_v) * up * (square ? 2.0f : 1.0f);
+            double corr_u, corr_v;
+            mass_terms(nm, cut_scale, dot_u, dot_v, corr_u, corr_v);
+            float ku, kv;
+            grad_scale(nm, up, square, finite, ku, kv);
             const f32x2 k2 = pack2(ku, kv);
             // ---- tiles in reverse: suffix sums of dL/dCDF, chain rule, x 2x, x upstream --------------------------
             double suf_u = 0.0, suf_v = 0.0;  // sum of dL/dCDF of the tiles after this one
@@ -379,10 +324,7 @@ __global__ void __launch_bounds__(TPB) sot_long_kernel(const FrameArgs args, flo
             __syncthreads();  // every read of g is done before the next frame's walk writes it
         }
     }
-    if (tid == 0 && args.loss_sum != nullptr) {
-        atomicAdd(args.loss_sum, cta_loss);  // one atomic per CTA
-        if (args.ticket != nullptr) finish_mean(args);
-    }
+    if (tid == 0 && args.loss_sum != nullptr) add_cta_loss(args, cta_loss);  // one atomic per CTA
 }
 
 template <bool GRAD, bool RAW>

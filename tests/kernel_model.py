@@ -1,4 +1,4 @@
-"""Executable model (numpy, scalar loops) of the ALGORITHM the CUDA kernel runs for one frame.
+"""Executable model (numpy) of the ALGORITHM the CUDA kernels run for one frame.
 
 It follows `csrc/sot_kernels.cuh` stage by stage -- merge-path partition per chunk, the sequential
 walk with tie-group tracking, the one-slot peek across the chunk boundary, the look-back carry
@@ -158,55 +158,62 @@ def frame_loss_and_grads(x, y, pu, pv, p, square, cut_scale, limit, T, L):
 
 
 def cdf_segments(per_thread):
-    """Segment boundaries of a thread's local prefix sums (csrc/sot_kernels.cuh: NSEG, seg_begin)."""
+    """Segment boundaries of a thread's local prefix sums (csrc/sot_device.cuh: cdf_segments, seg_begin)."""
     nseg = 4 if per_thread >= 25 else 1
     return [(per_thread * s) // nseg for s in range(nseg + 1)]
 
 
-def cdf_stage_model(x, threads, per_thread, mass_floor=EPS, square=True, inv64=None, return_inv=False):
-    """Model of the kernel's CDF stage (csrc/sot_kernels.cuh, stage 2) for one row `x` (float32):
-    thread t owns bins [t*E, t*E+E), cut into segments (one for E < 25, four for 33 bins); fp32 prefix sums
-    restart in every segment (x^2 fused into the add); a thread's sum = fp32 sum of its segment sums; the
-    per-thread sums are added up in fp64 -> exclusive offsets; entry = fl32(head + fl32(prefix * inv32 + ride))
-    where (head, tail) is the fp32 split of offset * inv64 and `ride` is the tail in the first segment, afterwards
-    the fl32(prefix * inv32 + ride) of the previous segment's last entry; every entry is capped by the next
-    thread's head.  Returns the float32 CDF row.  (fl32(x*x + acc) is formed in float64 and rounded once: x*x is
-    exact there.)  `inv64`: 1/mass to scale by (cutoff mode scales the target row by the prediction's); default:
-    this row's own (`return_inv`: also return the 1/mass used)."""
+def cdf_stage_model(x, threads, per_thread, mass_floor=EPS, square=True, inv64=None, return_inv=False, tile=None,
+                    exact_end=False):
+    """Model of the CDF stage of both kernels (csrc/sot_device.cuh: cdf_scale, cdf_entries) for one row `x`
+    (float32), vectorised over the threads: thread t owns bins [t*E, t*E+E), cut into segments (one for E < 25, four
+    for 33 bins); fp32 prefix sums restart in every segment (x^2 fused into the add); a thread's sum = fp32 sum of its
+    segment sums; the per-thread sums are added up in fp64 -> exclusive offsets (with `tile`: a scan within each tile of
+    that many threads plus the fp64 carry of the tiles before, as the split-frame kernel does); entry =
+    fl32(head + fl32(prefix * inv32 + ride)) where (head, tail) is the fp32 split of offset * inv64 and `ride` is the
+    tail in the first segment, afterwards the fl32(prefix * inv32 + ride) of the previous segment's last entry; every
+    entry is capped by the next thread's head.  `exact_end`: the row end is fl32(mass * inv64), never below the entry
+    before it (the split-frame kernel).  Returns the float32 CDF row.  (fl32(x*x + acc) is formed in float64 and
+    rounded once: x*x is exact there.)  `inv64`: 1/mass to scale by (cutoff mode scales the target row by the
+    prediction's); default: this row's own (`return_inv`: also return the 1/mass used and the fp64 mass)."""
     n = len(x)
     E = per_thread
     bounds = cdf_segments(E)
     xs = np.zeros(threads * E, np.float64)
     xs[:n] = np.asarray(x, np.float32).astype(np.float64)
+    xs = xs.reshape(threads, E)
     local = np.zeros((threads, E), np.float32)
-    totals = np.zeros(threads, np.float64)
-    for t in range(threads):
-        tot = F32(0.0)
-        for s in range(len(bounds) - 1):
-            acc = F32(0.0)
-            for c in range(bounds[s], bounds[s + 1]):
-                v = xs[t * E + c]
-                acc = F32((v * v if square else v) + np.float64(acc))
-                local[t, c] = acc
-            tot = acc if len(bounds) == 2 else F32(tot + acc)
-        totals[t] = tot
-    offsets = np.concatenate(([0.0], np.cumsum(totals)))  # offsets[t] exclusive, offsets[threads] = total
+    totals = np.zeros(threads, np.float32)
+    for s in range(len(bounds) - 1):
+        acc = np.zeros(threads, np.float32)
+        for c in range(bounds[s], bounds[s + 1]):
+            v = xs[:, c]
+            acc = ((v * v if square else v) + acc.astype(np.float64)).astype(np.float32)
+            local[:, c] = acc
+        totals = acc if len(bounds) == 2 else (totals + acc).astype(np.float32)
+    tile = threads if tile is None else tile
+    offsets = np.zeros(threads + 1)  # offsets[t] exclusive, offsets[threads] = total
+    carry = 0.0
+    for t0 in range(0, threads, tile):
+        excl = np.concatenate(([0.0], np.cumsum(totals[t0:t0 + tile].astype(np.float64))))
+        offsets[t0:t0 + len(excl)] = carry + excl
+        carry = carry + excl[-1]
     mass = F32(offsets[-1])
     if inv64 is None:
         inv64 = 1.0 / np.float64(mass if mass > mass_floor else mass_floor)
-    inv32 = F32(inv64)
-    out = np.zeros(n, np.float32)
-    for t in range(threads):
-        base = offsets[t] * inv64
-        head = F32(base)
-        ride = F32(base - np.float64(head))
-        cap = F32(offsets[t + 1] * inv64)
-        for s in range(len(bounds) - 1):
-            inner = ride
-            for c in range(bounds[s], bounds[s + 1]):
-                i = t * E + c
-                inner = F32(np.float64(local[t, c]) * np.float64(inv32) + np.float64(ride))  # one FFMA
-                if i < n:
-                    out[i] = min(F32(head + inner), cap)
-            ride = inner
-    return (out, inv64) if return_inv else out
+    inv32 = np.float64(F32(inv64))
+    base = offsets[:-1] * inv64
+    head = base.astype(np.float32).astype(np.float64)
+    ride = (base - head).astype(np.float32)
+    cap = (offsets[1:] * inv64).astype(np.float32)
+    out = np.zeros((threads, E), np.float32)
+    for s in range(len(bounds) - 1):
+        inner = ride
+        for c in range(bounds[s], bounds[s + 1]):
+            inner = (local[:, c].astype(np.float64) * inv32 + ride.astype(np.float64)).astype(np.float32)  # one FFMA
+            out[:, c] = np.minimum((head + inner.astype(np.float64)).astype(np.float32), cap)
+        ride = inner
+    out = out.reshape(-1)[:n].copy()
+    if exact_end:
+        out[-1] = max(F32(offsets[-1] * inv64), out[-2] if n > 1 else F32(0))
+    return (out, inv64, offsets[-1]) if return_inv else out

@@ -165,7 +165,7 @@ def test_cdf_stage_model_on_the_reference_fixtures_one_warp_per_frame(name):
         return int(np.abs(a.view(np.int32).astype(np.int64) - b.view(np.int32).astype(np.int64)).max())
 
     for r in range(x.shape[0]):
-        cu, inv = KM.cdf_stage_model(x[r].numpy(), 32, 33, square=kw["square"], return_inv=True)
+        cu, inv, _ = KM.cdf_stage_model(x[r].numpy(), 32, 33, square=kw["square"], return_inv=True)
         cv = KM.cdf_stage_model(y[r].numpy(), 32, 33, square=kw["square"], inv64=inv if kw["cut_scale"] else None)
         assert np.all(np.diff(cu) >= 0) and np.all(np.diff(cv) >= 0)
         assert ulps(cu, c64u[r]) <= 3 and ulps(cv, c64v[r]) <= 3, (r, ulps(cu, c64u[r]), ulps(cv, c64v[r]))

@@ -172,6 +172,15 @@ class _on_device:
         return False
 
 
+def _launch(name: str, device, *args, stream=None) -> None:
+    """Calls the C entry point `name` with `args` and the current stream of `device` (or `stream`, a
+    `torch.cuda.Stream`) on that device; raises on a non-zero return code."""
+    fn = getattr(load(), name)
+    handle = _stream(device) if stream is None else ctypes.c_void_p(stream.cuda_stream)
+    with _on_device(device):
+        _check(fn(*args, handle))
+
+
 def make_problem(u, v, pos_u, pos_v, p: float, flags: int) -> SotProblem:
     """u: (N, n), v: (N, m) contiguous CUDA float32; pos_*: (n,) shared or (N, n) per frame.
 
@@ -182,6 +191,11 @@ def make_problem(u, v, pos_u, pos_v, p: float, flags: int) -> SotProblem:
         raise TypeError(f"sot_b200: `x` and `y` must have the same dtype, got {u.dtype} and {v.dtype}")
     if u.is_complex():
         flags = int(flags) | SOT_COMPLEX_INPUT
+    return _problem(u, v, pos_u, pos_v, p, flags)
+
+
+def _problem(u, v, pos_u, pos_v, p: float, flags: int) -> SotProblem:
+    """The shape and stride rules shared by the device entry points and the host-buffer one."""
     if u.ndim != 2 or v.ndim != 2 or u.shape[0] != v.shape[0]:
         raise ValueError(f"sot_b200: expected (N, n) and (N, m) rows, got {tuple(u.shape)} and {tuple(v.shape)}")
     if not (u.is_contiguous() and v.is_contiguous() and pos_u.is_contiguous() and pos_v.is_contiguous()):
@@ -203,16 +217,13 @@ def make_problem(u, v, pos_u, pos_v, p: float, flags: int) -> SotProblem:
 
 
 def forward(u, v, pos_u, pos_v, p, flags) -> torch.Tensor:
-    lib = load()
     prob = make_problem(u, v, pos_u, pos_v, p, flags)
     loss = torch.empty(u.shape[0], dtype=torch.float32, device=u.device)
-    with torch.cuda.device(u.device):
-        _check(lib.sot_forward_device(ctypes.byref(prob), _ptr(loss), _stream(u.device)))
+    _launch("sot_forward_device", u.device, ctypes.byref(prob), _ptr(loss))
     return loss
 
 
 def forward_backward(u, v, pos_u, pos_v, p, flags, upstream=None, want_loss=True, want_gu=True, want_gv=True):
-    lib = load()
     prob = make_problem(u, v, pos_u, pos_v, p, flags)
     if upstream is not None:
         _dev_tensor(upstream, "upstream")
@@ -221,9 +232,8 @@ def forward_backward(u, v, pos_u, pos_v, p, flags, upstream=None, want_loss=True
     loss = torch.empty(u.shape[0], dtype=torch.float32, device=u.device) if want_loss else None
     gu = torch.empty_like(u) if want_gu else None
     gv = torch.empty_like(v) if want_gv else None
-    with torch.cuda.device(u.device):
-        _check(lib.sot_forward_backward_device(ctypes.byref(prob), _ptr(upstream), _ptr(loss), _ptr(gu), _ptr(gv),
-                                               _stream(u.device)))
+    _launch("sot_forward_backward_device", u.device, ctypes.byref(prob), _ptr(upstream), _ptr(loss), _ptr(gu),
+            _ptr(gv))
     return loss, gu, gv
 
 
@@ -249,7 +259,6 @@ def mean_step(u, v, pos_u, pos_v, p, flags, grad_scale: float, mean_scale: float
     (sum, count_value) instead of / besides the mean; `post` = (mailbox pointers, rank, seq): the last CTA also
     stores (sum, count_value, seq) into every peer's mailbox (seq: an int, or a one-element int64 DEVICE tensor
     holding the previous call number).  Returns (mean or None, rows or None, gu, gv)."""
-    lib = load()
     prob = make_problem(u, v, pos_u, pos_v, p, flags)
     dev = u.device
     if want_mean is None:
@@ -271,27 +280,27 @@ def mean_step(u, v, pos_u, pos_v, p, flags, grad_scale: float, mean_scale: float
     keep = None
     if post is not None:
         ptrs, rank, seq = post
-        keep = ptrs if isinstance(ptrs, ctypes.Array) else mailbox_array(ptrs)
+        keep = mailbox_array(ptrs)
         plan.post_mailboxes, plan.post_world, plan.post_rank = keep, len(keep), int(rank)
         if isinstance(seq, torch.Tensor):
             plan.post_seq, plan.post_seq_device = 0, seq.data_ptr()
         else:
             plan.post_seq = int(seq)
-    with _on_device(dev):
-        _check(lib.sot_mean_step_device(ctypes.byref(prob), ctypes.byref(plan), _ptr(rows), _ptr(gu), _ptr(gv),
-                                        _stream(dev)))
+    _launch("sot_mean_step_device", dev, ctypes.byref(prob), ctypes.byref(plan), _ptr(rows), _ptr(gu), _ptr(gv))
     return mean, rows, gu, gv
 
 
 def mailbox_array(ptrs):
-    """ctypes array of the peers' mailbox pointers (build it once, pass it to every call)."""
+    """ctypes array of the peers' mailbox pointers (build it once, pass it to every call); an array is returned as
+    it is."""
+    if isinstance(ptrs, ctypes.Array):
+        return ptrs
     return (ctypes.c_void_p * len(ptrs))(*[ctypes.c_void_p(int(q)) for q in ptrs])
 
 
 def scale_inplace(a, b, scale) -> None:
     """a *= scale; b *= scale in place (either may be None); `scale` = one-element float32 DEVICE tensor.  The
     kernel leaves at once when the scalar is exactly 1."""
-    lib = load()
     _dev_tensor(scale, "scale")
     if scale.numel() != 1:
         raise ValueError("sot_b200: the scale must hold one element")
@@ -305,24 +314,21 @@ def scale_inplace(a, b, scale) -> None:
             raise ValueError("sot_b200: rows to scale must be contiguous and on the scale's device")
         views.append(torch.view_as_real(t) if t.is_complex() else t)
     va, vb = views
-    with _on_device(dev):
-        _check(lib.sot_scale_inplace_device(_ptr(va), 0 if va is None else va.numel(), _ptr(vb),
-                                            0 if vb is None else vb.numel(), _ptr(scale), _stream(dev)))
+    _launch("sot_scale_inplace_device", dev, _ptr(va), 0 if va is None else va.numel(), _ptr(vb),
+            0 if vb is None else vb.numel(), _ptr(scale))
 
 
 def scale_rows(unit, scale) -> torch.Tensor:
-    lib = load()
-    _dev_tensor(unit, "unit"), _dev_tensor(scale, "scale")
+    """unit (N, F) float32 or complex64 rows times scale (N,): a new tensor."""
+    _dev_tensor(unit, "unit", True), _dev_tensor(scale, "scale")
     out = torch.empty_like(unit)
-    with torch.cuda.device(unit.device):
-        _check(lib.sot_scale_rows_device(_ptr(unit), _ptr(scale), _ptr(out), unit.shape[0], unit.shape[1],
-                                         _stream(unit.device)))
+    width = 2 * unit.shape[1] if unit.is_complex() else unit.shape[1]  # (interleaved re, im pairs)
+    _launch("sot_scale_rows_device", unit.device, _ptr(unit), _ptr(scale), _ptr(out), unit.shape[0], width)
     return out
 
 
 def quantiles(u, v, pos_u, pos_v, flags, from_cdf=False, want_indices=False):
     """(uq, vq, qs, cu, cv[, iu, iv]); with `from_cdf` the rows ARE the CDFs (parity harness)."""
-    lib = load()
     prob = make_problem(u, v, pos_u, pos_v, 2.0, flags)
     N, n = u.shape
     m = v.shape[1]
@@ -330,32 +336,28 @@ def quantiles(u, v, pos_u, pos_v, flags, from_cdf=False, want_indices=False):
     uq, vq, qs = (torch.empty(N, n + m, **f32) for _ in range(3))
     iu = torch.empty(N, n + m, dtype=torch.int32, device=u.device) if want_indices else None
     iv = torch.empty(N, n + m, dtype=torch.int32, device=u.device) if want_indices else None
-    with torch.cuda.device(u.device):
-        if from_cdf:
-            cu, cv = u, v
-            _check(lib.sot_plan_from_cdf_device(ctypes.byref(prob), _ptr(uq), _ptr(vq), _ptr(qs), _ptr(iu), _ptr(iv),
-                                                _stream(u.device)))
-        else:
-            cu, cv = torch.empty(N, n, **f32), torch.empty(N, m, **f32)
-            _check(lib.sot_quantiles_device(ctypes.byref(prob), _ptr(uq), _ptr(vq), _ptr(qs), _ptr(cu), _ptr(cv),
-                                            _ptr(iu), _ptr(iv), _stream(u.device)))
+    if from_cdf:
+        cu, cv = u, v
+        _launch("sot_plan_from_cdf_device", u.device, ctypes.byref(prob), _ptr(uq), _ptr(vq), _ptr(qs), _ptr(iu),
+                _ptr(iv))
+    else:
+        cu, cv = torch.empty(N, n, **f32), torch.empty(N, m, **f32)
+        _launch("sot_quantiles_device", u.device, ctypes.byref(prob), _ptr(uq), _ptr(vq), _ptr(qs), _ptr(cu),
+                _ptr(cv), _ptr(iu), _ptr(iv))
     return (uq, vq, qs, cu, cv, iu, iv) if want_indices else (uq, vq, qs, cu, cv)
 
 
 def loss_from_cdf(cu, cv, pos_u, pos_v, p, flags, want_grads=True):
     """Parity harness: per-frame loss and dL/dcu, dL/dcv from injected CDF rows."""
-    lib = load()
     prob = make_problem(cu, cv, pos_u, pos_v, p, flags)
     loss = torch.empty(cu.shape[0], dtype=torch.float32, device=cu.device)
     g_cu = torch.empty_like(cu) if want_grads else None
     g_cv = torch.empty_like(cv) if want_grads else None
-    with torch.cuda.device(cu.device):
-        _check(lib.sot_loss_from_cdf_device(ctypes.byref(prob), _ptr(loss), _ptr(g_cu), _ptr(g_cv), _stream(cu.device)))
+    _launch("sot_loss_from_cdf_device", cu.device, ctypes.byref(prob), _ptr(loss), _ptr(g_cu), _ptr(g_cv))
     return loss, g_cu, g_cv
 
 
 def quantile_lookup(qs, cws, xs) -> torch.Tensor:
-    lib = load()
     for t, name in ((qs, "qs"), (cws, "cws"), (xs, "xs")):
         _dev_tensor(t, name)
         if t.ndim != 2 or not t.is_contiguous():
@@ -363,9 +365,8 @@ def quantile_lookup(qs, cws, xs) -> torch.Tensor:
     if cws.shape != xs.shape or qs.shape[0] != cws.shape[0]:
         raise ValueError("sot_b200: quantile_function shape mismatch")
     out = torch.empty_like(qs)
-    with torch.cuda.device(qs.device):
-        _check(lib.sot_quantile_lookup_device(_ptr(qs), _ptr(cws), _ptr(xs), _ptr(out), qs.shape[0], qs.shape[1],
-                                              cws.shape[1], _stream(qs.device)))
+    _launch("sot_quantile_lookup_device", qs.device, _ptr(qs), _ptr(cws), _ptr(xs), _ptr(out), qs.shape[0],
+            qs.shape[1], cws.shape[1])
     return out
 
 
@@ -373,21 +374,16 @@ def loss_grad_host(u, v, pos_u, pos_v, p, flags, upstream=None, want_loss=True, 
                    device=0, out=None):
     """Host-buffer entry point: CPU tensors in (ideally pinned), CPU tensors out; all copies and
     kernels happen inside the one C call.  `out` may carry preallocated (pinned) result tensors."""
-    lib = load()
     for t, name in ((u, "x"), (v, "y"), (pos_u, "x_pos"), (pos_v, "y_pos")):
         if t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous():
             raise ValueError(f"sot_b200: `{name}` must be a contiguous float32 CPU tensor for the host entry point")
-    N, n = u.shape
-    m = v.shape[1]
-    su = 0 if pos_u.ndim == 1 else n
-    sv = 0 if pos_v.ndim == 1 else m
-    prob = SotProblem(N, n, m, u.data_ptr(), v.data_ptr(), pos_u.data_ptr(), pos_v.data_ptr(), su, sv, float(p),
-                      int(flags))
+    prob = _problem(u, v, pos_u, pos_v, p, flags)
+    N = u.shape[0]
     out = out or {}
     loss = out.get("loss", torch.empty(N) if want_loss else None)
     gu = out.get("grad_u", torch.empty_like(u) if want_gu else None)
     gv = out.get("grad_v", torch.empty_like(v) if want_gv else None)
-    _check(lib.sot_loss_grad_host(ctypes.byref(prob), _ptr(upstream), _ptr(loss), _ptr(gu), _ptr(gv), int(device)))
+    _check(load().sot_loss_grad_host(ctypes.byref(prob), _ptr(upstream), _ptr(loss), _ptr(gu), _ptr(gv), int(device)))
     return loss, gu, gv
 
 
@@ -420,27 +416,22 @@ def _mss_check(zt, zv):
 
 def mss_forward(zt, zv, mag_weight, logmag_weight, loss_type, post_scale, total=None):
     """total (1,) float64 += post_scale * sum_i [mag_w d(|zt|,|zv|) + logmag_w d(safe_log|zt|, safe_log|zv|)]."""
-    lib = load()
     _mss_check(zt, zv)
     if total is None:
         total = torch.zeros(1, dtype=torch.float64, device=zt.device)
-    with torch.cuda.device(zt.device):
-        _check(lib.sot_mss_forward_device(_ptr(zt), _ptr(zv), zt.numel(), float(mag_weight), float(logmag_weight),
-                                          int(loss_type), float(post_scale), _ptr(total), _stream(zt.device)))
+    _launch("sot_mss_forward_device", zt.device, _ptr(zt), _ptr(zv), zt.numel(), float(mag_weight),
+            float(logmag_weight), int(loss_type), float(post_scale), _ptr(total))
     return total
 
 
 def mss_backward(zt, zv, mag_weight, logmag_weight, loss_type, post_scale, scale, want_t=True, want_v=True):
     """Complex gradients of scale * post_scale * S w.r.t. zt / zv (same layout as the inputs)."""
-    lib = load()
     _mss_check(zt, zv)
     _dev_tensor(scale, "scale")
     gt = torch.empty_like(zt) if want_t else None
     gv = torch.empty_like(zv) if want_v else None
-    with torch.cuda.device(zt.device):
-        _check(lib.sot_mss_backward_device(_ptr(zt), _ptr(zv), zt.numel(), float(mag_weight), float(logmag_weight),
-                                           int(loss_type), float(post_scale), _ptr(scale), _ptr(gt), _ptr(gv),
-                                           _stream(zt.device)))
+    _launch("sot_mss_backward_device", zt.device, _ptr(zt), _ptr(zv), zt.numel(), float(mag_weight),
+            float(logmag_weight), int(loss_type), float(post_scale), _ptr(scale), _ptr(gt), _ptr(gv))
     return gt, gv
 
 
@@ -450,14 +441,11 @@ def p2p_mailbox_doubles(world: int) -> int:
 
 def p2p_allreduce(values, out, mailbox_ptrs, rank: int, seq: int):
     """out[:] = sum over ranks of `values` (float64, <= 8 elements) through peer-mapped mailboxes."""
-    lib = load()
     if values.dtype != torch.float64 or out.dtype != torch.float64 or not values.is_cuda or not out.is_cuda:
         raise TypeError("sot_b200: p2p_allreduce works on CUDA float64 tensors")
-    world = len(mailbox_ptrs)
-    arr = (ctypes.c_void_p * world)(*[ctypes.c_void_p(int(p)) for p in mailbox_ptrs])
-    with torch.cuda.device(values.device):
-        _check(lib.sot_p2p_allreduce_device(_ptr(values), _ptr(out), values.numel(), arr, world, int(rank), int(seq),
-                                            _stream(values.device)))
+    arr = mailbox_array(mailbox_ptrs)
+    _launch("sot_p2p_allreduce_device", values.device, _ptr(values), _ptr(out), values.numel(), arr, len(arr),
+            int(rank), int(seq))
     return out
 
 
@@ -466,31 +454,23 @@ def p2p_wait_mean(mailbox_ptrs, rank: int, seq, expected_count: float = 0.0, sta
     """Collects call `seq` of every rank from this rank's mailbox (the stores were made by the last CTA of
     `mean_step(..., post=...)` on every rank) and returns the global mean, a 0-dim float32 tensor.  `stream`: a
     `torch.cuda.Stream` to launch on (default: the current one); `out`: where to write (default: a new tensor)."""
-    lib = load()
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     if out is None:
         out = torch.empty((), dtype=torch.float32, device=dev)
-    arr = mailbox_ptrs if isinstance(mailbox_ptrs, ctypes.Array) else mailbox_array(mailbox_ptrs)
-    handle = _stream(dev) if stream is None else ctypes.c_void_p(stream.cuda_stream)
+    arr = mailbox_array(mailbox_ptrs)
     on_device = isinstance(seq, torch.Tensor)  # one-element int64 device tensor: the previous call number
-    with _on_device(dev):
-        _check(lib.sot_p2p_wait_mean_device(_ptr(out), float(expected_count),
-                                            ctypes.c_void_p(status_ptr) if status_ptr else None, arr, len(arr),
-                                            int(rank), 0 if on_device else int(seq), _ptr(seq) if on_device else None,
-                                            int(timeout_ms), handle))
+    _launch("sot_p2p_wait_mean_device", dev, _ptr(out), float(expected_count),
+            ctypes.c_void_p(status_ptr) if status_ptr else None, arr, len(arr), int(rank),
+            0 if on_device else int(seq), _ptr(seq) if on_device else None, int(timeout_ms), stream=stream)
     return out
 
 
 def p2p_global_mean(local_sum, local_count: float, mailbox_ptrs, rank: int, seq: int):
     """(mean, 1 / count) over all ranks as two (1,) float32 tensors from this rank's (1,) float64 sum and its count."""
-    lib = load()
     if local_sum.dtype != torch.float64 or not local_sum.is_cuda or local_sum.numel() != 1:
         raise TypeError("sot_b200: p2p_global_mean takes a (1,) CUDA float64 sum")
     out = torch.empty(2, dtype=torch.float32, device=local_sum.device)
-    world = len(mailbox_ptrs)
-    arr = (ctypes.c_void_p * world)(*[ctypes.c_void_p(int(p)) for p in mailbox_ptrs])
-    with torch.cuda.device(local_sum.device):
-        _check(lib.sot_p2p_global_mean_device(_ptr(local_sum), float(local_count), _ptr(out),
-                                              ctypes.c_void_p(out.data_ptr() + 4), arr, world, int(rank), int(seq),
-                                              _stream(local_sum.device)))
+    arr = mailbox_array(mailbox_ptrs)
+    _launch("sot_p2p_global_mean_device", local_sum.device, _ptr(local_sum), float(local_count), _ptr(out),
+            ctypes.c_void_p(out.data_ptr() + 4), arr, len(arr), int(rank), int(seq))
     return out[0:1], out[1:2]

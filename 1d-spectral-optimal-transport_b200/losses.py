@@ -56,19 +56,12 @@ class _SotFrames(torch.autograd.Function):
         grad_loss = grad_loss.contiguous().float()
         if ctx.mode == "fused":
             gu, gv = ctx.saved_tensors
-            gu = _scale_rows(gu, grad_loss) if need_u else None
-            gv = _scale_rows(gv, grad_loss) if need_v else None
+            gu = _capi.scale_rows(gu, grad_loss) if need_u else None
+            gv = _capi.scale_rows(gv, grad_loss) if need_v else None
         else:
             u, v, pos_u, pos_v = ctx.saved_tensors
             _, gu, gv = _capi.forward_backward(u, v, pos_u, pos_v, ctx.p, ctx.flags, grad_loss, False, need_u, need_v)
         return gu, gv, None, None, None, None, None
-
-
-def _scale_rows(unit: torch.Tensor, scale: torch.Tensor) -> torch.Tensor:
-    if not unit.is_complex():
-        return _capi.scale_rows(unit, scale)
-    flat = torch.view_as_real(unit).reshape(unit.shape[0], -1)  # (N, 2F) interleaved
-    return torch.view_as_complex(_capi.scale_rows(flat, scale).reshape(unit.shape[0], -1, 2))
 
 
 # --------------------------------------------------------------------------------------
@@ -77,14 +70,18 @@ def _scale_rows(unit: torch.Tensor, scale: torch.Tensor) -> torch.Tensor:
 _sorted_cache: dict = {}  # id(user tensor) -> (weakref, version, ascending?)
 
 
+def _require_cuda(t: torch.Tensor, name: str) -> None:
+    if not t.is_cuda:
+        raise _capi.SotError(f"sot_b200: `{name}` lives on {t.device}; the SOT kernels are CUDA only "
+                             "(no CPU fallback exists by design)")
+
+
 def _rows(t: torch.Tensor, name: str) -> torch.Tensor:
     """(B, T, F) or (N, F) -> contiguous float32 (N, F) (losses.py:158-165).
 
     complex64 rows (an STFT that has not been through `.abs()`, features.py:236) are kept complex:
     the kernels form the magnitude themselves and return complex gradients."""
-    if not t.is_cuda:
-        raise _capi.SotError(f"sot_b200: `{name}` lives on {t.device}; the SOT kernels are CUDA only "
-                             "(no CPU fallback exists by design)")
+    _require_cuda(t, name)
     if t.dtype in (torch.float16, torch.bfloat16, torch.float64):
         t = t.float()  # (float64: the reference accepts it; the kernels compute in float32, the result is cast back)
     elif t.dtype not in (torch.float32, torch.complex64):
@@ -97,10 +94,12 @@ def _rows(t: torch.Tensor, name: str) -> torch.Tensor:
     return t.contiguous()
 
 
-def _support(pos: torch.Tensor, like: torch.Tensor, name: str) -> torch.Tensor:
+def _support(pos: torch.Tensor, like: torch.Tensor, name: str, attach: bool = False) -> torch.Tensor:
     """1-D -> shared grid (the reference `expand`s it, losses.py:167-170; an expanded view is
-    recognised and collapsed back); 2-D / 3-D -> per-frame rows."""
-    pos = pos.detach()  # (gradients w.r.t. the positions, when asked for, come from `_position_term`)
+    recognised and collapsed back); 2-D / 3-D -> per-frame rows.  `attach` keeps the positions in the
+    autograd graph (`_position_term`); the kernels never see them attached."""
+    if not attach:
+        pos = pos.detach()
     if pos.device != like.device:
         raise ValueError(f"sot_b200: `{name}` is on {pos.device} but the spectra are on {like.device}")
     if pos.dtype != torch.float32:
@@ -153,7 +152,8 @@ def _is_ascending(pos: torch.Tensor, owner: torch.Tensor) -> bool:
 def _order(pos: torch.Tensor, w: torch.Tensor, owner: torch.Tensor):
     """`require_sort` (losses.py:286-290) hoisted out of the kernel: supports that are already
     ascending (every linear grid, the log grid at n_fft 512) cost nothing; otherwise positions
-    and weights are permuted once with a stable argsort before the launch."""
+    and weights are permuted once with a stable argsort before the launch.  Positions attached to
+    the autograd graph stay attached through the sort."""
     if _is_ascending(pos, owner):
         return pos, w
     if pos.ndim == 1:
@@ -202,29 +202,46 @@ def _uniform_grid(pu: torch.Tensor, pv: torch.Tensor, owner_u: torch.Tensor, own
     return uniform
 
 
-def _prepare(x, y, x_pos, y_pos, p, square, cut_scale, limit, require_sort, raw_weights):
-    """Reference prologue that stays on the host: flatten, canonicalise supports, hoisted sort."""
-    assert p >= 1, f"The OT loss is only valid for p>=1, {p} was given"  # losses.py:271
+def _magnitude(t: torch.Tensor) -> torch.Tensor:
+    return t.abs() if t.is_complex() else t
+
+
+def _canonical(x, y, x_pos, y_pos, require_sort, raw_weights, keep_complex=False, attach_positions=False):
+    """The reference's prologue that stays on the host, shared by every launch so that they all see the same rows:
+    flatten, canonicalise the supports, hoisted sort.  Returns (u, v, pu, pv, (sorted u?, sorted v?)).
+
+    Complex rows stay complex only for the fused loss launch (`keep_complex`), and only when both sides are complex
+    and short enough for its |z| prologue in shared memory; otherwise |z| is taken in torch (the real path takes any
+    length).  `attach_positions` keeps the positions in the autograd graph for `_position_term`."""
+    if not keep_complex:
+        x, y = _magnitude(x), _magnitude(y)
     u, v = _rows(x, "x"), _rows(y, "y")
-    if u.is_complex() != v.is_complex():  # one side already a magnitude: take |.| of the other in torch
-        u, v = (u.abs() if u.is_complex() else u), (v.abs() if v.is_complex() else v)
-    if u.is_complex() and max(u.shape[1], v.shape[1]) > _capi.MAX_COMPLEX_BINS:
-        # complex rows too long for the fused |z| prologue (shared memory): |z| in torch, the real path takes any length
-        u, v = u.abs(), v.abs()
+    if not (u.is_complex() and v.is_complex() and max(u.shape[1], v.shape[1]) <= _capi.MAX_COMPLEX_BINS):
+        u, v = _magnitude(u), _magnitude(v)
     if u.is_complex() and raw_weights:
         raise TypeError("sot_b200: `wasserstein_1d` weights must be real")
     if u.shape[0] != v.shape[0]:
         raise ValueError(f"sot_b200: x has {u.shape[0]} frames, y has {v.shape[0]}")
-    pu, pv = _support(x_pos, u, "x_pos"), _support(y_pos, v, "y_pos")
+    pu, pv = _support(x_pos, u, "x_pos", attach_positions), _support(y_pos, v, "y_pos", attach_positions)
     sort_u, sort_v = require_sort if isinstance(require_sort, tuple) else (require_sort, require_sort)
     if sort_u:
         pu, u = _order(pu, u, x_pos)
     if sort_v:
         pv, v = _order(pv, v, y_pos)
-    flags = ((_capi.SOT_SQUARE if square else 0) | (_capi.SOT_CUT_SCALE if cut_scale else 0) |
-             (_capi.SOT_LIMIT if limit else 0) | (_capi.SOT_RAW_WEIGHTS if raw_weights else 0) |
-             (_capi.SOT_UNIFORM_GRID if _uniform_grid(pu, pv, x_pos, y_pos, (bool(sort_u), bool(sort_v))) else 0))
-    return u, v, pu, pv, flags
+    return u, v, pu, pv, (bool(sort_u), bool(sort_v))
+
+
+def _flags(square, cut_scale, raw_weights, limit=False, uniform=False) -> int:
+    return ((_capi.SOT_SQUARE if square else 0) | (_capi.SOT_CUT_SCALE if cut_scale else 0) |
+            (_capi.SOT_LIMIT if limit else 0) | (_capi.SOT_RAW_WEIGHTS if raw_weights else 0) |
+            (_capi.SOT_UNIFORM_GRID if uniform else 0))
+
+
+def _prepare(x, y, x_pos, y_pos, p, square, cut_scale, limit, require_sort, raw_weights):
+    """Rows, supports and flags of the loss and gradient launches."""
+    assert p >= 1, f"The OT loss is only valid for p>=1, {p} was given"  # losses.py:271
+    u, v, pu, pv, sort = _canonical(x, y, x_pos, y_pos, require_sort, raw_weights, keep_complex=True)
+    return u, v, pu, pv, _flags(square, cut_scale, raw_weights, limit, _uniform_grid(pu, pv, x_pos, y_pos, sort))
 
 
 # --------------------------------------------------------------------------------------
@@ -255,37 +272,10 @@ def _position_term(x, y, x_pos, y_pos, p, square, cut_scale, limit, require_sort
     kernel (`OUT_PLAN`) finds the merged grid and the indices, `position_term_from_plan` is differentiated by torch.
     A path the paper's configurations never take (trainer.py:187-197 builds the positions without gradients): an extra
     plan launch and ATen-sized temporaries, only when a position tensor requires a gradient."""
-    x, y = x.detach(), y.detach()
-    x, y = (x.abs() if x.is_complex() else x), (y.abs() if y.is_complex() else y)
-    u, v = _rows(x, "x"), _rows(y, "y")
-
-    def attached(pos, like):  # `_support` without the detach
-        pos = pos.to(torch.float32)
-        if pos.ndim == 3:
-            pos = pos.reshape(-1, pos.shape[-1])
-        if pos.ndim == 2 and (pos.shape[0] == 1 or pos.stride(0) == 0):
-            pos = pos[0]
-        _support(pos, like, "positions")  # shape / device checks
-        return pos
-
-    pu, pv = attached(x_pos, u), attached(y_pos, v)
-    sort_u, sort_v = require_sort if isinstance(require_sort, tuple) else (require_sort, require_sort)
-
-    def ordered(pos, w):  # `_order` with the sorted positions kept in the graph
-        if pos.ndim == 1:
-            pos_sorted, perm = torch.sort(pos, stable=True)
-            return pos_sorted, w.index_select(1, perm)
-        pos_sorted, perm = torch.sort(pos, dim=1, stable=True)
-        return pos_sorted, torch.gather(w, 1, perm)
-
-    if sort_u:
-        pu, u = ordered(pu, u)
-    if sort_v:
-        pv, v = ordered(pv, v)
-    flags = ((_capi.SOT_SQUARE if square else 0) | (_capi.SOT_CUT_SCALE if cut_scale else 0) |
-             (_capi.SOT_RAW_WEIGHTS if raw_weights else 0))
-    _, _, qs, _, _, iu, iv = _capi.quantiles(u.contiguous(), v.contiguous(), pu.detach().contiguous(),
-                                             pv.detach().contiguous(), flags, want_indices=True)
+    u, v, pu, pv, _ = _canonical(x.detach(), y.detach(), x_pos, y_pos, require_sort, raw_weights,
+                                 attach_positions=True)
+    _, _, qs, _, _, iu, iv = _capi.quantiles(u, v, pu.detach(), pv.detach(), _flags(square, cut_scale, raw_weights),
+                                             want_indices=True)
     return position_term_from_plan(qs, iu, iv, pu, pv, p, limit)
 
 
@@ -434,24 +424,17 @@ class Wasserstein1D(torch.nn.Module):
                           backward_mode="recompute" if mode == "recompute" else "fused")
         if self.hinge:  # losses.py:203-205: the ctor flag gates, the call kwarg is the threshold
             loss = torch.nn.functional.relu(loss - kwargs.get("hinge", 0.0))
-        loss = loss.reshape(original_shape)
-        if as64:
-            loss = loss.double()
-        return torch.mean(loss, dim=kwargs.get("dims", None))  # losses.py:211
+        return self._reduce_frames(loss.reshape(original_shape), kwargs.get("dims", None), as64)
+
+    def _reduce_frames(self, loss, dims, as64):
+        """The reference's final `torch.mean(loss, dim=dims)` (losses.py:211) of the per-frame values, cast back to
+        float64 when an input was.  `sharding.ShardedWasserstein1D` overrides this."""
+        return torch.mean(loss.double() if as64 else loss, dim=dims)
 
 
 def _quantiles(x, y, x_pos, y_pos, square, cut_scale, require_sort, raw_weights=False):
-    x, y = (x.abs() if x.is_complex() else x), (y.abs() if y.is_complex() else y)  # metrics path: plain |.|
-    u, v = _rows(x.detach(), "x"), _rows(y.detach(), "y")
-    pu, pv = _support(x_pos, u, "x_pos"), _support(y_pos, v, "y_pos")
-    sort_u, sort_v = require_sort if isinstance(require_sort, tuple) else (require_sort, require_sort)
-    if sort_u:
-        pu, u = _order(pu, u, x_pos)
-    if sort_v:
-        pv, v = _order(pv, v, y_pos)
-    flags = ((_capi.SOT_SQUARE if square else 0) | (_capi.SOT_CUT_SCALE if cut_scale else 0) |
-             (_capi.SOT_RAW_WEIGHTS if raw_weights else 0))
-    return _capi.quantiles(u.contiguous(), v.contiguous(), pu, pv, flags)
+    u, v, pu, pv, _ = _canonical(x.detach(), y.detach(), x_pos, y_pos, require_sort, raw_weights)
+    return _capi.quantiles(u, v, pu, pv, _flags(square, cut_scale, raw_weights))
 
 
 def quantile_function(qs, cws, xs):

@@ -52,12 +52,12 @@ class PeerReducer:
 
     def all_reduce(self, values: torch.Tensor) -> torch.Tensor:
         self.seq += 1
-        return _capi.p2p_allreduce(values, torch.empty_like(values), self.ptrs, self.rank, self.seq)
+        return _capi.p2p_allreduce(values, torch.empty_like(values), self.ptr_array, self.rank, self.seq)
 
     def global_mean(self, local_sum: torch.Tensor, local_count: float):
         """(sum over ranks of local_sum) / (sum of local_count) and 1 / (sum of local_count), (1,) float32 each."""
         self.seq += 1
-        return _capi.p2p_global_mean(local_sum, local_count, self.ptrs, self.rank, self.seq)
+        return _capi.p2p_global_mean(local_sum, local_count, self.ptr_array, self.rank, self.seq)
 
 
 class _GlobalMean(torch.autograd.Function):
@@ -285,22 +285,7 @@ class ShardedWasserstein1D(losses.Wasserstein1D):
                                          self.equal_shards)
         return self._reducer
 
-    def forward(self, x, y, x_pos=None, y_pos=None, **kwargs):
-        if kwargs.get("dims", None) is not None or kwargs.get("return_quantiles", False):
-            return super().forward(x, y, x_pos=x_pos, y_pos=y_pos, **kwargs)
-        if not self.hinge and x.numel() > 0:
-            return super().forward(x, y, x_pos=x_pos, y_pos=y_pos, **kwargs)  # fused global mean
-        if (x_pos is None or y_pos is None) and self.fixed_x is None:
-            raise ValueError("If fixed_x is not provided, x_pos and y_pos must be provided")
-        x_pos_ = self.fixed_x if x_pos is None else x_pos
-        y_pos_ = self.fixed_x if y_pos is None else y_pos
-        need_sort = (bool(self.require_sort) and x_pos is not None, bool(self.require_sort) and y_pos is not None)
-        mode = getattr(self, "backward_mode", losses.DEFAULT_BACKWARD_MODE)
-        rows = losses.sot_frames(
-            x, y, x_pos_.to(x.device), y_pos_.to(y.device), p=self.p, square=bool(self.square_dist),
-            cut_scale=bool(kwargs.get("dont_normalize", False) or self.dont_normalize),
-            limit=bool(kwargs.get("limit_quantile_range", False) or self.limit_quantile_range),
-            require_sort=need_sort, backward_mode="recompute" if mode == "recompute" else "fused")
-        if self.hinge:
-            rows = torch.nn.functional.relu(rows - kwargs.get("hinge", 0.0))
-        return global_mean(rows, self.process_group)
+    def _reduce_frames(self, loss, dims, as64):
+        if dims is not None:  # `dims` stays local
+            return super()._reduce_frames(loss, dims, as64)
+        return global_mean(loss, self.process_group)  # (float32 even for float64 inputs)

@@ -55,8 +55,26 @@ class SotMeanPlan(ctypes.Structure):
     ]
 
 
+class SotPairwiseProblem(ctypes.Structure):
+    """`struct sot_pairwise_problem` of include/sot_b200.h."""
+    _fields_ = [
+        ("batch", ctypes.c_int64),
+        ("rows_u", ctypes.c_int64),
+        ("rows_v", ctypes.c_int64),
+        ("n_u", ctypes.c_int32),
+        ("n_v", ctypes.c_int32),
+        ("u", ctypes.c_void_p),
+        ("v", ctypes.c_void_p),
+        ("pos_u", ctypes.c_void_p),
+        ("pos_v", ctypes.c_void_p),
+        ("p", ctypes.c_float),
+        ("flags", ctypes.c_int32),
+    ]
+
+
 # name -> (restype, argtypes); kept in one place so tests can check the exported symbol table
 _P = ctypes.POINTER(SotProblem)
+_PP = ctypes.POINTER(SotPairwiseProblem)
 _V = ctypes.c_void_p
 SIGNATURES = {
     "sot_forward_device": (ctypes.c_int, [_P, _V, _V]),
@@ -70,6 +88,8 @@ SIGNATURES = {
     "sot_plan_from_cdf_device": (ctypes.c_int, [_P, _V, _V, _V, _V, _V, _V]),
     "sot_loss_from_cdf_device": (ctypes.c_int, [_P, _V, _V, _V, _V]),
     "sot_loss_grad_host": (ctypes.c_int, [_P, _V, _V, _V, _V, ctypes.c_int32]),
+    "sot_pairwise_device": (ctypes.c_int, [_PP, _V, _V]),
+    "sot_pairwise_backward_device": (ctypes.c_int, [_PP, _V, _V, _V, _V]),
     "sot_host_release": (ctypes.c_int, [ctypes.c_int32]),
     "sot_abi_version": (ctypes.c_int, []),
     "sot_last_error": (ctypes.c_char_p, []),
@@ -345,6 +365,47 @@ def quantiles(u, v, pos_u, pos_v, flags, from_cdf=False, want_indices=False):
         _launch("sot_quantiles_device", u.device, ctypes.byref(prob), _ptr(uq), _ptr(vq), _ptr(qs), _ptr(cu),
                 _ptr(cv), _ptr(iu), _ptr(iv))
     return (uq, vq, qs, cu, cv, iu, iv) if want_indices else (uq, vq, qs, cu, cv)
+
+
+MAX_PAIRWISE_BINS = 8448  # longest row of the pairwise entry points (include/sot_b200.h)
+
+
+def pairwise_problem(u, v, pos_u, pos_v, p: float, flags: int) -> SotPairwiseProblem:
+    """u: (B, P, n), v: (B, R, m) contiguous CUDA float32; pos_u (n,), pos_v (m,) ascending."""
+    for t, name in ((u, "x"), (v, "y"), (pos_u, "x_pos"), (pos_v, "y_pos")):
+        _dev_tensor(t, name)
+        if not t.is_contiguous():
+            raise ValueError("sot_b200: tensors must be contiguous")
+    if u.ndim != 3 or v.ndim != 3 or u.shape[0] != v.shape[0]:
+        raise ValueError(f"sot_b200: expected (B, P, n) and (B, R, m) rows, got {tuple(u.shape)} and {tuple(v.shape)}")
+    if pos_u.shape != (u.shape[2],) or pos_v.shape != (v.shape[2],):
+        raise ValueError(f"sot_b200: positions of shape {tuple(pos_u.shape)} / {tuple(pos_v.shape)} for rows of "
+                         f"{u.shape[2]} / {v.shape[2]} bins")
+    if len({u.device, v.device, pos_u.device, pos_v.device}) != 1:
+        raise ValueError("sot_b200: all tensors must be on the same CUDA device")
+    return SotPairwiseProblem(u.shape[0], u.shape[1], v.shape[1], u.shape[2], v.shape[2], u.data_ptr(), v.data_ptr(),
+                              pos_u.data_ptr(), pos_v.data_ptr(), float(p), int(flags))
+
+
+def pairwise(u, v, pos_u, pos_v, p, flags) -> torch.Tensor:
+    """(B, P, R) float32: W_p^p of every (u[b, i], v[b, j])."""
+    prob = pairwise_problem(u, v, pos_u, pos_v, p, flags)
+    dist = torch.empty(u.shape[0], u.shape[1], v.shape[1], dtype=torch.float32, device=u.device)
+    _launch("sot_pairwise_device", u.device, ctypes.byref(prob), _ptr(dist))
+    return dist
+
+
+def pairwise_backward(u, v, pos_u, pos_v, p, flags, upstream, want_gu=True, want_gv=True):
+    """Gradients of sum_{b,i,j} upstream[b, i, j] * dist[b, i, j] w.r.t. u and v (None where not wanted)."""
+    prob = pairwise_problem(u, v, pos_u, pos_v, p, flags)
+    _dev_tensor(upstream, "upstream")
+    if upstream.shape != (u.shape[0], u.shape[1], v.shape[1]) or not upstream.is_contiguous():
+        raise ValueError("sot_b200: the upstream gradient must be a contiguous (B, P, R) tensor")
+    alloc = torch.zeros_like if upstream.numel() == 0 else torch.empty_like  # (no pairs: nothing is launched)
+    gu = alloc(u) if want_gu else None
+    gv = alloc(v) if want_gv else None
+    _launch("sot_pairwise_backward_device", u.device, ctypes.byref(prob), _ptr(upstream), _ptr(gu), _ptr(gv))
+    return gu, gv
 
 
 def loss_from_cdf(cu, cv, pos_u, pos_v, p, flags, want_grads=True):

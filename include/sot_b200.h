@@ -135,6 +135,27 @@ int sot_quantiles_device(const sot_problem* prob, float* uq, float* vq, float* q
 int sot_quantile_lookup_device(const float* qs, const float* cws, const float* xs, float* out,
                                int64_t rows, int32_t n_levels, int32_t n_bins, void* stream);
 
+/* ---- pairwise distances (the `torch.cdist` of the loss) ------------------------------------------
+ * dist[b, i, j] = per-frame W_p^p of the pair (u[b, i], v[b, j]), what sot_forward_device gives for that one pair
+ * (u is the target: in SOT_CUT_SCALE mode v is divided by u's mass), without materialising the B*P*R pairs: each
+ * row's CDF is built once.  Positions are one ascending grid per side.  Flags: SOT_SQUARE | SOT_CUT_SCALE | SOT_LIMIT
+ * only (anything else: SOT_EINVAL); rows of at most 8448 bins (else SOT_ETOOBIG); B*P*R at most 2^31 - 1;
+ * B*P*R == 0 launches nothing and returns 0.  Scratch is allocated stream-ordered on `stream` (capturable in a CUDA
+ * graph). */
+typedef struct sot_pairwise_problem {
+    int64_t batch, rows_u, rows_v; /* B, P, R */
+    int32_t n_u, n_v;              /* bins */
+    const float *u, *v;            /* [B, P, n_u], [B, R, n_v] contiguous */
+    const float *pos_u, *pos_v;    /* [n_u], [n_v], ascending */
+    float p;
+    int32_t flags;                 /* SOT_SQUARE | SOT_CUT_SCALE | SOT_LIMIT only */
+} sot_pairwise_problem;
+int sot_pairwise_device(const sot_pairwise_problem* prob, float* dist /* [B, P, R] */, void* stream);
+/* grad_u[b, i, :] = sum_j upstream[b, i, j] * d dist[b, i, j] / d u[b, i, :], grad_v likewise over i; either output
+ * nullable.  Deterministic: two calls give the same bits. */
+int sot_pairwise_backward_device(const sot_pairwise_problem* prob, const float* upstream /* [B, P, R] */,
+                                 float* grad_u, float* grad_v /* nullable */, void* stream);
+
 /* ---- parity harness (same kernels, prologue skipped) ------------------------------------------ */
 
 /* Treat prob->u / prob->v as already-computed CDF rows (e.g. the reference's own `cumsum`

@@ -72,9 +72,26 @@ class SotPairwiseProblem(ctypes.Structure):
     ]
 
 
+class SotBarycenterProblem(ctypes.Structure):
+    """`struct sot_barycenter_problem` of include/sot_b200.h."""
+    _fields_ = [
+        ("count", ctypes.c_int64),
+        ("k", ctypes.c_int32),
+        ("n", ctypes.c_int32),
+        ("n_out", ctypes.c_int32),
+        ("x", ctypes.c_void_p),
+        ("weights", ctypes.c_void_p),
+        ("weights_stride", ctypes.c_int64),
+        ("pos", ctypes.c_void_p),
+        ("pos_out", ctypes.c_void_p),
+        ("flags", ctypes.c_int32),
+    ]
+
+
 # name -> (restype, argtypes); kept in one place so tests can check the exported symbol table
 _P = ctypes.POINTER(SotProblem)
 _PP = ctypes.POINTER(SotPairwiseProblem)
+_PB = ctypes.POINTER(SotBarycenterProblem)
 _V = ctypes.c_void_p
 SIGNATURES = {
     "sot_forward_device": (ctypes.c_int, [_P, _V, _V]),
@@ -90,6 +107,8 @@ SIGNATURES = {
     "sot_loss_grad_host": (ctypes.c_int, [_P, _V, _V, _V, _V, ctypes.c_int32]),
     "sot_pairwise_device": (ctypes.c_int, [_PP, _V, _V]),
     "sot_pairwise_backward_device": (ctypes.c_int, [_PP, _V, _V, _V, _V]),
+    "sot_barycenter_device": (ctypes.c_int, [_PB, _V, _V]),
+    "sot_barycenter_backward_device": (ctypes.c_int, [_PB, _V, _V, _V]),
     "sot_host_release": (ctypes.c_int, [ctypes.c_int32]),
     "sot_abi_version": (ctypes.c_int, []),
     "sot_last_error": (ctypes.c_char_p, []),
@@ -406,6 +425,47 @@ def pairwise_backward(u, v, pos_u, pos_v, p, flags, upstream, want_gu=True, want
     gv = alloc(v) if want_gv else None
     _launch("sot_pairwise_backward_device", u.device, ctypes.byref(prob), _ptr(upstream), _ptr(gu), _ptr(gv))
     return gu, gv
+
+
+MAX_BARYCENTER_ENTRIES = 1 << 24  # K x n per barycenter (include/sot_b200.h)
+
+
+def barycenter_problem(x, weights, pos, pos_out, flags: int) -> SotBarycenterProblem:
+    """x: (N, K, n) contiguous CUDA float32; weights (K,) shared or (N, K); pos (n,), pos_out (M,) ascending."""
+    for t, name in ((x, "x"), (weights, "weights"), (pos, "pos"), (pos_out, "out_pos")):
+        _dev_tensor(t, name)
+        if not t.is_contiguous():
+            raise ValueError("sot_b200: tensors must be contiguous")
+    if x.ndim != 3:
+        raise ValueError(f"sot_b200: expected (N, K, n) rows, got {tuple(x.shape)}")
+    N, K, n = x.shape
+    if weights.shape not in ((K,), (N, K)):
+        raise ValueError(f"sot_b200: weights of shape {tuple(weights.shape)} for {K} rows per barycenter")
+    if pos.shape != (n,) or pos_out.ndim != 1:
+        raise ValueError(f"sot_b200: positions of shape {tuple(pos.shape)} / {tuple(pos_out.shape)} for rows of {n} bins")
+    if len({x.device, weights.device, pos.device, pos_out.device}) != 1:
+        raise ValueError("sot_b200: all tensors must be on the same CUDA device")
+    return SotBarycenterProblem(N, K, n, pos_out.shape[0], x.data_ptr(), weights.data_ptr(),
+                                0 if weights.ndim == 1 else K, pos.data_ptr(), pos_out.data_ptr(), int(flags))
+
+
+def barycenter(x, weights, pos, pos_out, flags) -> torch.Tensor:
+    """(N, M) float32: the W2 barycenter of each x[b] as mass per point of `pos_out`."""
+    prob = barycenter_problem(x, weights, pos, pos_out, flags)
+    out = torch.empty(x.shape[0], pos_out.shape[0], dtype=torch.float32, device=x.device)
+    _launch("sot_barycenter_device", x.device, ctypes.byref(prob), _ptr(out))
+    return out
+
+
+def barycenter_backward(x, weights, pos, pos_out, flags, upstream) -> torch.Tensor:
+    """Gradient of sum_{b,m} upstream[b, m] * out[b, m] w.r.t. x, (N, K, n)."""
+    prob = barycenter_problem(x, weights, pos, pos_out, flags)
+    _dev_tensor(upstream, "upstream")
+    if upstream.shape != (x.shape[0], pos_out.shape[0]) or not upstream.is_contiguous():
+        raise ValueError("sot_b200: the upstream gradient must be a contiguous (N, M) tensor")
+    grad = torch.empty_like(x)
+    _launch("sot_barycenter_backward_device", x.device, ctypes.byref(prob), _ptr(upstream), _ptr(grad))
+    return grad
 
 
 def loss_from_cdf(cu, cv, pos_u, pos_v, p, flags, want_grads=True):

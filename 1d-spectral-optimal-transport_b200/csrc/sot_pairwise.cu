@@ -685,6 +685,44 @@ int finish(int rc, void* scratch, cudaStream_t stream) {
 
 }  // namespace
 
+namespace sot {
+namespace pairwise {
+
+// `rows` unpaired rows of n bins as one pairwise problem: the first half is the u lane, the rest the v lane, so the
+// lanes' CDF rows, masses, dL/dCDF rows and gradient rows each follow one another in the caller's buffers.
+static Args unpaired(const float* x, long long rows, int n, bool square, float* cdf, double* mass) {
+    const long long h = (rows + 1) / 2;
+    Args a{};
+    a.batch = 1;
+    a.rows_u = h;
+    a.rows_v = rows - h;
+    a.n = a.m = n;
+    a.u = x;
+    a.v = x + h * n;
+    a.flags = square ? FLAG_SQUARE : 0;
+    a.cu = cdf;
+    a.cv = cdf + h * pad4(n + 2);
+    a.mass_u = mass;
+    a.mass_v = mass + h;
+    return a;
+}
+
+int launch_row_cdfs(const float* x, long long rows, int n, bool square, float* cdf, double* mass, cudaStream_t s) {
+    return launch_cdfs(unpaired(x, rows, n, square, cdf, mass), s);
+}
+
+int launch_row_grads(const float* x, long long rows, int n, bool square, const double* mass, float* dcdf, float* grad,
+                     cudaStream_t s) {
+    const Args a = unpaired(x, rows, n, square, nullptr, const_cast<double*>(mass));
+    const long long h = a.rows_u;
+    sot_pairwise_rowgrad_kernel<false><<<static_cast<unsigned>(h), TPB, 0, s>>>(a, dcdf, 1, nullptr, dcdf + h * n, 1,
+                                                                                  grad, grad + h * n);
+    return sot::launched(cudaGetLastError(), "sot_pairwise_rowgrad_kernel");
+}
+
+}  // namespace pairwise
+}  // namespace sot
+
 extern "C" {
 
 int sot_pairwise_device(const sot_pairwise_problem* prob, float* dist, void* stream) {

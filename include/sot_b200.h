@@ -156,6 +156,32 @@ int sot_pairwise_device(const sot_pairwise_problem* prob, float* dist /* [B, P, 
 int sot_pairwise_backward_device(const sot_pairwise_problem* prob, const float* upstream /* [B, P, R] */,
                                  float* grad_u, float* grad_v /* nullable */, void* stream);
 
+/* ---- Wasserstein barycenters (W2) ------------------------------------------------------------------------------
+ * out[b, :] = the W2 barycenter of the K rows x[b, 0..K-1, :] with weights w[b, :] (weights_stride K) or w[:] (stride
+ * 0), as mass per point of the ascending grid pos_out (each row sums to 1).  Each row is normalised by its own mass
+ * (weights = x^2 with SOT_SQUARE), its CDF c_j formed, qs = the stable sort of all K*n CDF entries, and the step
+ * qs_k - qs_{k-1} (qs_{-1} = 0) is placed at z_k = sum_j w_j pos[min(searchsorted_left(c_j, qs_k), n-1)] and split
+ * linearly between the two grid points around it (below the grid: point 0; at or above its last point: point n_out-1).
+ * Weights are used as given and must be non-negative; a barycenter with a negative or non-finite weight or a
+ * non-finite input row gives a NaN row (and NaN gradient rows).  Flags: SOT_SQUARE only (anything else: SOT_EINVAL);
+ * k, n, n_out >= 1; k * n at most 2^24 per barycenter (else SOT_ETOOBIG); count == 0 launches nothing and returns 0.
+ * Deterministic (two calls give the same bits; a barycenter's result does not depend on the others in the call); no
+ * host synchronisation; scratch is allocated stream-ordered on `stream` (capturable in a CUDA graph). */
+typedef struct sot_barycenter_problem {
+    int64_t count;              /* N barycenters */
+    int32_t k, n, n_out;        /* rows per barycenter, bins per row, output points */
+    const float* x;             /* [N, k, n] contiguous */
+    const float* weights;       /* [k] (weights_stride 0) or [N, k] (weights_stride k) */
+    int64_t weights_stride;
+    const float *pos, *pos_out; /* [n], [n_out], ascending */
+    int32_t flags;              /* SOT_SQUARE only */
+} sot_barycenter_problem;
+int sot_barycenter_device(const sot_barycenter_problem* prob, float* out /* [N, n_out] */, void* stream);
+/* grad_x[b, j, :] = d (sum_m upstream[b, m] * out[b, m]) / d x[b, j, :]; the gradient flows through the steps of qs
+ * only (z depends on the grid and the weights). */
+int sot_barycenter_backward_device(const sot_barycenter_problem* prob, const float* upstream /* [N, n_out] */,
+                                   float* grad_x /* [N, k, n] */, void* stream);
+
 /* ---- parity harness (same kernels, prologue skipped) ------------------------------------------ */
 
 /* Treat prob->u / prob->v as already-computed CDF rows (e.g. the reference's own `cumsum`

@@ -88,10 +88,27 @@ class SotBarycenterProblem(ctypes.Structure):
     ]
 
 
+class SotBarycenterGroupsProblem(ctypes.Structure):
+    """`struct sot_barycenter_groups_problem` of include/sot_b200.h."""
+    _fields_ = [
+        ("groups", ctypes.c_int64),
+        ("rows", ctypes.c_int64),
+        ("n", ctypes.c_int32),
+        ("n_out", ctypes.c_int32),
+        ("x", ctypes.c_void_p),
+        ("offsets", ctypes.c_void_p),
+        ("weights", ctypes.c_void_p),
+        ("pos", ctypes.c_void_p),
+        ("pos_out", ctypes.c_void_p),
+        ("flags", ctypes.c_int32),
+    ]
+
+
 # name -> (restype, argtypes); kept in one place so tests can check the exported symbol table
 _P = ctypes.POINTER(SotProblem)
 _PP = ctypes.POINTER(SotPairwiseProblem)
 _PB = ctypes.POINTER(SotBarycenterProblem)
+_PG = ctypes.POINTER(SotBarycenterGroupsProblem)
 _V = ctypes.c_void_p
 SIGNATURES = {
     "sot_forward_device": (ctypes.c_int, [_P, _V, _V]),
@@ -109,6 +126,8 @@ SIGNATURES = {
     "sot_pairwise_backward_device": (ctypes.c_int, [_PP, _V, _V, _V, _V]),
     "sot_barycenter_device": (ctypes.c_int, [_PB, _V, _V]),
     "sot_barycenter_backward_device": (ctypes.c_int, [_PB, _V, _V, _V]),
+    "sot_barycenter_groups_device": (ctypes.c_int, [_PG, _V, _V]),
+    "sot_barycenter_groups_backward_device": (ctypes.c_int, [_PG, _V, _V, _V]),
     "sot_host_release": (ctypes.c_int, [ctypes.c_int32]),
     "sot_abi_version": (ctypes.c_int, []),
     "sot_last_error": (ctypes.c_char_p, []),
@@ -465,6 +484,52 @@ def barycenter_backward(x, weights, pos, pos_out, flags, upstream) -> torch.Tens
         raise ValueError("sot_b200: the upstream gradient must be a contiguous (N, M) tensor")
     grad = torch.empty_like(x)
     _launch("sot_barycenter_backward_device", x.device, ctypes.byref(prob), _ptr(upstream), _ptr(grad))
+    return grad
+
+
+MAX_GROUPED_ENTRIES = (1 << 31) - 1  # R x n per grouped call (include/sot_b200.h)
+
+
+def barycenter_groups_problem(x, offsets, weights, pos, pos_out, flags: int) -> SotBarycenterGroupsProblem:
+    """x: (R, n) contiguous CUDA float32 in group order; offsets (G + 1,) int64; weights (R,) or None (1 / K_g);
+    pos (n,), pos_out (M,) ascending."""
+    for t, name in ((x, "x"), (pos, "pos"), (pos_out, "out_pos")) + (() if weights is None else ((weights, "weights"),)):
+        _dev_tensor(t, name)
+    if offsets.dtype != torch.int64 or offsets.ndim != 1 or offsets.shape[0] < 1 or not offsets.is_cuda:
+        raise ValueError(f"sot_b200: offsets must be a 1-D CUDA int64 tensor of G + 1 entries, got {offsets.dtype} "
+                         f"{tuple(offsets.shape)}")
+    if not all(t.is_contiguous() for t in (x, offsets, pos, pos_out) + (() if weights is None else (weights,))):
+        raise ValueError("sot_b200: tensors must be contiguous")
+    if x.ndim != 2:
+        raise ValueError(f"sot_b200: expected (R, n) rows, got {tuple(x.shape)}")
+    R, n = x.shape
+    if weights is not None and weights.shape != (R,):
+        raise ValueError(f"sot_b200: weights of shape {tuple(weights.shape)} for {R} rows")
+    if pos.shape != (n,) or pos_out.ndim != 1:
+        raise ValueError(f"sot_b200: positions of shape {tuple(pos.shape)} / {tuple(pos_out.shape)} for rows of {n} bins")
+    if len({x.device, offsets.device, pos.device, pos_out.device} | ({weights.device} if weights is not None else set())) != 1:
+        raise ValueError("sot_b200: all tensors must be on the same CUDA device")
+    return SotBarycenterGroupsProblem(offsets.shape[0] - 1, R, n, pos_out.shape[0], x.data_ptr(), offsets.data_ptr(),
+                                      None if weights is None else weights.data_ptr(), pos.data_ptr(),
+                                      pos_out.data_ptr(), int(flags))
+
+
+def barycenter_groups(x, offsets, weights, pos, pos_out, flags) -> torch.Tensor:
+    """(G, M) float32: the W2 barycenter of each group of rows x[offsets[g]:offsets[g + 1]]."""
+    prob = barycenter_groups_problem(x, offsets, weights, pos, pos_out, flags)
+    out = torch.empty(prob.groups, pos_out.shape[0], dtype=torch.float32, device=x.device)
+    _launch("sot_barycenter_groups_device", x.device, ctypes.byref(prob), _ptr(out))
+    return out
+
+
+def barycenter_groups_backward(x, offsets, weights, pos, pos_out, flags, upstream) -> torch.Tensor:
+    """Gradient of sum_{g,m} upstream[g, m] * out[g, m] w.r.t. x, (R, n)."""
+    prob = barycenter_groups_problem(x, offsets, weights, pos, pos_out, flags)
+    _dev_tensor(upstream, "upstream")
+    if upstream.shape != (prob.groups, pos_out.shape[0]) or not upstream.is_contiguous():
+        raise ValueError("sot_b200: the upstream gradient must be a contiguous (G, M) tensor")
+    grad = torch.empty_like(x)
+    _launch("sot_barycenter_groups_backward_device", x.device, ctypes.byref(prob), _ptr(upstream), _ptr(grad))
     return grad
 
 

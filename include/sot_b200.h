@@ -182,6 +182,34 @@ int sot_barycenter_device(const sot_barycenter_problem* prob, float* out /* [N, 
 int sot_barycenter_backward_device(const sot_barycenter_problem* prob, const float* upstream /* [N, n_out] */,
                                    float* grad_x /* [N, k, n] */, void* stream);
 
+/* ---- grouped Wasserstein barycenters (W2) ----------------------------------------------------------------------
+ * out[g, :] = the barycenter above of the rows offsets[g] .. offsets[g + 1] - 1 of x, in increasing row order, with
+ * their weights weights[row] (or, weights NULL, fl32(1 / K_g) each for a group of K_g rows): bit for bit what
+ * sot_barycenter_device gives for those rows alone.  Groups of any size: no padding and no per-group cap; R * n at
+ * most 2^31 - 1 per call (else SOT_ETOOBIG).  A group with no rows gets a NaN row, and so does a non-finite row or a
+ * negative or non-finite weight for its own group (and its gradient rows).  The offsets table is read on the device
+ * only: group g is used when 0 <= offsets[g] <= offsets[g + 1] <= rows and no earlier offset exceeds offsets[g]; any
+ * other group gets a NaN row, and no row outside x is read.  Flags: SOT_SQUARE only; n, n_out >= 1; groups, rows >= 0.
+ * groups == 0 launches nothing; rows == 0 (every group empty) sets the output rows to NaN with one memset and
+ * launches no kernel (the backward does nothing).  Deterministic, independent of the other groups in the call, no
+ * host synchronisation; scratch is allocated stream-ordered on `stream` for all the entries at once (about 24 bytes
+ * per entry R * n, 28 in the backward; DESIGN.md section 4). */
+typedef struct sot_barycenter_groups_problem {
+    int64_t groups, rows;        /* G, R */
+    int32_t n, n_out;
+    const float* x;              /* [R, n]: group g is rows offsets[g] .. offsets[g+1]-1 */
+    const int64_t* offsets;      /* [G + 1], device */
+    const float* weights;        /* [R], or NULL: 1/K_g within each group */
+    const float *pos, *pos_out;  /* [n], [n_out], ascending */
+    int32_t flags;               /* SOT_SQUARE only */
+} sot_barycenter_groups_problem;
+int sot_barycenter_groups_device(const sot_barycenter_groups_problem* prob, float* out /* [G, n_out] */,
+                                 void* stream);
+/* grad_x[r, :] = d (sum_{g,m} upstream[g, m] * out[g, m]) / d x[r, :]; zero for a row in no group. */
+int sot_barycenter_groups_backward_device(const sot_barycenter_groups_problem* prob,
+                                          const float* upstream /* [G, n_out] */, float* grad_x /* [R, n] */,
+                                          void* stream);
+
 /* ---- parity harness (same kernels, prologue skipped) ------------------------------------------ */
 
 /* Treat prob->u / prob->v as already-computed CDF rows (e.g. the reference's own `cumsum`

@@ -124,6 +124,7 @@ SIGNATURES = {
     "sot_loss_grad_host": (ctypes.c_int, [_P, _V, _V, _V, _V, ctypes.c_int32]),
     "sot_pairwise_device": (ctypes.c_int, [_PP, _V, _V]),
     "sot_pairwise_backward_device": (ctypes.c_int, [_PP, _V, _V, _V, _V]),
+    "sot_pairwise_knn_device": (ctypes.c_int, [_PP, ctypes.c_int32, _V, _V, _V, _V]),
     "sot_barycenter_device": (ctypes.c_int, [_PB, _V, _V]),
     "sot_barycenter_backward_device": (ctypes.c_int, [_PB, _V, _V, _V]),
     "sot_barycenter_groups_device": (ctypes.c_int, [_PG, _V, _V]),
@@ -444,6 +445,22 @@ def pairwise_backward(u, v, pos_u, pos_v, p, flags, upstream, want_gu=True, want
     gv = alloc(v) if want_gv else None
     _launch("sot_pairwise_backward_device", u.device, ctypes.byref(prob), _ptr(upstream), _ptr(gu), _ptr(gv))
     return gu, gv
+
+
+KNN_MAX_K = 128  # largest k of sot_pairwise_knn_device (include/sot_b200.h)
+
+
+def pairwise_knn(u, v, pos_u, pos_v, p, flags, k: int, want_walked: bool = False):
+    """(values (B, P, k) float32, indices (B, P, k) int64, walked (1,) int64 or None): the k smallest W_p^p of each
+    u[b, i] against the v[b, :] rows, ascending, NaN last, the lower index first on equal values."""
+    prob = pairwise_problem(u, v, pos_u, pos_v, p, flags)
+    B, P = u.shape[0], u.shape[1]
+    values = torch.empty(B, P, k, dtype=torch.float32, device=u.device)
+    indices = torch.empty(B, P, k, dtype=torch.int64, device=u.device)
+    walked = torch.empty(1, dtype=torch.int64, device=u.device) if want_walked else None
+    _launch("sot_pairwise_knn_device", u.device, ctypes.byref(prob), int(k), _ptr(values), _ptr(indices),
+            _ptr(walked))
+    return values, indices, walked
 
 
 MAX_BARYCENTER_ENTRIES = 1 << 24  # K x n per barycenter (include/sot_b200.h)

@@ -20,6 +20,7 @@
 #include <cuda_runtime.h>
 
 #include <atomic>
+#include <cmath>
 
 #include "../../include/sot_b200.h"
 #include "sot_device.cuh"
@@ -559,6 +560,310 @@ __global__ void __launch_bounds__(TPB) sot_pairwise_rowgrad_kernel(const Args a,
     }
 }
 
+// ---- exact k nearest v rows of every u row, with walks pruned by a quantile lower bound (DESIGN.md §4) -------------
+// Q(t) = pos[min(lb(t), n - 1)] is the step quantile function of a stored CDF row (lb(t): entries below t); the walk
+// integrates |Q_u - Q_v|^p over [0, max(end_u, end_v)].  a_l = the mean of Q over I_l = [l h, (l + 1) h], h = t0 / L,
+// and Jensen on each interval gives D >= LB = h sum_l |a_u,l - a_v,l|^p.  The kernels compute LB from fp64 means and
+// a pair is skipped only when LB (1 - eta) - eps exceeds tau, the k-th value walked so far: its fp32 value would then
+// be strictly above tau (eta, eps and the shrink `del` of the means are derived in DESIGN.md §4).
+constexpr int KL = 32;                      // intervals of [0, t0]
+constexpr double kT0 = 1.0 - 0x1p-20;       // the bound covers [0, t0]; a row is bounded when its CDF ends >= t0
+constexpr int KQ = 32;                      // queries (u rows) per CTA: one per lane
+constexpr int KD = 32;                      // database (v) rows per tile: four per warp
+constexpr int KW = 8;                       // warps per CTA
+constexpr int kKnnCap = 128;                // largest k: the per-query lists are KQ * k (value, index) pairs in smem
+constexpr int kMaxSlices = 256;             // database slices per query tile (merge heads per warp in smem)
+constexpr long long kKnnTargetCtas = 592;   // CTAs the database is sliced for (4 per SM) ...
+constexpr long long kMinSliceRows = 1024;   // ... in slices long enough for the threshold to tighten after its seeding
+
+struct Knn {
+    int k, slices;
+    const double* emb_u;  // [batch * rows_u][KL] interval means, fp64
+    const double* del_u;  // [batch * rows_u]: bound on their rounding, < 0 for a row without a bound
+    const double* emb_v;
+    const double* del_v;
+    unsigned* tau;        // [batch * rows_u]: float bits of the smallest published k-th value (0xffffffff: none)
+    float* lv;            // [batch * rows_u][slices][k]: each slice's sorted best values ...
+    int* li;              // ... and their v row indices
+    unsigned long long* walked;  // nullable
+    double coef, expo, eta, eps;  // LB = coef * S^expo (S = sum_l d_l, or sum_l d_l^2 when expo = p / 2)
+    bool squares;
+};
+
+// total order of the results: value ascending, NaN after every number, then the lower index
+SOT_DEVINL bool knn_less(float v, int i, float w, int j) {
+    const bool nv = v != v, nw = w != w;
+    if (nv != nw) return nw;
+    if (!nv && v != w) return v < w;
+    return i < j;
+}
+
+// One warp per row (u rows first, then v rows): lane l forms the mean of Q over I_l in fp64 and a bound on its rounding.
+__global__ void __launch_bounds__(256) sot_pairwise_knn_embed_kernel(const Args a, double* __restrict__ emb_u,
+                                                                    double* __restrict__ del_u,
+                                                                    double* __restrict__ emb_v,
+                                                                    double* __restrict__ del_v) {
+    const int lane = threadIdx.x & 31;
+    const long long row = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+    const long long nu_rows = a.batch * a.rows_u;
+    if (row >= nu_rows + a.batch * a.rows_v) return;
+    const bool is_u = row < nu_rows;
+    const long long k = is_u ? row : row - nu_rows;
+    const int n = is_u ? a.n : a.m;
+    const float* const c = is_u ? a.cu + k * pad4(a.n + 2) : a.cv + k * pad4(a.m + 2);
+    const float* const pos = is_u ? a.pos_u : a.pos_v;
+    const double mass = is_u ? a.mass_u[k] : a.mass_v[k];
+    // the walk integrates Q only for a non-decreasing row (NaN fails the test)
+    bool ok = true;
+    for (int i = lane; i < n; i += 32) ok = ok && c[i] >= (i > 0 ? c[i - 1] : 0.0f);
+    const double h = kT0 / KL, lo = lane * h, hi = lo + h;  // (exact: t0 has 20 significant bits)
+    int i = 0, top = n;  // first entry above lo: segment i is (c[i - 1], c[i]] (c[-1] = 0), where Q = pos[i]
+    while (i < top) {
+        const int mid = (i + top) >> 1;
+        if (static_cast<double>(c[mid]) <= lo) i = mid + 1; else top = mid;
+    }
+    double sum = 0.0, asum = 0.0;
+    for (; i < n; ++i) {
+        const double s0 = fmax(i > 0 ? static_cast<double>(c[i - 1]) : 0.0, lo);
+        const double s1 = fmin(static_cast<double>(c[i]), hi);
+        if (s1 > s0) {
+            const double x = pos[i];
+            sum += x * (s1 - s0);
+            asum += fabs(x) * (s1 - s0);
+        }
+        if (static_cast<double>(c[i]) >= hi) break;
+    }
+    const double mean = sum / h;
+    // |fl(mean) - mean| <= (segments + 3) 2^-53 mean(|pos|) with at most n + 1 segments: twice that, for margin
+    double del = static_cast<double>(n + 8) * 0x1p-52 * (asum / h);
+    ok = ok && isfinite(mean) && isfinite(del);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) del = fmax(del, __shfl_xor_sync(FULL_MASK, del, off));
+    const bool bounded = __all_sync(FULL_MASK, ok) && isfinite(mass) && static_cast<float>(mass) > SAFE_EPS &&
+                         static_cast<double>(c[n - 1]) >= kT0;
+    (is_u ? emb_u : emb_v)[k * KL + lane] = mean;
+    if (lane == 0) (is_u ? del_u : del_v)[k] = bounded ? del : -1.0;
+}
+
+// One CTA per (batch entry, tile of KQ u rows, slice of the v rows).  Per tile of KD v rows: LB of the KQ x KD pairs
+// against each query's threshold, the survivors walked one warp per pair on the CDF rows in global memory (walk_pair +
+// warp_sum: the bits of sot_pairwise_loss_kernel), and each query's k best kept in shared memory.  The threshold is
+// the smaller of this CTA's k-th value and the one other slices published with atomicMin.  PRUNE off (cut mode, the
+// `qs > 1` mask): every pair is walked.  Writes the slice's sorted list of each query.
+template <bool PRUNE, bool CUT>
+__global__ void __launch_bounds__(256) sot_pairwise_knn_kernel(const Args a, const Knn kx) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int n = a.n, m = a.m, K = kx.k;
+    double* const qemb = reinterpret_cast<double*>(smem);  // [KL][KQ]
+    double* const qdel = qemb + KL * KQ;
+    double* const demb = qdel + KQ;  // [KD][KL]
+    double* const ddel = demb + KD * KL;
+    float* const spu = reinterpret_cast<float*>(ddel + KD);
+    float* const spv = spu + pad4(n);
+    float* const lv = spv + pad4(m);  // [KQ][K]
+    int* const li = reinterpret_cast<int*>(lv + KQ * K);
+    int* const surv = li + KQ * K;  // [KQ * KD] survivors q * KD + j
+    float* const sval = reinterpret_cast<float*>(surv + KQ * KD);
+    float* const teff = sval + KQ * KD;  // [KQ] threshold of the tile
+    float* const tloc = teff + KQ;       // [KQ] this CTA's k-th value (+inf until k numbers are kept)
+    int* const lcnt = reinterpret_cast<int*>(tloc + KQ);
+    int* const lworst = lcnt + KQ;
+    int* const nsurv = lworst + KQ;
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    long long blk = blockIdx.x;
+    const int slice = static_cast<int>(blk % kx.slices);
+    blk /= kx.slices;
+    const long long qtiles = (a.rows_u + KQ - 1) / KQ;
+    const long long qt = blk % qtiles, b = blk / qtiles;
+    const int cnt_q = static_cast<int>(min(static_cast<long long>(KQ), a.rows_u - qt * KQ));
+    const long long gq0 = b * a.rows_u + qt * KQ;  // global u row of query 0
+    const long long lo = a.rows_v * slice / kx.slices, hi = a.rows_v * (slice + 1) / kx.slices;
+    for (int e = tid; e < n; e += blockDim.x) spu[e] = a.pos_u[e];
+    for (int e = tid; e < m; e += blockDim.x) spv[e] = a.pos_v[e];
+    if constexpr (PRUNE) {
+        for (int e = tid; e < KL * KQ; e += blockDim.x) {
+            const int q = e % KQ, l = e / KQ;
+            qemb[e] = q < cnt_q ? kx.emb_u[(gq0 + q) * KL + l] : 0.0;
+        }
+        if (tid < KQ) qdel[tid] = tid < cnt_q ? kx.del_u[gq0 + tid] : -1.0;
+    }
+    if (tid < KQ) {
+        lcnt[tid] = 0;
+        lworst[tid] = 0;
+        tloc[tid] = f_inf();
+    }
+    const float thr = thr_of(a.flags);
+    unsigned long long walked = 0;
+    for (long long j0 = lo; j0 < hi; j0 += KD) {
+        const int cnt_d = static_cast<int>(min(static_cast<long long>(KD), hi - j0));
+        const long long gv0 = b * a.rows_v + j0;
+        if constexpr (PRUNE) {
+            for (int e = tid; e < KD * KL; e += blockDim.x)
+                demb[e] = e / KL < cnt_d ? kx.emb_v[gv0 * KL + e] : 0.0;
+            if (tid < KD) ddel[tid] = tid < cnt_d ? kx.del_v[gv0 + tid] : -1.0;
+            if (tid < cnt_q) teff[tid] = fminf(tloc[tid], __uint_as_float(__ldcg(kx.tau + gq0 + tid)));  // (NaN: none)
+        }
+        if (tid == 0) *nsurv = 0;
+        __syncthreads();
+        // ---- bounds: lane = query, warp w takes v rows w, w + 8, w + 16, w + 24 of the tile ----
+        {
+            constexpr int RPW = KD / KW;
+            bool keep[RPW];
+#pragma unroll
+            for (int r = 0; r < RPW; ++r) keep[r] = lane < cnt_q && wid + KW * r < cnt_d;
+            if constexpr (PRUNE) {
+                double s[RPW], shrink[RPW];
+#pragma unroll
+                for (int r = 0; r < RPW; ++r) {
+                    s[r] = 0.0;
+                    shrink[r] = qdel[lane] + ddel[wid + KW * r];
+                }
+#pragma unroll 8
+                for (int l = 0; l < KL; ++l) {
+                    const double qa = qemb[l * KQ + lane];
+#pragma unroll
+                    for (int r = 0; r < RPW; ++r) {
+                        const double d = fmax(fabs(qa - demb[(wid + KW * r) * KL + l]) - shrink[r], 0.0);
+                        s[r] = kx.squares ? fma(d, d, s[r]) : s[r] + d;
+                    }
+                }
+                const double tau = static_cast<double>(teff[lane]);
+#pragma unroll
+                for (int r = 0; r < RPW; ++r) {
+                    if (!keep[r] || qdel[lane] < 0.0 || ddel[wid + KW * r] < 0.0) continue;
+                    const double lb = kx.coef * (kx.expo == 1.0 ? s[r] : pow(s[r], kx.expo));
+                    keep[r] = !(lb * (1.0 - kx.eta) - kx.eps > tau);
+                }
+            }
+#pragma unroll
+            for (int r = 0; r < RPW; ++r)
+                if (keep[r]) surv[atomicAdd(nsurv, 1)] = lane * KD + wid + KW * r;
+        }
+        __syncthreads();
+        const int ns = *nsurv;
+        walked += ns;
+        // ---- walks: one warp per surviving pair ----
+        for (int t = wid; t < ns; t += KW) {
+            const int q = surv[t] / KD, j = surv[t] % KD;
+            const long long gu = gq0 + q, gv = gv0 + j;
+            const float* const crow_u = a.cu + gu * pad4(n + 2);
+            const float* const crow_v = a.cv + gv * pad4(m + 2);
+            VScale r;
+            const double mu = a.mass_u[gu], mv = a.mass_v[gv];
+            const Norm nm = pair_norm<CUT>(mu, mv, crow_v, m, r);
+            const bool finite = finite_frame(mu, mv, nm);  // (warp uniform)
+            float acc = 0.0f;
+            if (finite)
+                acc = walk_pair<false, CUT>(PairRows{crow_u, crow_v, spu, spv, n, m, r, a.p, thr}, lane, nullptr,
+                                            [](int, float) {});
+            const double s = warp_sum(static_cast<double>(acc));
+            if (lane == 0) sval[t] = finite ? static_cast<float>(s) : f_nan();
+        }
+        __syncthreads();
+        // ---- each query's thread keeps its k best ----
+        if (tid < cnt_q) {
+            float* const L = lv + tid * K;
+            int* const I = li + tid * K;
+            int cnt = lcnt[tid], worst = lworst[tid];
+            const auto find_worst = [&]() {
+                worst = 0;
+                for (int e = 1; e < K; ++e)
+                    if (knn_less(L[worst], I[worst], L[e], I[e])) worst = e;
+            };
+            for (int t = 0; t < ns; ++t) {
+                if (surv[t] / KD != tid) continue;
+                const float v = sval[t];
+                const int idx = static_cast<int>(j0) + surv[t] % KD;
+                if (cnt < K) {
+                    L[cnt] = v;
+                    I[cnt] = idx;
+                    if (++cnt == K) find_worst();
+                } else if (knn_less(v, idx, L[worst], I[worst])) {
+                    L[worst] = v;
+                    I[worst] = idx;
+                    find_worst();
+                }
+            }
+            lcnt[tid] = cnt;
+            lworst[tid] = worst;
+            // publish the k-th value: a number walked here, never NaN (and +0 for a -0)
+            if (PRUNE && cnt == K && L[worst] == L[worst] && L[worst] < tloc[tid]) {
+                tloc[tid] = L[worst];
+                atomicMin(kx.tau + gq0 + tid, __float_as_uint(L[worst] + 0.0f));
+            }
+        }
+        __syncthreads();
+    }
+    // ---- the slice's list of each query, sorted; empty places hold (NaN, INT_MAX), which rank last ----
+    if (tid < cnt_q) {
+        float* const L = lv + tid * K;
+        int* const I = li + tid * K;
+        const int cnt = lcnt[tid];
+        for (int e = 1; e < cnt; ++e) {
+            const float v = L[e];
+            const int idx = I[e];
+            int f = e;
+            for (; f > 0 && knn_less(v, idx, L[f - 1], I[f - 1]); --f) {
+                L[f] = L[f - 1];
+                I[f] = I[f - 1];
+            }
+            L[f] = v;
+            I[f] = idx;
+        }
+        const long long at = ((gq0 + tid) * kx.slices + slice) * K;
+        for (int e = 0; e < K; ++e) {
+            kx.lv[at + e] = e < cnt ? L[e] : f_nan();
+            kx.li[at + e] = e < cnt ? I[e] : 0x7fffffff;
+        }
+    }
+    if (tid == 0 && kx.walked != nullptr) atomicAdd(kx.walked, walked);
+}
+
+// One warp per query: the k smallest of its slices' sorted lists, in order.
+__global__ void __launch_bounds__(256) sot_pairwise_knn_merge_kernel(const Knn kx, long long queries,
+                                                                    float* __restrict__ values,
+                                                                    int64_t* __restrict__ indices) {
+    __shared__ int head[KW][kMaxSlices];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const long long q = static_cast<long long>(blockIdx.x) * KW + wid;
+    if (q >= queries) return;
+    const int S = kx.slices, K = kx.k;
+    for (int s = lane; s < S; s += 32) head[wid][s] = 0;
+    __syncwarp();
+    const long long base = q * S * K;
+    for (int e = 0; e < K; ++e) {
+        float bv = f_nan();
+        int bi = 0x7fffffff, bs = 0x7fffffff;
+        for (int s = lane; s < S; s += 32) {
+            const int h = head[wid][s];
+            if (h >= K) continue;
+            const float v = kx.lv[base + s * K + h];
+            const int i = kx.li[base + s * K + h];
+            if (knn_less(v, i, bv, bi) || (!knn_less(bv, bi, v, i) && s < bs)) {
+                bv = v;
+                bi = i;
+                bs = s;
+            }
+        }
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) {
+            const float v = __shfl_xor_sync(FULL_MASK, bv, off);
+            const int i = __shfl_xor_sync(FULL_MASK, bi, off), s = __shfl_xor_sync(FULL_MASK, bs, off);
+            if (knn_less(v, i, bv, bi) || (!knn_less(bv, bi, v, i) && s < bs)) {
+                bv = v;
+                bi = i;
+                bs = s;
+            }
+        }
+        if (lane == 0) {
+            values[q * K + e] = bv;
+            indices[q * K + e] = bi;
+            head[wid][bs] += 1;
+        }
+        __syncwarp();
+    }
+}
+
 // ---- host side ------------------------------------------------------------------------------------------------------
 // Largest tile (rows of each side) whose shared memory fits the budget; 1 otherwise (<= 169 KB at 8448 bins).
 int tile_rows(int n, int m, bool grad) {
@@ -607,7 +912,8 @@ using sot::fail;
 using sot::pairwise::Args;
 using sot::pairwise::pad4;
 
-int validate_pairwise(const sot_pairwise_problem* p) {
+// sizes, flags, p and bins: the rules every pairwise entry point shares
+int validate_rows(const sot_pairwise_problem* p) {
     if (p == nullptr) return fail(SOT_EINVAL, "problem is NULL");
     if (p->batch < 0 || p->rows_u < 0 || p->rows_v < 0 || p->n_u < 1 || p->n_v < 1)
         return fail(SOT_EINVAL, "bad sizes: batch=%lld rows_u=%lld rows_v=%lld n_u=%d n_v=%d", (long long)p->batch,
@@ -620,6 +926,11 @@ int validate_pairwise(const sot_pairwise_problem* p) {
     if (p->n_u > sot::pairwise::kMaxBins || p->n_v > sot::pairwise::kMaxBins)
         return fail(SOT_ETOOBIG, "pairwise rows of %d / %d bins: the limit is %d bins", p->n_u, p->n_v,
                     sot::pairwise::kMaxBins);
+    return SOT_OK;
+}
+
+int validate_pairwise(const sot_pairwise_problem* p) {
+    if (int rc = validate_rows(p)) return rc;
     // every grid (one CTA per row index, per tile of T x T pairs, at worst T = 1) within 2^31 - 1 CTAs
     const long long rows = p->rows_u > p->rows_v ? p->rows_u : p->rows_v;
     if (p->batch > 0 && rows > 0 && (p->rows_u > 0x7fffffffLL / p->batch / (p->rows_v > 0 ? p->rows_v : 1) ||
@@ -812,6 +1123,92 @@ int sot_pairwise_backward_device(const sot_pairwise_problem* prob, const float* 
             sot::pairwise::sot_pairwise_rowgrad_kernel<false><<<g, sot::pairwise::TPB, 0, s>>>(
                 a, part_u, slices_u, part_s, part_v, slices_v, grad_u, grad_v);
         rc = sot::launched(cudaGetLastError(), "sot_pairwise_rowgrad_kernel");
+    }
+    return finish(rc, scratch, s);
+}
+
+int sot_pairwise_knn_device(const sot_pairwise_problem* prob, int32_t k, float* values, int64_t* indices,
+                            int64_t* walked, void* stream) {
+    using namespace sot::pairwise;
+    if (int rc = validate_rows(prob)) return rc;
+    if (k < 1 || k > kKnnCap || k > prob->rows_v)
+        return fail(SOT_EINVAL, "k = %d: it must be at least 1 and at most min(rows_v = %lld, %d)", k,
+                    (long long)prob->rows_v, kKnnCap);
+    const long long BP = prob->batch * prob->rows_u, BR = prob->batch * prob->rows_v;
+    if (prob->batch > 0 && (prob->rows_u > 0x7fffffffLL / prob->batch || prob->rows_v > 0x7fffffffLL / prob->batch))
+        return fail(SOT_ETOOBIG, "too many rows for one launch (batch x rows above 2^31 - 1)");
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (BP > 0 && (prob->u == nullptr || prob->v == nullptr || prob->pos_u == nullptr || prob->pos_v == nullptr))
+        return fail(SOT_EINVAL, "u, v, pos_u or pos_v is NULL");
+    if (BP > 0 && (values == nullptr || indices == nullptr)) return fail(SOT_EINVAL, "values or indices is NULL");
+    if (walked != nullptr) {
+        const cudaError_t e = cudaMemsetAsync(walked, 0, sizeof(int64_t), s);
+        if (e != cudaSuccess) return fail(static_cast<int>(e), "cudaMemsetAsync: %s", cudaGetErrorString(e));
+    }
+    if (BP == 0) return SOT_OK;
+    const bool cut = prob->flags & SOT_CUT_SCALE, prune = !(prob->flags & (SOT_CUT_SCALE | SOT_LIMIT));
+    Args a = args_of(prob);
+    const long long qtiles = (a.rows_u + KQ - 1) / KQ;
+    const long long long_slices = (a.rows_v + kMinSliceRows - 1) / kMinSliceRows;
+    long long S = (kKnnTargetCtas + a.batch * qtiles - 1) / (a.batch * qtiles);
+    S = S < long_slices ? S : long_slices;
+    S = S < kMaxSlices ? S : kMaxSlices;
+    Knn kx{};
+    kx.k = k;
+    kx.slices = static_cast<int>(S);
+    kx.walked = reinterpret_cast<unsigned long long*>(walked);
+    // LB = h sum_l d_l^p >= h L^(1 - e) (sum_l d_l^(p / e))^e with e = p / 2 for p >= 2 (sums of squares), else e = p
+    const double pd = prob->p, h = kT0 / KL;
+    kx.squares = pd >= 2.0;
+    kx.expo = kx.squares ? pd / 2.0 : pd;
+    kx.coef = h * std::pow(static_cast<double>(KL), 1.0 - kx.expo);
+    // relative rounding of the fp32 walk (lane sums of ceil((n + m) / 32) terms, the step, the gap, |d|^p, the sum and
+    // the cast) and of the fp64 bound; eps: absolute error of subnormal terms (DESIGN.md §4)
+    const long long per_lane = (a.n + a.m + 31) / 32;
+    kx.eta = (static_cast<double>(per_lane) + std::ceil(pd) + 16.0) * 0x1p-24 + (pd + 1.0) * 0x1p-40;
+    kx.eps = 0x1p-100;
+    sot::pairwise::Carve c;
+    const CdfScratch cs = carve_cdfs(c, a);
+    const long long at_eu = c.take(prune ? 8LL * KL * BP : 0), at_du = c.take(prune ? 8LL * BP : 0);
+    const long long at_ev = c.take(prune ? 8LL * KL * BR : 0), at_dv = c.take(prune ? 8LL * BR : 0);
+    const long long at_tau = c.take(4LL * BP);
+    const long long at_lv = c.take(4LL * BP * S * k), at_li = c.take(4LL * BP * S * k);
+    char* scratch = nullptr;
+    cudaError_t e = cudaMallocAsync(reinterpret_cast<void**>(&scratch), static_cast<size_t>(c.bytes), s);
+    if (e != cudaSuccess) return fail(static_cast<int>(e), "pairwise scratch: %s", cudaGetErrorString(e));
+    place_cdfs(a, cs, scratch);
+    double* const emb_u = reinterpret_cast<double*>(scratch + at_eu);
+    double* const del_u = reinterpret_cast<double*>(scratch + at_du);
+    double* const emb_v = reinterpret_cast<double*>(scratch + at_ev);
+    double* const del_v = reinterpret_cast<double*>(scratch + at_dv);
+    kx.emb_u = emb_u;
+    kx.del_u = del_u;
+    kx.emb_v = emb_v;
+    kx.del_v = del_v;
+    kx.tau = reinterpret_cast<unsigned*>(scratch + at_tau);
+    kx.lv = reinterpret_cast<float*>(scratch + at_lv);
+    kx.li = reinterpret_cast<int*>(scratch + at_li);
+    e = cudaMemsetAsync(kx.tau, 0xff, 4 * static_cast<size_t>(BP), s);  // no threshold published yet
+    int rc = e == cudaSuccess ? SOT_OK : fail(static_cast<int>(e), "cudaMemsetAsync: %s", cudaGetErrorString(e));
+    if (rc == SOT_OK) rc = launch_cdfs(a, s);
+    if (rc == SOT_OK && prune) {
+        const long long grid = (BP + BR + KW - 1) / KW;
+        sot_pairwise_knn_embed_kernel<<<static_cast<unsigned>(grid), 32 * KW, 0, s>>>(a, emb_u, del_u, emb_v, del_v);
+        rc = sot::launched(cudaGetLastError(), "sot_pairwise_knn_embed_kernel");
+    }
+    if (rc == SOT_OK) {
+        const long long grid = a.batch * qtiles * S;
+        const long long smem = 8LL * (KL * KQ + KQ + KD * KL + KD) +
+                               4LL * (pad4(a.n) + pad4(a.m) + 2LL * KQ * k + 2LL * KQ * KD + 4 * KQ + 1);
+        e = prune ? launch_big<sot_pairwise_knn_kernel<true, false>>(grid, 32 * KW, smem, s, a, kx)
+            : cut ? launch_big<sot_pairwise_knn_kernel<false, true>>(grid, 32 * KW, smem, s, a, kx)
+                  : launch_big<sot_pairwise_knn_kernel<false, false>>(grid, 32 * KW, smem, s, a, kx);
+        rc = sot::launched(e, "sot_pairwise_knn_kernel");
+    }
+    if (rc == SOT_OK) {
+        sot_pairwise_knn_merge_kernel<<<static_cast<unsigned>((BP + KW - 1) / KW), 32 * KW, 0, s>>>(kx, BP, values,
+                                                                                                   indices);
+        rc = sot::launched(cudaGetLastError(), "sot_pairwise_knn_merge_kernel");
     }
     return finish(rc, scratch, s);
 }

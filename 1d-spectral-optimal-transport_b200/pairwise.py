@@ -6,15 +6,21 @@ without materialising the P x R pairs: the kernels behind `sot_pairwise_device` 
 only the merge of each pair.  Entry [b, i, j] is what `losses.sot_frames` gives for the single pair
 (x[b, i], y[b, j]) with the same options; the result is differentiable with respect to x and y.
 
+`wasserstein_knn(x, y, k, x_pos, y_pos)` returns each row's k nearest rows of `y` under the same distance, exactly
+the first k columns of a stable sort of `wasserstein_cdist`, without forming the matrix and, in the default mode,
+without walking the pairs that a lower bound rules out.
+
 CUDA only, like the rest of the package: there is no CPU or eager fallback.
 """
 from __future__ import annotations
+
+from typing import NamedTuple
 
 import torch
 
 from . import _capi, losses
 
-__all__ = ["wasserstein_cdist"]
+__all__ = ["wasserstein_cdist", "wasserstein_knn", "KnnResult"]
 
 
 class _Cdist(torch.autograd.Function):
@@ -44,14 +50,8 @@ def _side(t: torch.Tensor, name: str, batched: bool) -> torch.Tensor:
     return losses._magnitude(t)  # complex rows: |z| in torch (no fused complex prologue here)
 
 
-def wasserstein_cdist(x, y, x_pos, y_pos, p=1, square_dist=False, dont_normalize=False, limit_quantile_range=False,
-                      require_sort=True) -> torch.Tensor:
-    """W_p^p of every pair of rows: `x` (P, n) or (B, P, n) targets, `y` (R, m) or (B, R, m) predictions ->
-    (P, R) or (B, P, R) float32, following `torch.cdist`'s batching.  `x_pos` (n,) and `y_pos` (m,) are one grid per
-    side (n may differ from m); unsorted grids are sorted once with the columns permuted when `require_sort`.
-    Options as in `losses.Wasserstein1D`: `square_dist` (weights = magnitude^2), `dont_normalize` (cut mode: y divided
-    by x's mass), `limit_quantile_range` (strict `qs > 1` mask).  float16 / bfloat16 / float64 inputs are converted
-    to float32 as `losses.sot_frames` converts them; complex rows are reduced to |z| first."""
+def _prologue(x, y, x_pos, y_pos, p, square_dist, dont_normalize, limit_quantile_range, require_sort):
+    """The checks and conversions of both entry points: (u (B, P, n), v (B, R, m), pu, pv, flags, batched)."""
     assert p >= 1, f"The OT loss is only valid for p>=1, {p} was given"  # losses.py:271
     batched = x.ndim == 3
     x, y = _side(x, "x", batched), _side(y, "y", batched)
@@ -76,6 +76,54 @@ def wasserstein_cdist(x, y, x_pos, y_pos, p=1, square_dist=False, dont_normalize
     B = lead_u[0] if batched else 1
     u = u.reshape(B, lead_u[-1], n)
     v = v.reshape(B, lead_v[-1], m)
-    flags = losses._flags(square_dist, dont_normalize, False, limit_quantile_range)
+    return u, v, pu, pv, losses._flags(square_dist, dont_normalize, False, limit_quantile_range), batched
+
+
+def wasserstein_cdist(x, y, x_pos, y_pos, p=1, square_dist=False, dont_normalize=False, limit_quantile_range=False,
+                      require_sort=True) -> torch.Tensor:
+    """W_p^p of every pair of rows: `x` (P, n) or (B, P, n) targets, `y` (R, m) or (B, R, m) predictions ->
+    (P, R) or (B, P, R) float32, following `torch.cdist`'s batching.  `x_pos` (n,) and `y_pos` (m,) are one grid per
+    side (n may differ from m); unsorted grids are sorted once with the columns permuted when `require_sort`.
+    Options as in `losses.Wasserstein1D`: `square_dist` (weights = magnitude^2), `dont_normalize` (cut mode: y divided
+    by x's mass), `limit_quantile_range` (strict `qs > 1` mask).  float16 / bfloat16 / float64 inputs are converted
+    to float32 as `losses.sot_frames` converts them; complex rows are reduced to |z| first."""
+    u, v, pu, pv, flags, batched = _prologue(x, y, x_pos, y_pos, p, square_dist, dont_normalize, limit_quantile_range,
+                                             require_sort)
     dist = _Cdist.apply(u, v, pu, pv, float(p), flags)
     return dist if batched else dist[0]
+
+
+class KnnResult(NamedTuple):
+    values: torch.Tensor   # float32 (P, k) or (B, P, k)
+    indices: torch.Tensor  # int64, rows of `y`
+
+
+def wasserstein_knn(x, y, k, x_pos, y_pos, p=1, square_dist=False, dont_normalize=False, limit_quantile_range=False,
+                    require_sort=True) -> KnnResult:
+    """The k nearest rows of `y` to each row of `x` under `wasserstein_cdist` with the same options: exactly
+    `torch.sort(wasserstein_cdist(x, y, x_pos, y_pos, ...), dim=-1, stable=True)` cut to its first k columns -- values
+    bit for bit, ascending, NaN after every number, the lower index first on equal values -- without forming the
+    (P, R) matrix.  Without `dont_normalize` and `limit_quantile_range`, pairs whose lower bound exceeds the k-th value
+    found so far are not walked; the result does not depend on which were.  1 <= k <= min(R, 128).  No gradient: pass
+    rows that do not require one (or run under `torch.no_grad()`), and re-evaluate the selected pairs with
+    `wasserstein_cdist` or `losses.sot_frames` where gradients are wanted."""
+    for t, name in ((x, "x"), (y, "y")):
+        if t.requires_grad and torch.is_grad_enabled():
+            raise NotImplementedError(f"sot_b200: `{name}` requires a gradient: wasserstein_knn has none (detach it, "
+                                      "or re-evaluate the selected pairs with wasserstein_cdist or losses.sot_frames "
+                                      "to get gradients)")
+    u, v, pu, pv, flags, batched = _prologue(x, y, x_pos, y_pos, p, square_dist, dont_normalize, limit_quantile_range,
+                                             require_sort)
+    if isinstance(k, bool) or int(k) != k:
+        raise ValueError(f"sot_b200: k must be an integer, got {k!r}")
+    k, R = int(k), v.shape[1]
+    if k < 1 or k > R:
+        raise ValueError(f"sot_b200: k = {k} must be at least 1 and at most the {R} rows of `y`")
+    if k > _capi.KNN_MAX_K:
+        raise ValueError(f"sot_b200: k = {k} is above the cap of {_capi.KNN_MAX_K} neighbours")
+    if u.shape[0] * u.shape[1] == 0:
+        values = torch.empty(u.shape[0], u.shape[1], k, dtype=torch.float32, device=u.device)
+        indices = torch.empty(u.shape[0], u.shape[1], k, dtype=torch.int64, device=u.device)
+    else:
+        values, indices, _ = _capi.pairwise_knn(u, v, pu, pv, float(p), flags, k)
+    return KnnResult(values, indices) if batched else KnnResult(values[0], indices[0])

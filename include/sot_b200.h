@@ -155,6 +155,18 @@ int sot_pairwise_device(const sot_pairwise_problem* prob, float* dist /* [B, P, 
  * nullable.  Deterministic: two calls give the same bits. */
 int sot_pairwise_backward_device(const sot_pairwise_problem* prob, const float* upstream /* [B, P, R] */,
                                  float* grad_u, float* grad_v /* nullable */, void* stream);
+/* Exact k nearest neighbours: for every u[b, i], the k smallest dist[b, i, :] of sot_pairwise_device, sorted ascending
+ * (NaN after every number, the lower index first on equal values), as values[b, i, :k] (the same bits as the dist
+ * entries) and their v row indices indices[b, i, :k] -- the first k columns of a stable sort of dist, without forming
+ * it.  1 <= k <= min(rows_v, 128) (else SOT_EINVAL): 128 keeps 32 queries' lists in one CTA's shared memory.  Without
+ * SOT_CUT_SCALE and SOT_LIMIT, a pair is walked only when a lower bound on its distance (interval means of the two
+ * quantile functions) does not exceed the k-th value found so far; skipping it provably cannot change the result.  In
+ * the other modes every pair is walked.  `walked` (nullable, device) receives the number of pairs walked, which may
+ * vary from call to call; the results do not.  Problem rules as above, except that only batch * rows_u and
+ * batch * rows_v (not the pairs) are capped at 2^31 - 1; batch * rows_u == 0 launches no kernel.  No host
+ * synchronisation; scratch is stream-ordered (capturable in a CUDA graph). */
+int sot_pairwise_knn_device(const sot_pairwise_problem* prob, int32_t k, float* values /* [B, P, k] */,
+                            int64_t* indices /* [B, P, k] */, int64_t* walked /* nullable */, void* stream);
 
 /* ---- Wasserstein barycenters (W2) ------------------------------------------------------------------------------
  * out[b, :] = the W2 barycenter of the K rows x[b, 0..K-1, :] with weights w[b, :] (weights_stride K) or w[:] (stride

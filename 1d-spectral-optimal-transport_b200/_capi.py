@@ -125,6 +125,7 @@ SIGNATURES = {
     "sot_pairwise_device": (ctypes.c_int, [_PP, _V, _V]),
     "sot_pairwise_backward_device": (ctypes.c_int, [_PP, _V, _V, _V, _V]),
     "sot_pairwise_knn_device": (ctypes.c_int, [_PP, ctypes.c_int32, _V, _V, _V, _V]),
+    "sot_pairwise_radius_device": (ctypes.c_int, [_PP, ctypes.c_float, ctypes.c_int64, _V, _V, _V, _V, _V, _V]),
     "sot_barycenter_device": (ctypes.c_int, [_PB, _V, _V]),
     "sot_barycenter_backward_device": (ctypes.c_int, [_PB, _V, _V, _V]),
     "sot_barycenter_groups_device": (ctypes.c_int, [_PG, _V, _V]),
@@ -461,6 +462,22 @@ def pairwise_knn(u, v, pos_u, pos_v, p, flags, k: int, want_walked: bool = False
     _launch("sot_pairwise_knn_device", u.device, ctypes.byref(prob), int(k), _ptr(values), _ptr(indices),
             _ptr(walked))
     return values, indices, walked
+
+
+def pairwise_radius(u, v, pos_u, pos_v, p, flags, radius: float, capacity: int, want_walked: bool = False):
+    """(rows, cols, values, count, walked): count (1,) int64 on the device is the number of (b, i, j) whose W_p^p is
+    <= radius (fp32); when it is at most `capacity`, the first count entries of rows (b * P + i) and cols (j), int64,
+    and values, float32, (capacity,) each, are those pairs in row-major order.  walked: (1,) int64 or None."""
+    prob = pairwise_problem(u, v, pos_u, pos_v, p, flags)
+    dev = u.device
+    rows = torch.empty(capacity, dtype=torch.int64, device=dev)
+    cols = torch.empty(capacity, dtype=torch.int64, device=dev)
+    values = torch.empty(capacity, dtype=torch.float32, device=dev)
+    count = torch.empty(1, dtype=torch.int64, device=dev)
+    walked = torch.empty(1, dtype=torch.int64, device=dev) if want_walked else None
+    _launch("sot_pairwise_radius_device", dev, ctypes.byref(prob), float(radius), int(capacity), _ptr(rows),
+            _ptr(cols), _ptr(values), _ptr(count), _ptr(walked))
+    return rows, cols, values, count, walked
 
 
 MAX_BARYCENTER_ENTRIES = 1 << 24  # K x n per barycenter (include/sot_b200.h)

@@ -21,6 +21,7 @@
 
 #include <atomic>
 #include <cmath>
+#include <cub/device/device_radix_sort.cuh>
 
 #include "../../include/sot_b200.h"
 #include "sot_device.cuh"
@@ -576,6 +577,13 @@ constexpr int kMaxSlices = 256;             // database slices per query tile (m
 constexpr long long kKnnTargetCtas = 592;   // CTAs the database is sliced for (4 per SM) ...
 constexpr long long kMinSliceRows = 1024;   // ... in slices long enough for the threshold to tighten after its seeding
 
+// The skip rule of both searches: LB = coef * S^expo (S = sum_l d_l, or sum_l d_l^2 when `squares`, expo = p / 2), and
+// a pair of bounded rows is skipped when LB (1 - eta) - eps exceeds the threshold (bound_of below sets them).
+struct Bound {
+    double coef, expo, eta, eps;
+    bool squares;
+};
+
 struct Knn {
     int k, slices;
     const double* emb_u;  // [batch * rows_u][KL] interval means, fp64
@@ -586,8 +594,7 @@ struct Knn {
     float* lv;            // [batch * rows_u][slices][k]: each slice's sorted best values ...
     int* li;              // ... and their v row indices
     unsigned long long* walked;  // nullable
-    double coef, expo, eta, eps;  // LB = coef * S^expo (S = sum_l d_l, or sum_l d_l^2 when expo = p / 2)
-    bool squares;
+    Bound bd;
 };
 
 // total order of the results: value ascending, NaN after every number, then the lower index
@@ -643,6 +650,36 @@ __global__ void __launch_bounds__(256) sot_pairwise_knn_embed_kernel(const Args 
                          static_cast<double>(c[n - 1]) >= kT0;
     (is_u ? emb_u : emb_v)[k * KL + lane] = mean;
     if (lane == 0) (is_u ? del_u : del_v)[k] = bounded ? del : -1.0;
+}
+
+// The bounds of one tile of KQ queries x KD v rows: lane = query, warp w takes v rows w, w + 8, w + 16, w + 24 (the
+// query means in shared memory [l][q], the v rows' means [j][l]).  keep[r] is cleared for a pair of bounded rows
+// whose LB (1 - eta) - eps exceeds tau.  (sot_pairwise_knn_kernel has these lines inline: calling this helper there
+// changes its instruction schedule.)
+SOT_DEVINL void tile_bounds(const Bound& bd, const double* qemb, const double* qdel, const double* demb,
+                            const double* ddel, int lane, int wid, double tau, bool (&keep)[KD / KW]) {
+    constexpr int RPW = KD / KW;
+    double s[RPW], shrink[RPW];
+#pragma unroll
+    for (int r = 0; r < RPW; ++r) {
+        s[r] = 0.0;
+        shrink[r] = qdel[lane] + ddel[wid + KW * r];
+    }
+#pragma unroll 8
+    for (int l = 0; l < KL; ++l) {
+        const double qa = qemb[l * KQ + lane];
+#pragma unroll
+        for (int r = 0; r < RPW; ++r) {
+            const double d = fmax(fabs(qa - demb[(wid + KW * r) * KL + l]) - shrink[r], 0.0);
+            s[r] = bd.squares ? fma(d, d, s[r]) : s[r] + d;
+        }
+    }
+#pragma unroll
+    for (int r = 0; r < RPW; ++r) {
+        if (!keep[r] || qdel[lane] < 0.0 || ddel[wid + KW * r] < 0.0) continue;
+        const double lb = bd.coef * (bd.expo == 1.0 ? s[r] : pow(s[r], bd.expo));
+        keep[r] = !(lb * (1.0 - bd.eta) - bd.eps > tau);
+    }
 }
 
 // One CTA per (batch entry, tile of KQ u rows, slice of the v rows).  Per tile of KD v rows: LB of the KQ x KD pairs
@@ -724,15 +761,15 @@ __global__ void __launch_bounds__(256) sot_pairwise_knn_kernel(const Args a, con
 #pragma unroll
                     for (int r = 0; r < RPW; ++r) {
                         const double d = fmax(fabs(qa - demb[(wid + KW * r) * KL + l]) - shrink[r], 0.0);
-                        s[r] = kx.squares ? fma(d, d, s[r]) : s[r] + d;
+                        s[r] = kx.bd.squares ? fma(d, d, s[r]) : s[r] + d;
                     }
                 }
                 const double tau = static_cast<double>(teff[lane]);
 #pragma unroll
                 for (int r = 0; r < RPW; ++r) {
                     if (!keep[r] || qdel[lane] < 0.0 || ddel[wid + KW * r] < 0.0) continue;
-                    const double lb = kx.coef * (kx.expo == 1.0 ? s[r] : pow(s[r], kx.expo));
-                    keep[r] = !(lb * (1.0 - kx.eta) - kx.eps > tau);
+                    const double lb = kx.bd.coef * (kx.bd.expo == 1.0 ? s[r] : pow(s[r], kx.bd.expo));
+                    keep[r] = !(lb * (1.0 - kx.bd.eta) - kx.bd.eps > tau);
                 }
             }
 #pragma unroll
@@ -864,6 +901,143 @@ __global__ void __launch_bounds__(256) sot_pairwise_knn_merge_kernel(const Knn k
     }
 }
 
+// ---- every v row within a fixed radius of each u row, with the same bound and walk (DESIGN.md §4) -----------------
+constexpr long long kRadiusTargetCtas = 4736;    // CTAs the database is sliced for (about ten waves of three per SM,
+constexpr long long kRadiusMinSliceRows = 1024;  // so that uneven hit counts even out); slices need no merge step
+
+struct Radius {
+    int slices;
+    float radius;
+    long long capacity;
+    const double* emb_u;  // as in Knn
+    const double* del_u;
+    const double* emb_v;
+    const double* del_v;
+    unsigned long long* count;   // pairs within the radius
+    unsigned long long* keys;    // [capacity]: (b P + i) R + j of each of them, in no particular order ...
+    float* vals;                 // ... and its distance
+    unsigned long long* walked;  // nullable
+    Bound bd;
+};
+
+// One CTA per (batch entry, tile of KQ u rows, slice of the v rows), as in sot_pairwise_knn_kernel, with the radius
+// as every query's threshold from the first tile on.  Per tile of KD v rows: the bounds, the survivors walked one warp
+// per pair (walk_pair + warp_sum: the bits of sot_pairwise_loss_kernel), and the pairs with dist <= radius reserved
+// slots with one atomicAdd on the counter per tile; slots at or past `capacity` are counted but not written.  PRUNE
+// off (cut mode, the `qs > 1` mask): every pair is walked.
+template <bool PRUNE, bool CUT>
+__global__ void __launch_bounds__(256) sot_pairwise_radius_kernel(const Args a, const Radius rx) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int n = a.n, m = a.m;
+    double* const qemb = reinterpret_cast<double*>(smem);  // [KL][KQ]
+    double* const qdel = qemb + KL * KQ;
+    double* const demb = qdel + KQ;  // [KD][KL]
+    double* const ddel = demb + KD * KL;
+    float* const spu = reinterpret_cast<float*>(ddel + KD);
+    float* const spv = spu + pad4(n);
+    int* const surv = reinterpret_cast<int*>(spv + pad4(m));  // [KQ * KD] survivors q * KD + j
+    int* const hit = surv + KQ * KD;                         // [KQ * KD] the survivors within the radius ...
+    float* const hval = reinterpret_cast<float*>(hit + KQ * KD);  // ... and their distances
+    unsigned long long* const hbase = reinterpret_cast<unsigned long long*>(hval + KQ * KD);  // the tile's first slot
+    int* const nsurv = reinterpret_cast<int*>(hbase + 1);
+    int* const nhit = nsurv + 1;
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    long long blk = blockIdx.x;
+    const int slice = static_cast<int>(blk % rx.slices);
+    blk /= rx.slices;
+    const long long qtiles = (a.rows_u + KQ - 1) / KQ;
+    const long long qt = blk % qtiles, b = blk / qtiles;
+    const int cnt_q = static_cast<int>(min(static_cast<long long>(KQ), a.rows_u - qt * KQ));
+    const long long gq0 = b * a.rows_u + qt * KQ;  // global u row of query 0, b P + i
+    const long long lo = a.rows_v * slice / rx.slices, hi = a.rows_v * (slice + 1) / rx.slices;
+    for (int e = tid; e < n; e += blockDim.x) spu[e] = a.pos_u[e];
+    for (int e = tid; e < m; e += blockDim.x) spv[e] = a.pos_v[e];
+    if constexpr (PRUNE) {
+        for (int e = tid; e < KL * KQ; e += blockDim.x) {
+            const int q = e % KQ, l = e / KQ;
+            qemb[e] = q < cnt_q ? rx.emb_u[(gq0 + q) * KL + l] : 0.0;
+        }
+        if (tid < KQ) qdel[tid] = tid < cnt_q ? rx.del_u[gq0 + tid] : -1.0;
+    }
+    const float thr = thr_of(a.flags), radius = rx.radius;
+    unsigned long long walked = 0;
+    for (long long j0 = lo; j0 < hi; j0 += KD) {
+        const int cnt_d = static_cast<int>(min(static_cast<long long>(KD), hi - j0));
+        const long long gv0 = b * a.rows_v + j0;
+        if constexpr (PRUNE) {
+            for (int e = tid; e < KD * KL; e += blockDim.x)
+                demb[e] = e / KL < cnt_d ? rx.emb_v[gv0 * KL + e] : 0.0;
+            if (tid < KD) ddel[tid] = tid < cnt_d ? rx.del_v[gv0 + tid] : -1.0;
+        }
+        if (tid == 0) {
+            *nsurv = 0;
+            *nhit = 0;
+        }
+        __syncthreads();
+        {
+            bool keep[KD / KW];
+#pragma unroll
+            for (int r = 0; r < KD / KW; ++r) keep[r] = lane < cnt_q && wid + KW * r < cnt_d;
+            if constexpr (PRUNE) tile_bounds(rx.bd, qemb, qdel, demb, ddel, lane, wid, radius, keep);
+#pragma unroll
+            for (int r = 0; r < KD / KW; ++r)
+                if (keep[r]) surv[atomicAdd(nsurv, 1)] = lane * KD + wid + KW * r;
+        }
+        __syncthreads();
+        const int ns = *nsurv;
+        walked += ns;
+        for (int t = wid; t < ns; t += KW) {
+            const int q = surv[t] / KD, j = surv[t] % KD;
+            const long long gu = gq0 + q, gv = gv0 + j;
+            const float* const crow_u = a.cu + gu * pad4(n + 2);
+            const float* const crow_v = a.cv + gv * pad4(m + 2);
+            VScale r;
+            const double mu = a.mass_u[gu], mv = a.mass_v[gv];
+            const Norm nm = pair_norm<CUT>(mu, mv, crow_v, m, r);
+            const bool finite = finite_frame(mu, mv, nm);  // (warp uniform)
+            float acc = 0.0f;
+            if (finite)
+                acc = walk_pair<false, CUT>(PairRows{crow_u, crow_v, spu, spv, n, m, r, a.p, thr}, lane, nullptr,
+                                            [](int, float) {});
+            const double s = warp_sum(static_cast<double>(acc));
+            const float d = finite ? static_cast<float>(s) : f_nan();
+            if (lane == 0 && d <= radius) {  // (NaN never counts)
+                const int h = atomicAdd(nhit, 1);
+                hit[h] = surv[t];
+                hval[h] = d;
+            }
+        }
+        __syncthreads();
+        const int nh = *nhit;
+        if (nh > 0) {  // (CTA uniform)
+            if (tid == 0) *hbase = atomicAdd(rx.count, static_cast<unsigned long long>(nh));
+            __syncthreads();
+            const unsigned long long at = *hbase;
+            for (int e = tid; e < nh; e += blockDim.x) {
+                if (at + e >= static_cast<unsigned long long>(rx.capacity)) break;
+                const int q = hit[e] / KD, j = hit[e] % KD;
+                rx.keys[at + e] = static_cast<unsigned long long>((gq0 + q) * a.rows_v + j0 + j);
+                rx.vals[at + e] = hval[e];
+            }
+        }
+        __syncthreads();  // the tile's lists and counters are reused by the next one
+    }
+    if (tid == 0 && rx.walked != nullptr) atomicAdd(rx.walked, walked);
+}
+
+// The keys, sorted into `rows`, split in place into the row b P + i and the column j of each of the first
+// min(count, capacity) pairs.
+__global__ void __launch_bounds__(256) sot_pairwise_radius_split_kernel(const unsigned long long* __restrict__ count,
+                                                                       long long capacity, long long rows_v,
+                                                                       int64_t* __restrict__ rows,
+                                                                       int64_t* __restrict__ cols) {
+    const long long e = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (e >= capacity || static_cast<unsigned long long>(e) >= *count) return;
+    const long long key = rows[e], row = key / rows_v;
+    rows[e] = row;
+    cols[e] = key - row * rows_v;
+}
+
 // ---- host side ------------------------------------------------------------------------------------------------------
 // Largest tile (rows of each side) whose shared memory fits the budget; 1 otherwise (<= 169 KB at 8448 bins).
 int tile_rows(int n, int m, bool grad) {
@@ -902,6 +1076,22 @@ struct Carve {
         return at;
     }
 };
+
+// The constants of the skip rule for p and rows of n and m bins (DESIGN.md §4).
+Bound bound_of(float p, int n, int m) {
+    Bound bd{};
+    // LB = h sum_l d_l^p >= h L^(1 - e) (sum_l d_l^(p / e))^e with e = p / 2 for p >= 2 (sums of squares), else e = p
+    const double pd = p, h = kT0 / KL;
+    bd.squares = pd >= 2.0;
+    bd.expo = bd.squares ? pd / 2.0 : pd;
+    bd.coef = h * std::pow(static_cast<double>(KL), 1.0 - bd.expo);
+    // relative rounding of the fp32 walk (lane sums of ceil((n + m) / 32) terms, the step, the gap, |d|^p, the sum and
+    // the cast) and of the fp64 bound; eps: absolute error of subnormal terms
+    const long long per_lane = (n + m + 31) / 32;
+    bd.eta = (static_cast<double>(per_lane) + std::ceil(pd) + 16.0) * 0x1p-24 + (pd + 1.0) * 0x1p-40;
+    bd.eps = 0x1p-100;
+    return bd;
+}
 
 }  // namespace pairwise
 }  // namespace sot
@@ -992,6 +1182,24 @@ int finish(int rc, void* scratch, cudaStream_t stream) {
     const cudaError_t e = cudaFreeAsync(scratch, stream);
     if (rc == SOT_OK && e != cudaSuccess) return fail(static_cast<int>(e), "cudaFreeAsync: %s", cudaGetErrorString(e));
     return rc;
+}
+
+// the interval means of every u and v row (after the CDF pre-pass): what both searches prune with
+int launch_embed(const Args& a, double* emb_u, double* del_u, double* emb_v, double* del_v, cudaStream_t s) {
+    using sot::pairwise::KW;
+    const long long grid = (a.batch * (a.rows_u + a.rows_v) + KW - 1) / KW;
+    sot::pairwise::sot_pairwise_knn_embed_kernel<<<static_cast<unsigned>(grid), 32 * KW, 0, s>>>(a, emb_u, del_u,
+                                                                                                  emb_v, del_v);
+    return sot::launched(cudaGetLastError(), "sot_pairwise_knn_embed_kernel");
+}
+
+// both searches cap B * P and B * R, not the pairs; the inputs are read when there is a pair (`any`)
+int validate_search(const sot_pairwise_problem* p, bool any) {
+    if (p->batch > 0 && (p->rows_u > 0x7fffffffLL / p->batch || p->rows_v > 0x7fffffffLL / p->batch))
+        return fail(SOT_ETOOBIG, "too many rows for one launch (batch x rows above 2^31 - 1)");
+    if (any && (p->u == nullptr || p->v == nullptr || p->pos_u == nullptr || p->pos_v == nullptr))
+        return fail(SOT_EINVAL, "u, v, pos_u or pos_v is NULL");
+    return SOT_OK;
 }
 
 }  // namespace
@@ -1135,11 +1343,8 @@ int sot_pairwise_knn_device(const sot_pairwise_problem* prob, int32_t k, float* 
         return fail(SOT_EINVAL, "k = %d: it must be at least 1 and at most min(rows_v = %lld, %d)", k,
                     (long long)prob->rows_v, kKnnCap);
     const long long BP = prob->batch * prob->rows_u, BR = prob->batch * prob->rows_v;
-    if (prob->batch > 0 && (prob->rows_u > 0x7fffffffLL / prob->batch || prob->rows_v > 0x7fffffffLL / prob->batch))
-        return fail(SOT_ETOOBIG, "too many rows for one launch (batch x rows above 2^31 - 1)");
+    if (int rc = validate_search(prob, BP > 0)) return rc;
     const cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (BP > 0 && (prob->u == nullptr || prob->v == nullptr || prob->pos_u == nullptr || prob->pos_v == nullptr))
-        return fail(SOT_EINVAL, "u, v, pos_u or pos_v is NULL");
     if (BP > 0 && (values == nullptr || indices == nullptr)) return fail(SOT_EINVAL, "values or indices is NULL");
     if (walked != nullptr) {
         const cudaError_t e = cudaMemsetAsync(walked, 0, sizeof(int64_t), s);
@@ -1157,16 +1362,7 @@ int sot_pairwise_knn_device(const sot_pairwise_problem* prob, int32_t k, float* 
     kx.k = k;
     kx.slices = static_cast<int>(S);
     kx.walked = reinterpret_cast<unsigned long long*>(walked);
-    // LB = h sum_l d_l^p >= h L^(1 - e) (sum_l d_l^(p / e))^e with e = p / 2 for p >= 2 (sums of squares), else e = p
-    const double pd = prob->p, h = kT0 / KL;
-    kx.squares = pd >= 2.0;
-    kx.expo = kx.squares ? pd / 2.0 : pd;
-    kx.coef = h * std::pow(static_cast<double>(KL), 1.0 - kx.expo);
-    // relative rounding of the fp32 walk (lane sums of ceil((n + m) / 32) terms, the step, the gap, |d|^p, the sum and
-    // the cast) and of the fp64 bound; eps: absolute error of subnormal terms (DESIGN.md §4)
-    const long long per_lane = (a.n + a.m + 31) / 32;
-    kx.eta = (static_cast<double>(per_lane) + std::ceil(pd) + 16.0) * 0x1p-24 + (pd + 1.0) * 0x1p-40;
-    kx.eps = 0x1p-100;
+    kx.bd = bound_of(prob->p, a.n, a.m);
     sot::pairwise::Carve c;
     const CdfScratch cs = carve_cdfs(c, a);
     const long long at_eu = c.take(prune ? 8LL * KL * BP : 0), at_du = c.take(prune ? 8LL * BP : 0);
@@ -1191,11 +1387,7 @@ int sot_pairwise_knn_device(const sot_pairwise_problem* prob, int32_t k, float* 
     e = cudaMemsetAsync(kx.tau, 0xff, 4 * static_cast<size_t>(BP), s);  // no threshold published yet
     int rc = e == cudaSuccess ? SOT_OK : fail(static_cast<int>(e), "cudaMemsetAsync: %s", cudaGetErrorString(e));
     if (rc == SOT_OK) rc = launch_cdfs(a, s);
-    if (rc == SOT_OK && prune) {
-        const long long grid = (BP + BR + KW - 1) / KW;
-        sot_pairwise_knn_embed_kernel<<<static_cast<unsigned>(grid), 32 * KW, 0, s>>>(a, emb_u, del_u, emb_v, del_v);
-        rc = sot::launched(cudaGetLastError(), "sot_pairwise_knn_embed_kernel");
-    }
+    if (rc == SOT_OK && prune) rc = launch_embed(a, emb_u, del_u, emb_v, del_v, s);
     if (rc == SOT_OK) {
         const long long grid = a.batch * qtiles * S;
         const long long smem = 8LL * (KL * KQ + KQ + KD * KL + KD) +
@@ -1209,6 +1401,96 @@ int sot_pairwise_knn_device(const sot_pairwise_problem* prob, int32_t k, float* 
         sot_pairwise_knn_merge_kernel<<<static_cast<unsigned>((BP + KW - 1) / KW), 32 * KW, 0, s>>>(kx, BP, values,
                                                                                                    indices);
         rc = sot::launched(cudaGetLastError(), "sot_pairwise_knn_merge_kernel");
+    }
+    return finish(rc, scratch, s);
+}
+
+int sot_pairwise_radius_device(const sot_pairwise_problem* prob, float radius, int64_t capacity, int64_t* rows,
+                               int64_t* cols, float* values, int64_t* count, int64_t* walked, void* stream) {
+    using namespace sot::pairwise;
+    if (int rc = validate_rows(prob)) return rc;
+    if (radius != radius) return fail(SOT_EINVAL, "the radius is NaN");
+    if (capacity < 0) return fail(SOT_EINVAL, "capacity = %lld: it must be at least 0", (long long)capacity);
+    const long long BP = prob->batch * prob->rows_u, BR = prob->batch * prob->rows_v;
+    const long long pairs = BP * prob->rows_v;  // (< 2^62 under the caps)
+    if (int rc = validate_search(prob, pairs > 0)) return rc;
+    if (count == nullptr) return fail(SOT_EINVAL, "count is NULL");
+    if (pairs > 0 && capacity > 0 && (rows == nullptr || cols == nullptr || values == nullptr))
+        return fail(SOT_EINVAL, "rows, cols or values is NULL");
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    for (int64_t* counter : {count, walked}) {
+        if (counter == nullptr) continue;
+        const cudaError_t e = cudaMemsetAsync(counter, 0, sizeof(int64_t), s);
+        if (e != cudaSuccess) return fail(static_cast<int>(e), "cudaMemsetAsync: %s", cudaGetErrorString(e));
+    }
+    if (pairs == 0) return SOT_OK;
+    const bool cut = prob->flags & SOT_CUT_SCALE, prune = !(prob->flags & (SOT_CUT_SCALE | SOT_LIMIT));
+    const long long cap = capacity < pairs ? capacity : pairs;  // (no more slots can be used)
+    Args a = args_of(prob);
+    const long long qtiles = (a.rows_u + KQ - 1) / KQ;
+    const long long long_slices = (a.rows_v + kRadiusMinSliceRows - 1) / kRadiusMinSliceRows;
+    long long S = (kRadiusTargetCtas + a.batch * qtiles - 1) / (a.batch * qtiles);
+    S = S < long_slices ? S : long_slices;
+    Radius rx{};
+    rx.slices = static_cast<int>(S);
+    rx.radius = radius;
+    rx.capacity = cap;
+    rx.count = reinterpret_cast<unsigned long long*>(count);
+    rx.walked = reinterpret_cast<unsigned long long*>(walked);
+    rx.bd = bound_of(prob->p, a.n, a.m);
+    // the hits' keys (b P + i) R + j are unique and below 2^end_bit - 1, the key of an unused slot's 0xff..f: a radix
+    // sort of the low end_bit bits puts them in torch.nonzero's order, the unused slots last
+    int end_bit = 1;
+    while (end_bit < 64 && (pairs >> end_bit) != 0) ++end_bit;
+    unsigned long long* const keys_out = reinterpret_cast<unsigned long long*>(rows);
+    size_t sort_bytes = 0;
+    if (cap > 0) {
+        const cudaError_t e = cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, rx.keys, keys_out, rx.vals, values,
+                                                              cap, 0, end_bit, s);
+        if (e != cudaSuccess) return fail(static_cast<int>(e), "radix sort set-up: %s", cudaGetErrorString(e));
+    }
+    sot::pairwise::Carve c;
+    const CdfScratch cs = carve_cdfs(c, a);
+    const long long at_eu = c.take(prune ? 8LL * KL * BP : 0), at_du = c.take(prune ? 8LL * BP : 0);
+    const long long at_ev = c.take(prune ? 8LL * KL * BR : 0), at_dv = c.take(prune ? 8LL * BR : 0);
+    const long long at_keys = c.take(8LL * cap), at_vals = c.take(4LL * cap);
+    const long long at_sort = c.take(static_cast<long long>(sort_bytes));
+    char* scratch = nullptr;
+    cudaError_t e = cudaMallocAsync(reinterpret_cast<void**>(&scratch), static_cast<size_t>(c.bytes), s);
+    if (e != cudaSuccess) return fail(static_cast<int>(e), "pairwise scratch: %s", cudaGetErrorString(e));
+    place_cdfs(a, cs, scratch);
+    double* const emb_u = reinterpret_cast<double*>(scratch + at_eu);
+    double* const del_u = reinterpret_cast<double*>(scratch + at_du);
+    double* const emb_v = reinterpret_cast<double*>(scratch + at_ev);
+    double* const del_v = reinterpret_cast<double*>(scratch + at_dv);
+    rx.emb_u = emb_u;
+    rx.del_u = del_u;
+    rx.emb_v = emb_v;
+    rx.del_v = del_v;
+    rx.keys = reinterpret_cast<unsigned long long*>(scratch + at_keys);
+    rx.vals = reinterpret_cast<float*>(scratch + at_vals);
+    e = cudaMemsetAsync(rx.keys, 0xff, 8 * static_cast<size_t>(cap), s);  // unused slots sort last
+    int rc = e == cudaSuccess ? SOT_OK : fail(static_cast<int>(e), "cudaMemsetAsync: %s", cudaGetErrorString(e));
+    if (rc == SOT_OK) rc = launch_cdfs(a, s);
+    if (rc == SOT_OK && prune) rc = launch_embed(a, emb_u, del_u, emb_v, del_v, s);
+    if (rc == SOT_OK) {
+        const long long grid = a.batch * qtiles * S;
+        const long long smem = 8LL * (KL * KQ + KQ + KD * KL + KD + 1) +
+                               4LL * (pad4(a.n) + pad4(a.m) + 3LL * KQ * KD + 2);
+        e = prune ? launch_big<sot_pairwise_radius_kernel<true, false>>(grid, 32 * KW, smem, s, a, rx)
+            : cut ? launch_big<sot_pairwise_radius_kernel<false, true>>(grid, 32 * KW, smem, s, a, rx)
+                  : launch_big<sot_pairwise_radius_kernel<false, false>>(grid, 32 * KW, smem, s, a, rx);
+        rc = sot::launched(e, "sot_pairwise_radius_kernel");
+    }
+    if (rc == SOT_OK && cap > 0) {
+        e = cub::DeviceRadixSort::SortPairs(scratch + at_sort, sort_bytes, rx.keys, keys_out, rx.vals, values, cap, 0,
+                                            end_bit, s);
+        rc = sot::launched(e, "cub::DeviceRadixSort::SortPairs");
+    }
+    if (rc == SOT_OK && cap > 0) {
+        sot_pairwise_radius_split_kernel<<<static_cast<unsigned>((cap + 255) / 256), 256, 0, s>>>(rx.count, cap,
+                                                                                                  a.rows_v, rows, cols);
+        rc = sot::launched(cudaGetLastError(), "sot_pairwise_radius_split_kernel");
     }
     return finish(rc, scratch, s);
 }

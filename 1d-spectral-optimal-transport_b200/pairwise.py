@@ -8,19 +8,21 @@ only the merge of each pair.  Entry [b, i, j] is what `losses.sot_frames` gives 
 
 `wasserstein_knn(x, y, k, x_pos, y_pos)` returns each row's k nearest rows of `y` under the same distance, exactly
 the first k columns of a stable sort of `wasserstein_cdist`, without forming the matrix and, in the default mode,
-without walking the pairs that a lower bound rules out.
+without walking the pairs that a lower bound rules out.  `wasserstein_radius(x, y, r, x_pos, y_pos)` returns every
+pair within distance r, exactly `(wasserstein_cdist(...) <= r).nonzero()` and its values, pruned by the same bound.
 
 CUDA only, like the rest of the package: there is no CPU or eager fallback.
 """
 from __future__ import annotations
 
+import numbers
 from typing import NamedTuple
 
 import torch
 
 from . import _capi, losses
 
-__all__ = ["wasserstein_cdist", "wasserstein_knn", "KnnResult"]
+__all__ = ["wasserstein_cdist", "wasserstein_knn", "KnnResult", "wasserstein_radius", "RadiusResult"]
 
 
 class _Cdist(torch.autograd.Function):
@@ -98,6 +100,14 @@ class KnnResult(NamedTuple):
     indices: torch.Tensor  # int64, rows of `y`
 
 
+def _no_gradient(x, y, fn: str):
+    for t, name in ((x, "x"), (y, "y")):
+        if t.requires_grad and torch.is_grad_enabled():
+            raise NotImplementedError(f"sot_b200: `{name}` requires a gradient: {fn} has none (detach it, "
+                                      "or re-evaluate the selected pairs with wasserstein_cdist or losses.sot_frames "
+                                      "to get gradients)")
+
+
 def wasserstein_knn(x, y, k, x_pos, y_pos, p=1, square_dist=False, dont_normalize=False, limit_quantile_range=False,
                     require_sort=True) -> KnnResult:
     """The k nearest rows of `y` to each row of `x` under `wasserstein_cdist` with the same options: exactly
@@ -107,11 +117,7 @@ def wasserstein_knn(x, y, k, x_pos, y_pos, p=1, square_dist=False, dont_normaliz
     found so far are not walked; the result does not depend on which were.  1 <= k <= min(R, 128).  No gradient: pass
     rows that do not require one (or run under `torch.no_grad()`), and re-evaluate the selected pairs with
     `wasserstein_cdist` or `losses.sot_frames` where gradients are wanted."""
-    for t, name in ((x, "x"), (y, "y")):
-        if t.requires_grad and torch.is_grad_enabled():
-            raise NotImplementedError(f"sot_b200: `{name}` requires a gradient: wasserstein_knn has none (detach it, "
-                                      "or re-evaluate the selected pairs with wasserstein_cdist or losses.sot_frames "
-                                      "to get gradients)")
+    _no_gradient(x, y, "wasserstein_knn")
     u, v, pu, pv, flags, batched = _prologue(x, y, x_pos, y_pos, p, square_dist, dont_normalize, limit_quantile_range,
                                              require_sort)
     if isinstance(k, bool) or int(k) != k:
@@ -127,3 +133,45 @@ def wasserstein_knn(x, y, k, x_pos, y_pos, p=1, square_dist=False, dont_normaliz
     else:
         values, indices, _ = _capi.pairwise_knn(u, v, pu, pv, float(p), flags, k)
     return KnnResult(values, indices) if batched else KnnResult(values[0], indices[0])
+
+
+class RadiusResult(NamedTuple):
+    values: torch.Tensor   # float32 (E,)
+    indices: torch.Tensor  # int64 (E, 2): (row of x, row of y), or (E, 3): (batch entry, row of x, row of y)
+
+
+_FIRST_CAPACITY = 1 << 20  # pairs the first call has room for, at least (16 per row of x beyond 65 536 rows)
+
+
+def wasserstein_radius(x, y, r, x_pos, y_pos, p=1, square_dist=False, dont_normalize=False,
+                       limit_quantile_range=False, require_sort=True) -> RadiusResult:
+    """Every pair within distance `r` under `wasserstein_cdist` with the same options and shapes: with
+    `D = wasserstein_cdist(x, y, x_pos, y_pos, ...)` and `mask = D <= torch.tensor(r, dtype=torch.float32)`, `indices`
+    is `mask.nonzero()` ((E, 2), or (E, 3) for batched rows) and `values` is `D[mask]`, bit for bit, without forming
+    D.  A NaN distance is never within the radius.  Without `dont_normalize` and `limit_quantile_range`, pairs whose
+    lower bound exceeds r are not walked; the result does not depend on which were.
+
+    The call reads the number of pairs back to the host once (the result's size depends on it) and runs the search
+    again, with room for exactly that many, when the first guess of min(B P R, max(2^20, 16 B P)) pairs was too
+    small; to capture a CUDA graph, call `sot_pairwise_radius_device` with a fixed capacity.  No gradient, as for
+    `wasserstein_knn`: re-evaluate the selected pairs with `wasserstein_cdist` or `losses.sot_frames` to train
+    through them."""
+    _no_gradient(x, y, "wasserstein_radius")
+    if isinstance(r, bool) or not isinstance(r, numbers.Real) or r != r:
+        raise ValueError(f"sot_b200: the radius must be a real number and not NaN, got {r!r}")
+    u, v, pu, pv, flags, batched = _prologue(x, y, x_pos, y_pos, p, square_dist, dont_normalize, limit_quantile_range,
+                                             require_sort)
+    B, P, R = u.shape[0], u.shape[1], v.shape[1]
+    pairs = B * P * R
+    if pairs == 0:
+        rows = cols = torch.empty(0, dtype=torch.int64, device=u.device)
+        values = torch.empty(0, dtype=torch.float32, device=u.device)
+    else:
+        capacity = min(pairs, max(_FIRST_CAPACITY, 16 * B * P))
+        rows, cols, values, count, _ = _capi.pairwise_radius(u, v, pu, pv, float(p), flags, float(r), capacity)
+        E = int(count.item())
+        if E > capacity:
+            rows, cols, values, count, _ = _capi.pairwise_radius(u, v, pu, pv, float(p), flags, float(r), E)
+        rows, cols, values = rows[:E], cols[:E], values[:E]
+    parts = (rows // max(P, 1), rows % max(P, 1), cols) if batched else (rows, cols)
+    return RadiusResult(values, torch.stack(parts, 1))

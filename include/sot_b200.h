@@ -167,6 +167,21 @@ int sot_pairwise_backward_device(const sot_pairwise_problem* prob, const float* 
  * synchronisation; scratch is stream-ordered (capturable in a CUDA graph). */
 int sot_pairwise_knn_device(const sot_pairwise_problem* prob, int32_t k, float* values /* [B, P, k] */,
                             int64_t* indices /* [B, P, k] */, int64_t* walked /* nullable */, void* stream);
+/* Exact radius search: every (b, i, j) with dist[b, i, j] <= radius (compared in fp32, so a NaN distance never counts)
+ * for dist as sot_pairwise_device gives it.  *count (device) receives their number.  When *count <= capacity, the
+ * first *count entries of rows (b * P + i), cols (j) and values (the same bits as the dist entries) are exactly those
+ * pairs in ascending (b * P + i, j) order, torch.nonzero's row-major order.  When *count > capacity their contents are
+ * unspecified, and nothing is written at or past `capacity` in either case; capacity == 0 is a count-only call (the
+ * three arrays may then be NULL).  Without SOT_CUT_SCALE and SOT_LIMIT, a pair is walked only when the lower bound of
+ * sot_pairwise_knn_device does not rule it out against the radius; in the other modes every pair is walked, and
+ * radius = +inf never prunes.  `walked` (nullable, device) receives the number of pairs walked, which may vary from
+ * call to call; count, rows, cols and values do not.  A NaN radius or a negative capacity: SOT_EINVAL.  Problem rules
+ * as for sot_pairwise_knn_device; batch * rows_u * rows_v == 0 sets *count = 0 and launches no kernel.  No host
+ * synchronisation; scratch is stream-ordered (capturable in a CUDA graph with a fixed capacity). */
+int sot_pairwise_radius_device(const sot_pairwise_problem* prob, float radius, int64_t capacity,
+                               int64_t* rows /* [capacity] */, int64_t* cols /* [capacity] */,
+                               float* values /* [capacity] */, int64_t* count /* device, 1 */,
+                               int64_t* walked /* nullable */, void* stream);
 
 /* ---- Wasserstein barycenters (W2) ------------------------------------------------------------------------------
  * out[b, :] = the W2 barycenter of the K rows x[b, 0..K-1, :] with weights w[b, :] (weights_stride K) or w[:] (stride
